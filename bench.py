@@ -3,6 +3,7 @@
 decode+grad-psi kernel against its roofline and the CPU oracle port as baseline.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--batch B] [--precision fp32]
+                    [--dump-outputs DIR]
     N>1:  python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 ... bench.py --gpus N
 
 Workload (config.workload): BASELINE.json configs[1] -- LIDVAE(dataset='pinwheel'), latent_dim 2, ICNN(2,512) +
@@ -11,7 +12,7 @@ forward -> loss -> backward -> gradient all-reduce (N>1) -> Adam, i.e. lipschitz
 `value`  : inputs resident in HBM.           `e2e`: same step through the public module API with pinned HOST
 inputs (H2D copy) and the loss read back (D2H) inside the timed region.
 
-`--impl reference` runs the UNMODIFIED reference (oracle/_ref/, populated by oracle/fetch_ref.py in the build container):
+`--impl reference` runs the UNMODIFIED reference (oracle/_ref/, populated by oracle/fetch_ref.py from a reference checkout):
 its own `model.LIDVAE` driven by its own loop `lipschitz.train_model` (lipschitz.py:23-44) in PyTorch on the host cores,
 on the SAME config -- batch 65536 per step, encoder and Adam included, same weights, same synthetic data.  The numpy
 oracle port is only the fallback when oracle/_ref/ is absent (the line then says kind "port").
@@ -434,6 +435,52 @@ def mnist_shaped_times(dev, flush, precision):
     return out
 
 
+DUMP_MAX_BYTES = 60 * 1024 * 1024          # array data of --dump-outputs; with the .npy headers it stays under 64 MB
+
+
+def dump_step_outputs(out_dir, tr, losses, with_grads):
+    """--dump-outputs: what a caller of the timed train step holds after its last step -- the (total, recon, KL) losses
+    (mean over ranks), every parameter after the Adam update, the BatchNorm buffers and, on one GPU, the gradients that
+    update used -- as out_dir/<name>.npy in float32 (float64 for integer buffers), so that two builds can be compared
+    output for output.  (With several GPUs the flat gradient buffer of a rank holds its own or a partly reduced sum, not
+    the gradient the update used, so it is left out.)
+
+    Over the size budget, every array larger than one common element count C is replaced by a fixed sample of C of its
+    flattened elements, the same positions for every array of the same size (numpy default_rng(0)); the kept positions
+    are written beside it as <name>.index.npy (float64) and the original shape as <name>.shape.npy."""
+    import torch
+    arrays = {f"loss_{k}": v.reshape(1) for k, v in zip(("total", "recon", "kl"), losses)}
+    for name, p in tr.model.named_parameters():
+        arrays[f"param.{name}"] = p
+        if with_grads and p.grad is not None:
+            arrays[f"grad.{name}"] = p.grad
+    for name, b in tr.model.named_buffers():
+        arrays[f"buffer.{name}"] = b
+    out = {}
+    for name, t in arrays.items():
+        a = t.detach().cpu().numpy().reshape(t.shape)
+        out[name] = a.astype(np.float32 if a.dtype.kind == "f" and a.itemsize <= 4 else np.float64)
+
+    def cost(c):       # bytes written when arrays above c elements keep c of them (+ 8-byte positions, + shape)
+        return sum(a.nbytes if a.size <= c else c * (a.itemsize + 8) + 8 * a.ndim for a in out.values())
+    cap = max(a.size for a in out.values())
+    if cost(cap) > DUMP_MAX_BYTES:
+        lo, hi = 0, cap
+        while lo < hi:
+            mid = (lo + hi + 1) // 2
+            lo, hi = (mid, hi) if cost(mid) <= DUMP_MAX_BYTES else (lo, mid - 1)
+        cap = lo
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        if a.size > cap:
+            idx = np.sort(np.random.default_rng(0).choice(a.size, cap, replace=False))
+            np.save(os.path.join(out_dir, f"{name}.index.npy"), idx.astype(np.float64))
+            np.save(os.path.join(out_dir, f"{name}.shape.npy"), np.array(a.shape, dtype=np.float64))
+            a = a.reshape(-1)[idx]
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+    print(f"[bench] wrote {len(out)} arrays ({cost(cap) / 2**20:.1f} MiB) to {out_dir}", file=sys.stderr, flush=True)
+
+
 # ----------------------------------------------------------------------------------------- GPU arm
 def run_ours(args, rank, local_rank, world):
     import torch
@@ -493,8 +540,10 @@ def run_ours(args, rank, local_rank, world):
         tr.capture(dev_pool[0])
     run_step = tr.step_graphed if use_graph else tr.step
 
+    last_out = [None]
+
     def step_resident(i):
-        run_step(dev_pool[i % n_pool])
+        last_out[0] = run_step(dev_pool[i % n_pool])
 
     def step_e2e(i):
         if use_graph:      # H2D of THIS step's batch was started by the previous call (next_x): it overlaps that step
@@ -526,6 +575,10 @@ def run_ours(args, rank, local_rank, world):
     t_start = time.time()
     ms = timed(step_resident, args.steps, args.warmup)
     t_end = time.time()
+    if args.dump_outputs:
+        losses = tr.global_losses(*last_out[0])              # collective: every rank joins the mean over ranks
+        if rank == 0:                                        # parameters and buffers are identical on every replica
+            dump_step_outputs(args.dump_outputs, tr, losses, with_grads=world == 1)
     launches = launches_per_step * args.steps
     clocks = sampler.window(t_start, t_end) if sampler else {}
     if world > 1:
@@ -859,7 +912,15 @@ def main():
     ap.add_argument("--no-graph", action="store_true", help="launch the step eagerly instead of replaying a CUDA graph")
     ap.add_argument("--roofline-precision", default=None, choices=["fp32", "tf32", "tf32x3", "f16x3"],
                     help="precision of the kernel described by `roofline` (default: the step's --precision)")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="after the timed steps, write what the last one computed (losses averaged over ranks, updated "
+                         "parameters, BatchNorm buffers and, on one GPU, gradients) as DIR/<name>.npy; inputs and weights "
+                         "are seeded, so runs with the same arguments on two builds can be compared array by array")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to the GPU arm (--impl ours)")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     rank = int(os.environ.get("RANK", 0))
     local_rank = int(os.environ.get("LOCAL_RANK", 0))

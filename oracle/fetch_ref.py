@@ -1,12 +1,13 @@
 #!/usr/bin/env python
 """Populate oracle/_ref/ with the UNMODIFIED reference (test / baseline infrastructure, not product code).
 
-    python oracle/fetch_ref.py           # build container only: needs /root/reference
+    python oracle/fetch_ref.py       # reference: $VAE_SONG_REFERENCE, else ../reference or ../vae-song beside the repo
 
-The reference is a set of Python scripts without packaging (nothing to `pip install`), and /root/reference does not
-exist on the GPU box.  This recipe copies the reference's own files for the hot path -- module.py, model.py, utils.py,
-lipschitz.py, dataset.py -- byte for byte into the git-ignored oracle/_ref/ (listed in .gitignore, NOT in .gpurunignore,
-so it travels to the GPU box exactly like a built .so), plus SHA-256 digests in oracle/_ref/MANIFEST.json.  Nothing under
+The reference is a set of Python scripts without packaging (nothing to `pip install`), and the repository does not ship
+it: it is taken from $VAE_SONG_REFERENCE or, without that, from a checkout named `reference` or `vae-song` in the
+directory that holds this repository (`find_reference()`; build() runs `fetch()`).  This recipe copies the reference's own files for the hot path -- module.py, model.py, utils.py, lipschitz.py,
+dataset.py -- byte for byte into the git-ignored oracle/_ref/ (so that a copy of the tree taken to a GPU machine carries
+them like a built .so), plus SHA-256 digests in oracle/_ref/MANIFEST.json.  Nothing under
 oracle/_ref/ is ever committed, and the product package never imports it (tests/test_abi_host_cpu.py enforces that).
 
 `import_ref()` is how tests/, bench.py's reference arm and __graft_entry__.smoke() reach it: utils.py / lipschitz.py import
@@ -25,7 +26,23 @@ import sys
 import types
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-REF_SRC = os.environ.get("VAE_SONG_REFERENCE", "/root/reference")
+SIBLINGS = ("reference", "vae-song")       # checkout names looked for beside the repository
+
+
+def find_reference() -> str:
+    """Directory of the unmodified reference: $VAE_SONG_REFERENCE if set, else the first sibling checkout of this
+    repository in SIBLINGS that has the reference's module.py; "" when there is none."""
+    env = os.environ.get("VAE_SONG_REFERENCE")
+    if env:
+        return env
+    parent = os.path.dirname(os.path.dirname(HERE))
+    for name in SIBLINGS:
+        if os.path.isfile(os.path.join(parent, name, "module.py")):
+            return os.path.join(parent, name)
+    return ""
+
+
+REF_SRC = find_reference()
 REF_DST = os.path.join(HERE, "_ref")
 FILES = ("module.py", "model.py", "utils.py", "lipschitz.py", "dataset.py")
 
@@ -37,9 +54,10 @@ def _sha(path):
 
 def fetch(verbose=True) -> bool:
     """Copy FILES verbatim from the reference tree.  Returns False (and leaves _ref/ alone) when the tree is absent."""
-    if not os.path.isdir(REF_SRC):
+    if not (REF_SRC and os.path.isdir(REF_SRC)):
         if verbose:
-            print(f"fetch_ref: {REF_SRC} not present; keeping {REF_DST} as it is")
+            print(f"fetch_ref: no reference checkout (VAE_SONG_REFERENCE unset, no {' or '.join('../' + s for s in SIBLINGS)} "
+                  f"beside the repository); keeping {REF_DST} as it is")
         return False
     os.makedirs(REF_DST, exist_ok=True)
     manifest = {}
@@ -83,7 +101,7 @@ def import_ref(swap=None):
     if key is None and "ns" in _cache:
         return _cache["ns"]
     if not available():
-        raise FileNotFoundError(f"{REF_DST} is not populated: run `python oracle/fetch_ref.py` where /root/reference exists")
+        raise FileNotFoundError(f"{REF_DST} is not populated: run `python oracle/fetch_ref.py` where a reference checkout is found")
     for name in ("matplotlib", "matplotlib.pyplot"):
         if name not in sys.modules:
             sys.modules[name] = types.ModuleType(name)

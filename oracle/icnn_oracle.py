@@ -7,8 +7,8 @@ This file is a plain-numpy restatement of the reference algorithm.  Only
 
 Parity pinning: the reference ships no tests or golden vectors for this path
 (SURVEY.md section 4), so the oracle is pinned against outputs of the reference
-itself, run in the build container: ``oracle/make_golden.py`` imports
-``/root/reference/{module,model,utils}.py`` unmodified and writes the fixtures
+itself: ``oracle/make_golden.py`` imports ``{module,model,utils}.py`` of a
+reference checkout (``oracle/fetch_ref.find_reference``) unmodified and writes the fixtures
 under ``tests/golden/`` which ``tests/test_oracle_golden.py`` checks this file
 against (fp64: <=1e-12 relative; fp32 fixtures: fp32 noise floor).
 

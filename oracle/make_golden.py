@@ -1,9 +1,9 @@
 #!/usr/bin/env python
-"""Generate tests/golden/*.npz by RUNNING THE UNMODIFIED REFERENCE (build container only).
+"""Generate tests/golden/*.npz by RUNNING THE UNMODIFIED REFERENCE.
 
-    python oracle/make_golden.py            # needs /root/reference; writes tests/golden/
+    python oracle/make_golden.py            # needs a reference checkout (oracle/fetch_ref.find_reference); writes tests/golden/
 
-The reference (pure Python/PyTorch) is imported from /root/reference exactly as shipped; nothing
+The reference (pure Python/PyTorch) is imported from that checkout exactly as shipped; nothing
 is copied.  utils.py imports matplotlib (absent here) at module scope, so empty stub modules are
 registered first (SURVEY.md section 8(c)).  Inputs and ICNN parameters are drawn with numpy's
 ``default_rng`` through ``oracle.icnn_oracle.random_params`` so that tests can rebuild them
@@ -21,13 +21,16 @@ import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
-REF = os.environ.get("VAE_SONG_REFERENCE", "/root/reference")
 OUT = os.path.join(ROOT, "tests", "golden")
 
+from oracle import golden  # noqa: E402
 from oracle import icnn_oracle as io  # noqa: E402
+from oracle.fetch_ref import REF_SRC as REF  # noqa: E402
 
 
 def import_reference():
+    if not (REF and os.path.isfile(os.path.join(REF, "module.py"))):
+        raise FileNotFoundError("no reference checkout: set VAE_SONG_REFERENCE or place it beside the repository")
     for name in ("matplotlib", "matplotlib.pyplot"):
         if name not in sys.modules:
             m = types.ModuleType(name)
@@ -107,7 +110,7 @@ def gen_icnn(ref_module):
                     out[pre + "g_W0_sum"] = np.array([a.sum(dtype=np.float64), np.abs(a).sum(dtype=np.float64)])
                 else:
                     out[pre + "g_" + k] = a
-    np.savez_compressed(os.path.join(OUT, "icnn_cases.npz"), **out)
+    golden.save(os.path.join(OUT, "icnn_cases.npz"), out)
     print("icnn_cases.npz:", len(out), "arrays")
 
 
@@ -157,7 +160,7 @@ def gen_lidvae(ref_model):
             out[pre + "loss"] = np.array([float(total), float(lrec), float(lreg)])
             for k, q in m.named_parameters():
                 out[pre + "grad/" + k] = q.grad.numpy().copy()
-    np.savez_compressed(os.path.join(OUT, "lidvae_cases.npz"), **out)
+    golden.save(os.path.join(OUT, "lidvae_cases.npz"), out)
     print("lidvae_cases.npz:", len(out), "arrays")
 
 
@@ -192,7 +195,7 @@ def gen_mnist_shaped(ref_model):
             out[f"g{i}/{k}"] = a.grad.numpy().copy()
     out["z"], out["vy"], out["y"], out["dz"] = z, vy, y.detach().numpy(), zt.grad.numpy().copy()
     out["kappa"] = np.array(0.1)
-    np.savez_compressed(os.path.join(OUT, "mnist_shaped.npz"), **out)
+    golden.save(os.path.join(OUT, "mnist_shaped.npz"), out)
     print("mnist_shaped.npz:", len(out), "arrays")
 
 
@@ -231,7 +234,7 @@ def gen_losses(ref_model, ref_utils):
     out["lid_logmse/g_xh"], out["lid_logmse/g_mu"], out["lid_logmse/g_lv"] = (t.grad.numpy().copy() for t in (xht, mut, lvt))
     # utils.kld utils.py:140-141
     out["kld/val"] = np.array(ref_utils.kld(T(mu), T(lv)))
-    np.savez_compressed(os.path.join(OUT, "loss_cases.npz"), **out)
+    golden.save(os.path.join(OUT, "loss_cases.npz"), out)
     print("loss_cases.npz:", len(out), "arrays")
 
 
@@ -258,7 +261,7 @@ def gen_lipschitz(ref_model, ref_utils):
         out[f"{name}/Z"], out[f"{name}/Y"] = Z, Y
         out[f"{name}/i1"], out[f"{name}/i2"] = i1.numpy(), i2.numpy()
         out[f"{name}/res"] = np.array(res)
-    np.savez_compressed(os.path.join(OUT, "lipschitz_cases.npz"), **out)
+    golden.save(os.path.join(OUT, "lipschitz_cases.npz"), out)
     print("lipschitz_cases.npz:", len(out), "arrays")
 
 
@@ -325,7 +328,7 @@ def gen_families(ref_model):
     cd.backward()
     out["chamfer/a"], out["chamfer/b"], out["chamfer/cd"] = a, b, np.array(float(cd))
     out["chamfer/ga"], out["chamfer/gb"] = at.grad.numpy().copy(), bt.grad.numpy().copy()
-    np.savez_compressed(os.path.join(OUT, "family_cases.npz"), **out)
+    golden.save(os.path.join(OUT, "family_cases.npz"), out)
     print("family_cases.npz:", len(out), "arrays")
 
 
@@ -372,7 +375,7 @@ def gen_train_trajectory(ref_model):
     for k, a in sd_to_np(m.state_dict()).items():
         out[f"sd1/{k}"] = a
     out["cfg"] = np.array([nb, B, epochs])
-    np.savez_compressed(os.path.join(OUT, "train_trajectory.npz"), **out)
+    golden.save(os.path.join(OUT, "train_trajectory.npz"), out)
     print("train_trajectory.npz:", len(out), "arrays; first / last loss", losses[0][0], losses[-1][0])
 
 
@@ -410,7 +413,7 @@ def gen_host_logic(ref_model, ref_utils):
         ref_utils.apply_grad_clip(lin, cfg)
         out[f"clip/{tag}/w"] = lin.weight.grad.numpy().copy(); out[f"clip/{tag}/b"] = lin.bias.grad.numpy().copy()
     out["clip/g_w"], out["clip/g_b"] = g[0], g[1][:3]
-    np.savez_compressed(os.path.join(OUT, "host_cases.npz"), **out)
+    golden.save(os.path.join(OUT, "host_cases.npz"), out)
     print("host_cases.npz:", len(out), "arrays")
 
 
@@ -461,7 +464,7 @@ def gen_lidvae_baseline(ref_model):
             out["grad_sum/" + k] = np.array([g.sum(dtype=np.float64), np.abs(g).sum(dtype=np.float64), np.abs(g).max()])
         else:
             out["grad/" + k] = g.copy()
-    np.savez_compressed(os.path.join(OUT, "lidvae_baseline_icnn.npz"), **out)
+    golden.save(os.path.join(OUT, "lidvae_baseline_icnn.npz"), out)
     print("lidvae_baseline_icnn.npz:", len(out), "arrays")
 
 

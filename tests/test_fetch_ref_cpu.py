@@ -1,5 +1,5 @@
-"""oracle/fetch_ref.py: the recipe that puts the UNMODIFIED reference under the git-ignored oracle/_ref/ (so that it travels to
-the GPU box like a built .so) and imports it under private module names."""
+"""oracle/fetch_ref.py: the recipe that puts the UNMODIFIED reference under the git-ignored oracle/_ref/ (so that a copy of
+the tree taken to a GPU machine carries it like a built .so) and imports it under private module names."""
 import os
 import subprocess
 import sys
@@ -20,12 +20,39 @@ def test_ref_dir_is_git_ignored_but_travels():
     assert tracked == "", "reference sources must never be committed"
 
 
-@pytest.mark.skipif(not os.path.isdir(fetch_ref.REF_SRC), reason="reference tree only exists in the build container")
-def test_fetch_copies_verbatim():
+def test_fetch_copies_verbatim(tmp_path, monkeypatch):
+    """The copy is byte for byte (CRLF, trailing whitespace, non-UTF-8 bytes survive) and verify() notices an edit.  Runs on
+    a stand-in source tree so that it needs no checkout of the reference."""
+    src, dst = tmp_path / "reference", tmp_path / "_ref"
+    src.mkdir()
+    for i, n in enumerate(fetch_ref.FILES):
+        (src / n).write_bytes(b"# %s\r\nx = %d  \n\xff\xfe\n" % (n.encode(), i))
+    monkeypatch.setattr(fetch_ref, "REF_SRC", str(src))
+    monkeypatch.setattr(fetch_ref, "REF_DST", str(dst))
     assert fetch_ref.fetch(verbose=False)
     for n in fetch_ref.FILES:
         assert open(os.path.join(fetch_ref.REF_SRC, n), "rb").read() == open(os.path.join(fetch_ref.REF_DST, n), "rb").read()
-    assert fetch_ref.verify()
+    assert fetch_ref.available() and fetch_ref.verify()
+    (dst / fetch_ref.FILES[0]).write_bytes(b"edited\n")
+    assert not fetch_ref.verify()
+    monkeypatch.setattr(fetch_ref, "REF_SRC", "")
+    assert not fetch_ref.fetch(verbose=False)          # no reference tree given: nothing happens
+
+
+def test_find_reference_env_then_sibling_checkout(tmp_path, monkeypatch):
+    (tmp_path / "repo" / "oracle").mkdir(parents=True)
+    monkeypatch.setattr(fetch_ref, "HERE", str(tmp_path / "repo" / "oracle"))
+    monkeypatch.delenv("VAE_SONG_REFERENCE", raising=False)
+    assert fetch_ref.find_reference() == ""
+    (tmp_path / "vae-song").mkdir()
+    (tmp_path / "vae-song" / "module.py").write_text("")
+    assert fetch_ref.find_reference() == str(tmp_path / "vae-song")
+    (tmp_path / "reference").mkdir()
+    assert fetch_ref.find_reference() == str(tmp_path / "vae-song")          # a directory without module.py is not one
+    (tmp_path / "reference" / "module.py").write_text("")
+    assert fetch_ref.find_reference() == str(tmp_path / "reference")
+    monkeypatch.setenv("VAE_SONG_REFERENCE", str(tmp_path / "elsewhere"))
+    assert fetch_ref.find_reference() == str(tmp_path / "elsewhere")
 
 
 @pytest.mark.skipif(not fetch_ref.available(), reason="oracle/_ref not populated")

@@ -9,6 +9,7 @@ import numpy as np
 import pytest
 import torch
 
+from oracle import golden
 from oracle import icnn_oracle as io
 from oracle.make_golden import ICNN_CASES, case_inputs
 
@@ -57,7 +58,7 @@ def test_fwd_bwd_vs_oracle(case):
 def test_vs_reference_fp32_golden(case):
     """Against what the reference itself produced in fp32 on CPU (both sides carry fp32 noise)."""
     name, d, H, B, regime, mode, kappa, seed, with_gpsi = case
-    G = np.load(os.path.join(GOLDEN, "icnn_cases.npz"))
+    G = golden.load(os.path.join(GOLDEN, "icnn_cases.npz"))
     p, z, v, gpsi = case_inputs(d, H, B, regime, seed)
     psi, xhat, dz, g = run_ours(p, z, v, gpsi if with_gpsi else None, mode, kappa)
     pre = f"{name}/f32/"
@@ -139,7 +140,7 @@ def test_reference_idiom_double_backward():
     """module.ICNN used exactly as model.py:820-828 uses it: autograd.grad(create_graph=True) then
     backward -- on OUR module, compared with the golden of the reference module."""
     from vae_song_b200 import module
-    G = np.load(os.path.join(GOLDEN, "icnn_cases.npz"))
+    G = golden.load(os.path.join(GOLDEN, "icnn_cases.npz"))
     name, d, H, B, regime, mode, kappa, seed, _ = ICNN_CASES[0]
     p, z, v, _ = case_inputs(d, H, B, regime, seed)
     icnn = module.ICNN(d, H).cuda()

@@ -8,6 +8,7 @@ import numpy as np
 import pytest
 import torch
 
+from oracle import golden
 from oracle import icnn_oracle as io
 from oracle.make_golden import ICNN_CASES, case_inputs
 
@@ -65,7 +66,7 @@ def test_wide_vs_reference_golden(case):
     """Against what the unmodified reference produced (fp64 golden; oracle/make_golden.py)."""
     name, d, H, B, regime, mode, kappa, seed, with_gpsi = case
     assert not with_gpsi
-    G = np.load(os.path.join(GOLDEN, "icnn_cases.npz"))
+    G = golden.load(os.path.join(GOLDEN, "icnn_cases.npz"))
     p, z, v, _ = case_inputs(d, H, B, regime, seed)
     psi, xhat, dz, g = run_wide(p, z, v, mode, kappa)
     pre = f"{name}/f64/"

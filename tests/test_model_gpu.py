@@ -9,6 +9,7 @@ import torch
 
 from oracle import loss_oracle as lo
 
+from oracle import golden
 from oracle import icnn_oracle as io
 
 from conftest import GOLDEN
@@ -263,7 +264,7 @@ def test_wide_input_icnn_mnist_shaped():
     """MNIST-shaped ICNN decoder (reference defect D1 recipe, SURVEY 8(c)): ICNN(8,48) -> eye(784,8) pad ->
     ICNN(784,64); forward and every gradient against the reference-generated golden (fp64) and the oracle."""
     from vae_song_b200 import module
-    G = np.load(os.path.join(GOLDEN, "mnist_shaped.npz"))
+    G = golden.load(os.path.join(GOLDEN, "mnist_shaped.npz"))
     keys = ("A0w", "A0b", "A1w", "A1b", "A2w", "A2b", "W0", "W1")
     ics = []
     for i, (d, H) in enumerate(((8, 48), (784, 64))):
@@ -354,7 +355,7 @@ def test_unmodified_reference_driver_runs_on_this_package(precision):
     this package's batched driver returns."""
     from oracle import fetch_ref
     if not fetch_ref.available():
-        pytest.skip("oracle/_ref not populated (run oracle/fetch_ref.py where /root/reference exists)")
+        pytest.skip("oracle/_ref not populated (no reference checkout for oracle/fetch_ref.py)")
     from vae_song_b200 import lipschitz as our_lip, model, module, utils
     ns = fetch_ref.import_ref(swap={"module": module, "model": model, "utils": utils})
     assert fetch_ref.verify()                                           # the driver file is the unmodified reference

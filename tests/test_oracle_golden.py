@@ -6,6 +6,7 @@ import os
 import numpy as np
 import pytest
 
+from oracle import golden
 from oracle import icnn_oracle as io
 from oracle import loss_oracle as lo
 from oracle.make_golden import ICNN_CASES, case_inputs
@@ -20,7 +21,7 @@ def relmax(a, b):
 
 @pytest.fixture(scope="module")
 def icnn_golden():
-    return np.load(os.path.join(GOLDEN, "icnn_cases.npz"))
+    return golden.load(os.path.join(GOLDEN, "icnn_cases.npz"))
 
 
 @pytest.mark.parametrize("case", ICNN_CASES, ids=[c[0] for c in ICNN_CASES])
@@ -59,7 +60,7 @@ def test_icnn_oracle_fp32_noise_floor(case, icnn_golden):
 
 
 def test_mnist_shaped_decode_chain():
-    G = np.load(os.path.join(GOLDEN, "mnist_shaped.npz"))
+    G = golden.load(os.path.join(GOLDEN, "mnist_shaped.npz"))
     p0 = {k: G[f"p0/{k}"] for k in io.PARAM_KEYS}
     p1 = {k: G[f"p1/{k}"] for k in io.PARAM_KEYS}
     z, vy, kappa = G["z"], G["vy"].reshape(6, -1), float(G["kappa"])

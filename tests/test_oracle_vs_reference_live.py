@@ -1,7 +1,7 @@
-"""Randomised comparison of the CPU oracle with the UNMODIFIED reference, run live where the reference tree exists
-(this build container: /root/reference, or $VAE_SONG_REFERENCE); skipped elsewhere (the GPU box has no reference tree --
-there the committed fixtures of tests/golden/ are the pin).  Shapes, weight regimes, reparam modes, kappa and the
-psi-gradient path are drawn per seed, beyond the 11 fixed golden cases."""
+"""Randomised comparison of the CPU oracle with the UNMODIFIED reference, run live where a checkout of
+claviclecrusher/vae-song is found (oracle/fetch_ref.find_reference); skipped elsewhere (the repository does not ship the
+reference -- there the committed fixtures of tests/golden/, made from it by oracle/make_golden.py, are the pin).  Shapes, weight regimes,
+reparam modes, kappa and the psi-gradient path are drawn per seed, beyond the 11 fixed golden cases."""
 import os
 import sys
 
@@ -9,9 +9,12 @@ import numpy as np
 import pytest
 import torch
 
+from oracle import fetch_ref
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = os.environ.get("VAE_SONG_REFERENCE", "/root/reference")
-pytestmark = pytest.mark.skipif(not os.path.isfile(os.path.join(REF, "module.py")), reason="reference tree not present")
+REF = fetch_ref.REF_SRC
+pytestmark = pytest.mark.skipif(not (REF and os.path.isfile(os.path.join(REF, "module.py"))),
+                                reason="no checkout of the reference (VAE_SONG_REFERENCE, ../reference, ../vae-song)")
 
 
 @pytest.fixture(scope="module")
