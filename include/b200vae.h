@@ -45,8 +45,9 @@ extern "C" {
  * pair), three tcgen05 kind::f16 MMAs per K step, every operand scaled by an exact power of two into the fp16 range (per
  * tensor for the prepared weights, per sample row for the generated operands) and unscaled in the epilogue.  Same bounds as
  * TF32X3 / FP32.  The wide-input entry points run TF32X3 for it.
- * Every tensor-core precision (TF32, TF32X3, F16X3) of the d <= 4 entry points needs d <= 3 and H <= 1024 and returns
- * B200VAE_EUNSUP otherwise; FP32 takes d <= 4, H <= 4096. */
+ * Every tensor-core precision (TF32, TF32X3, F16X3) of the d <= 4 entry points needs d <= 3 and H <= 1024; FP32 takes
+ * d <= 4, H <= 4096.  Outside that, b200vae_icnn_workspace_bytes returns 0 and b200vae_icnn_prepare, _decode_fwd,
+ * _decode_bwd and _decode_bwd_params return B200VAE_EUNSUP. */
 #define B200VAE_PREC_F16X3 4
 
 /* Parameters of one module.ICNN(in_channel=d, hidden_channel=H) -- module.py:117-140.
@@ -63,7 +64,7 @@ typedef struct b200vae_icnn_grads {
 } b200vae_icnn_grads;
 
 /* Bytes of caller-owned workspace needed by prepare/fwd/bwd for these sizes. `for_backward`=0
- * sizes it for prepare+fwd only. */
+ * sizes it for prepare+fwd only.  0 for sizes or a precision the entry points refuse. */
 size_t b200vae_icnn_workspace_bytes(int B, int d, int H, int precision, int for_backward);
 
 /* Materialise the positive weights P = exp(W) | clamp(W,1e-2) (module.py:110/114) and the padded,

@@ -43,8 +43,8 @@ def test_dp0_generator_stores_are_bank_conflict_free():
 
 
 def test_k_major_sw64_offsets_cover_the_tile_once():
-    """K-major operand tiles of the forward / backward kernels (tc_common.cuh sw64_off): 64-byte rows, 16-byte chunk c of
-    row r at r*64 + ((c ^ ((r >> 1) & 3)) << 4); generator thread (rb, c) of icnn_tc3_fwd_kernel writes rows rb + 32 j."""
+    """K-major SWIZZLE_64B operand tiles of the forward / backward pair kernels (icnn_tc3.cu): 64-byte rows, 16-byte chunk c
+    of row r at r*64 + ((c ^ ((r >> 1) & 3)) << 4); generator thread (rb, c) of icnn_tc3_fwd_kernel writes rows rb + 32 j."""
     sw64 = lambda r, c: r * 64 + ((c ^ ((r >> 1) & 3)) << 4)
     offs = sorted(sw64(r, c) for r in range(128) for c in range(4))
     assert offs == list(range(0, 128 * 64, 16))

@@ -36,7 +36,6 @@ if __name__ == "__main__":
     precs = (4, 3, 1) if fwd_only else (0, 4, 3, 1)
     if "--precs" in sys.argv:
         precs = tuple(int(x) for x in sys.argv[sys.argv.index("--precs") + 1].split(","))
-    print("B200VAE_FWD =", os.environ.get("B200VAE_FWD", "3"))
     for prec in precs:
         for (d, H, B, regime) in ((2, 256, 256, "mixed"), (2, 96, 77, "mixed"), (3, 512, 1000, "mixed"), (2, 1024, 4096, "mixed"), (2, 1024, 512, "default")):
             run(d, H, B, regime, prec)

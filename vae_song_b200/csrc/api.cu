@@ -1,10 +1,8 @@
 // api.cu -- extern "C" entry points of libb200vae.so for the ICNN path (validation + dispatch).
-#include <cstdlib>
 #include <mutex>
 #include <unordered_map>
 
-#include "common.cuh"
-#include "tc_common.cuh"
+#include "icnn.cuh"
 
 namespace b200vae {
 int g_last_cuda_error = 0;
@@ -20,23 +18,6 @@ int sm_count() {
   return n;
 }
 
-int simt_prepare(const b200vae_icnn_params* p, int d, int H, int mode, float* ws, cudaStream_t st);
-int simt_fwd(const float* z, int B, int d, int H, float kappa, float* psi, float* xhat, uint32_t* mask1,
-             uint8_t* mask2, const float* ws, cudaStream_t st);
-int simt_bwd(const float* z, const float* v, const float* gpsi, const uint32_t* mask1, const uint8_t* mask2,
-             int B, int d, int H, const b200vae_icnn_params* p, int mode, float kappa,
-             const b200vae_icnn_grads* g, float* dz, float* ws, size_t mid_extra, cudaStream_t st);
-// tensor-core (tcgen05) variants, icnn_tc.cu
-int tc_prepare(const b200vae_icnn_params* p, int d, int H, int mode, int precision, float* ws, cudaStream_t st);
-int tc3_prepare(int d, int H, int precision, float* ws, cudaStream_t st);
-int tc3_fwd(const float* z, int B, int d, int H, float kappa, float* psi, float* xhat, uint32_t* mask1, uint8_t* mask2,
-            int precision, float* ws, float* accsave, cudaStream_t st);
-size_t tc_extra_ws_floats(int B, int d, int H, int precision);
-size_t tc_bwd_ws_floats(int B, int d, int H);
-int tc_bwd(const float* z, const float* v, const uint32_t* mask1, const uint8_t* mask2, int B, int d, int H,
-           const b200vae_icnn_params* p, int mode, float kappa, const b200vae_icnn_grads* g, float* dz, int precision,
-           float* ws, const float* accsave, int phase, cudaStream_t st);
-
 // ---- saved GEMM2 accumulators (training, 3xTF32) ------------------------------------------------------------------------
 // With a for_backward workspace and both masks requested, the pair forward kernel also stores its GEMM2 accumulators
 // (gx1 / s2, [Bp][Hq] fp32) at the end of the workspace; the backward then skips recomputing that GEMM (icnn_tc3.cu, SV
@@ -46,10 +27,6 @@ int tc_bwd(const float* z, const float* v, const uint32_t* mask1, const uint8_t*
 struct SavedAcc { const void* z; int B, d, H; };
 static std::mutex g_save_mu;
 static std::unordered_map<const void*, SavedAcc> g_saved;
-static bool save_enabled() {
-  static const bool on = [] { const char* e = getenv("B200VAE_SAVE_GX1"); return !e || atoi(e) != 0; }();
-  return on;
-}
 static void save_forget(const void* ws) {
   std::lock_guard<std::mutex> lk(g_save_mu);
   g_saved.erase(ws);
@@ -64,42 +41,80 @@ static bool save_matches(const void* ws, const void* z, int B, int d, int H) {
   auto it = g_saved.find(ws);
   return it != g_saved.end() && it->second.z == z && it->second.B == B && it->second.d == d && it->second.H == H;
 }
-static size_t bwd_floats_without_save(int B, int d, int H, int precision) {
-  const size_t extra = (precision != B200VAE_PREC_FP32) ? tc_extra_ws_floats(B, d, H, precision) : 0;
-  const WsLayout L = ws_layout(B, d, H, extra);
-  return (L.end + (extra ? tc_bwd_ws_floats(B, d, H) : 0) + 63) / 64 * 64;
+
+// ---- workspace layout (icnn.cuh) ----------------------------------------------------------------------------------------
+static int bwd_splits(int B, int Hp) {
+  // output-stationary dP0 kernel of the FP32 path: (Hp/128)^2 tiles x splits CTAs; aim for >= ~3 waves of 148 SMs
+  int tiles = (Hp / 128) * (Hp / 128);
+  int want = (148 * 3 + tiles - 1) / tiles;
+  int maxs = (B + 127) / 128;          // at least one 128-row slab per split
+  int s = want < maxs ? want : maxs;
+  if (s < 1) s = 1;
+  if (s > 64) s = 64;
+  return s;
 }
-static size_t accsave_floats(int B, int d, int H, int precision) {
-  if ((precision != B200VAE_PREC_TF32X3 && precision != B200VAE_PREC_F16X3) || d > 3 || !save_enabled()) return 0;
-  const Tc3Layout T3 = tc3_layout(B, d, H);
-  return (size_t)T3.Bp * T3.Hq + 64;
+
+WsLayout icnn_ws_layout(int B, int d, int H, int precision, bool for_backward) {
+  WsLayout L = {};
+  L.B = B; L.d = d; L.H = H;
+  L.Hp = round_up(H, 128); L.Hq = round_up(H, 256); L.K1 = L.Hq + 16; L.NP = L.Hq / 256; L.Bp = round_up(B, 256);
+  L.n_mtiles = (B + 127) / 128;
+  L.splits = bwd_splits(B, L.Hp);
+  const size_t Hp = L.Hp, Hq = L.Hq, Bp = L.Bp, NP = L.NP, tiles = Bp / 256;
+  const bool tc = precision != B200VAE_PREC_FP32;
+  size_t o = 0;
+  auto take = [&o](size_t n) { const size_t at = o; o += (n + 63) / 64 * 64; return at; };   // 256 B aligned regions
+  L.P0 = take(Hp * Hp);
+  L.P0T = take(Hp * Hp);
+  L.P1 = take(Hp);
+  L.A0p = take(Hp * (d + 1));
+  L.A1p = take(Hp * (d + 1));
+  L.A2p = take(16 > d + 1 ? 16 : d + 1);
+  if (tc) {
+    L.A0q = take(4 * Hq); L.A1q = take(4 * Hq); L.P1q = take(Hq);
+    L.B1ahi = take(Hq * L.K1); L.B1alo = take(Hq * L.K1); L.B2ghi = take(Hq * Hq); L.B2glo = take(Hq * Hq);
+    L.A0g = take(4 * Hq); L.E1 = take(4 * Hq); L.sumV = take(64); L.cnt = take(2 * kTc3MaxTiles);
+    L.scr1 = take(Bp * NP * 2 * 4); L.scr2 = take(Bp * NP * 2 * 4); L.imask = take(Bp * (Hq / 32));
+    const size_t units = 2 * tiles * NP;
+    L.cscr = take((units < (size_t)kTc3MaxClusters ? units : (size_t)kTc3MaxClusters) * 2 * k3ScrFloatsPerCta);
+  }
+  if (for_backward) {
+    L.colpart = take((size_t)L.n_mtiles * Hp * (2 * d + 3));
+    L.a2part = take((size_t)L.n_mtiles * (d + 1));
+    L.dP0part = take((size_t)L.splits * Hp * Hp);
+    if (tc) {
+      L.dp0_splits = dp0_splits(B, L.Hq, sm_count() / 2);
+      L.partA = take(tiles * 8 * (d + 1) * Hq); L.partB = take(tiles * 8 * (d + 1) * Hq);
+      L.a2part_tc = take(tiles * d);
+      L.dP0part_tc = take((size_t)L.dp0_splits * Hq * Hq);
+      L.dzpart = take(Bp * NP * 2 * 4);
+      if (precision == B200VAE_PREC_TF32X3 || precision == B200VAE_PREC_F16X3) L.accsave = take(Bp * Hq);
+    }
+  }
+  L.end = o;
+  return L;
 }
+static size_t ws_bytes_of(const WsLayout& L) { return L.end * sizeof(float) + 256; }   // + alignment of the base
 
 static bool params_ok(const b200vae_icnn_params* p) {
   return p && p->A0w && p->A0b && p->A1w && p->A1b && p->A2w && p->A2b && p->W0 && p->W1 && aligned4(p->A0w) &&
          aligned4(p->W0);
 }
-static int shape_ok(int B, int d, int H) {
+// every entry point's shape / precision check: FP32 takes d <= 4, H <= 4096; the tensor-core precisions d <= 3, H <= 1024
+static int shape_ok(int B, int d, int H, int precision) {
   if (B <= 0 || d <= 0 || H <= 0) return B200VAE_ESHAPE;
-  if (d > 4) return B200VAE_EUNSUP;      // fused small-d path; wider inputs go through the tiled path
-  if (H > 4096) return B200VAE_EUNSUP;
-  return B200VAE_OK;
-}
-static bool prec_ok(int precision) {
-  return precision == B200VAE_PREC_FP32 || precision == B200VAE_PREC_TF32 || precision == B200VAE_PREC_TF32X3 ||
-         precision == B200VAE_PREC_F16X3;   // 2 is reserved
+  if (precision == B200VAE_PREC_FP32) return (d <= 4 && H <= 4096) ? B200VAE_OK : B200VAE_EUNSUP;
+  if (precision != B200VAE_PREC_TF32 && precision != B200VAE_PREC_TF32X3 && precision != B200VAE_PREC_F16X3)
+    return B200VAE_EUNSUP;                                     // 2 is reserved
+  return (d <= 3 && round_up(H, 256) <= kTc3MaxHq) ? B200VAE_OK : B200VAE_EUNSUP;
 }
 }  // namespace b200vae
 
 using namespace b200vae;
 
 extern "C" size_t b200vae_icnn_workspace_bytes(int B, int d, int H, int precision, int for_backward) {
-  if (B <= 0 || d <= 0 || H <= 0) return 0;
-  const size_t extra = (precision != B200VAE_PREC_FP32) ? tc_extra_ws_floats(B, d, H, precision) : 0;
-  const WsLayout L = ws_layout(B, d, H, extra);
-  const size_t fl = for_backward ? bwd_floats_without_save(B, d, H, precision) + accsave_floats(B, d, H, precision)
-                                 : L.fwd_end + extra + 64;
-  return fl * sizeof(float) + 256;
+  if (shape_ok(B, d, H, precision)) return 0;
+  return ws_bytes_of(icnn_ws_layout(B, d, H, precision, for_backward != 0));
 }
 
 static float* ws_base(const void* ws) {
@@ -108,18 +123,16 @@ static float* ws_base(const void* ws) {
 
 extern "C" int b200vae_icnn_prepare(const b200vae_icnn_params* p, int d, int H, int weight_mode, int precision,
                                     void* ws, size_t ws_bytes, void* stream) {
+  int rc = shape_ok(1, d, H, precision);
+  if (rc) return rc;
   if (!params_ok(p) || !ws) return B200VAE_EALIGN;
-  int rc = shape_ok(1, d, H);
-  if (rc) return rc;
   if (weight_mode != B200VAE_WEIGHT_EXP && weight_mode != B200VAE_WEIGHT_CLAMP) return B200VAE_EUNSUP;
-  if (!prec_ok(precision)) return B200VAE_EUNSUP;
-  if (ws_bytes < b200vae_icnn_workspace_bytes(1, d, H, precision, 0)) return B200VAE_EWS;
+  const WsLayout L = icnn_ws_layout(1, d, H, precision, false);    // prepare writes only regions that do not depend on B
+  if (ws_bytes < ws_bytes_of(L)) return B200VAE_EWS;
   save_forget(ws_base(ws));
-  rc = simt_prepare(p, d, H, weight_mode, ws_base(ws), (cudaStream_t)stream);
+  rc = simt_prepare(p, L, weight_mode, ws_base(ws), (cudaStream_t)stream);
   if (rc || precision == B200VAE_PREC_FP32) return rc;
-  rc = tc_prepare(p, d, H, weight_mode, precision, ws_base(ws), (cudaStream_t)stream);
-  if (rc) return rc;
-  return tc3_prepare(d, H, precision, ws_base(ws), (cudaStream_t)stream);
+  return tc3_prepare(L, precision, ws_base(ws), (cudaStream_t)stream);
 }
 
 extern "C" int b200vae_icnn_decode_fwd(const float* z, int B, int d, int H, int weight_mode, float kappa, float* psi,
@@ -127,19 +140,16 @@ extern "C" int b200vae_icnn_decode_fwd(const float* z, int B, int d, int H, int 
                                        size_t ws_bytes, void* stream) {
   (void)weight_mode;
   if (!z || !ws || !aligned4(z)) return B200VAE_EALIGN;
-  int rc = shape_ok(B, d, H);
+  int rc = shape_ok(B, d, H, precision);
   if (rc) return rc;
-  if (!prec_ok(precision)) return B200VAE_EUNSUP;
   if (ws_bytes < b200vae_icnn_workspace_bytes(B, d, H, precision, 0)) return B200VAE_EWS;
+  const WsLayout L = icnn_ws_layout(B, d, H, precision, true);     // the forward's regions sit where they do without backward
   if (precision == B200VAE_PREC_FP32)
-    return simt_fwd(z, B, d, H, kappa, psi, xhat, mask1, mask2, ws_base(ws), (cudaStream_t)stream);
-  // persistent CTA pairs (icnn_tc3.cu); B200VAE_EUNSUP where they do not take the shape (d > 3, H > 1024)
+    return simt_fwd(z, L, kappa, psi, xhat, mask1, mask2, ws_base(ws), (cudaStream_t)stream);
   float* accsave = nullptr;
-  if (mask1 && mask2 && xhat && accsave_floats(B, d, H, precision) &&
-      ws_bytes >= b200vae_icnn_workspace_bytes(B, d, H, precision, 1))
-    accsave = ws_base(ws) + bwd_floats_without_save(B, d, H, precision);
+  if (mask1 && mask2 && xhat && L.accsave && ws_bytes >= ws_bytes_of(L)) accsave = ws_base(ws) + L.accsave;
   save_forget(ws_base(ws));
-  rc = tc3_fwd(z, B, d, H, kappa, psi, xhat, mask1, mask2, precision, ws_base(ws), accsave, (cudaStream_t)stream);
+  rc = tc3_fwd(z, L, kappa, psi, xhat, mask1, mask2, precision, ws_base(ws), accsave, (cudaStream_t)stream);
   if (rc == B200VAE_OK && accsave) save_record(ws_base(ws), z, B, d, H);
   return rc;
 }
@@ -150,20 +160,17 @@ extern "C" int b200vae_icnn_decode_bwd(const float* z, const float* v, const flo
                                        int precision, void* ws, size_t ws_bytes, void* stream) {
   if (!z || !mask1 || !mask2 || !ws || !params_ok(p)) return B200VAE_EALIGN;
   if (!v && !gpsi) return B200VAE_ESHAPE;
-  int rc = shape_ok(B, d, H);
+  int rc = shape_ok(B, d, H, precision);
   if (rc) return rc;
-  if (!prec_ok(precision)) return B200VAE_EUNSUP;
-  if (ws_bytes < b200vae_icnn_workspace_bytes(B, d, H, precision, 1)) return B200VAE_EWS;
+  const WsLayout L = icnn_ws_layout(B, d, H, precision, true);
+  if (ws_bytes < ws_bytes_of(L)) return B200VAE_EWS;
   if (precision != B200VAE_PREC_FP32 && !gpsi) { // tensor-core backward (gpsi path stays on the FP32 kernels)
     const float* accsave = nullptr;
-    if (accsave_floats(B, d, H, precision) && save_matches(ws_base(ws), z, B, d, H))
-      accsave = ws_base(ws) + bwd_floats_without_save(B, d, H, precision);
-    return tc_bwd(z, v, mask1, mask2, B, d, H, p, weight_mode, kappa, grads, dz, precision, ws_base(ws), accsave, 0,
+    if (L.accsave && save_matches(ws_base(ws), z, B, d, H)) accsave = ws_base(ws) + L.accsave;
+    return tc_bwd(z, v, mask1, mask2, L, p, weight_mode, kappa, grads, dz, precision, ws_base(ws), accsave, 0,
                   (cudaStream_t)stream);
   }
-  const size_t extra = (precision != B200VAE_PREC_FP32) ? tc_extra_ws_floats(B, d, H, precision) : 0;
-  return simt_bwd(z, v, gpsi, mask1, mask2, B, d, H, p, weight_mode, kappa, grads, dz, ws_base(ws), extra,
-                  (cudaStream_t)stream);
+  return simt_bwd(z, v, gpsi, mask1, mask2, L, p, weight_mode, kappa, grads, dz, ws_base(ws), (cudaStream_t)stream);
 }
 
 extern "C" int b200vae_icnn_decode_bwd_params(const float* z, const float* v, const uint32_t* mask1, const uint8_t* mask2,
@@ -171,11 +178,12 @@ extern "C" int b200vae_icnn_decode_bwd_params(const float* z, const float* v, co
                                               const b200vae_icnn_grads* grads, int precision, void* ws, size_t ws_bytes,
                                               void* stream) {
   if (!z || !v || !mask1 || !mask2 || !ws || !grads || !params_ok(p)) return B200VAE_EALIGN;
-  int rc = shape_ok(B, d, H);
+  int rc = shape_ok(B, d, H, precision);
   if (rc) return rc;
-  if (!prec_ok(precision) || precision == B200VAE_PREC_FP32) return B200VAE_EUNSUP;
-  if (ws_bytes < b200vae_icnn_workspace_bytes(B, d, H, precision, 1)) return B200VAE_EWS;
-  return tc_bwd(z, v, mask1, mask2, B, d, H, p, weight_mode, 0.f, grads, nullptr, precision, ws_base(ws), nullptr, 2,
+  if (precision == B200VAE_PREC_FP32) return B200VAE_EUNSUP;
+  const WsLayout L = icnn_ws_layout(B, d, H, precision, true);
+  if (ws_bytes < ws_bytes_of(L)) return B200VAE_EWS;
+  return tc_bwd(z, v, mask1, mask2, L, p, weight_mode, 0.f, grads, nullptr, precision, ws_base(ws), nullptr, 2,
                 (cudaStream_t)stream);
 }
 

@@ -29,61 +29,6 @@ inline bool aligned4(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 3
 
 int sm_count();
 
-// ---- workspace layout of the prepared (padded, kernel-layout) ICNN parameters -------------------
-// All offsets in floats from the (256 B aligned) workspace base.  Hp = H rounded up to 128.
-//   P0   [Hp,Hp]  P0[k][n] = positive(W0)[k][n]                (B operand of  gx1 = g1 . P0)
-//   P0T  [Hp,Hp]  P0T[n][k] = P0[k][n]                         (B operand of  h1  = x1 . P0^T)
-//   P1   [Hp]
-//   A0p  [Hp][d+1]  (A0w[n][0..d-1], A0b[n])
-//   A1p  [Hp][d+1]  (A1w[n][0..d-1], A1b[n])
-//   A2p  [d+1]      (A2w[0][0..d-1], A2b[0])     (padded to 16 floats)
-// backward scratch follows (see icnn_simt.cu).
-struct WsLayout {
-  int d, H, Hp;
-  size_t P0, P0T, P1, A0p, A1p, A2p, fwd_end;
-  // backward
-  int n_mtiles, splits;
-  size_t colpart;   // [n_mtiles][Hp][2d+3]  per-CTA column partials: dA0w(d) dA0b dA1w(d) dP1 (+1 pad)
-  size_t a2part;    // [n_mtiles][d+1]
-  size_t dP0part;   // [splits][Hp][Hp]
-  size_t end;
-};
-
-inline int bwd_splits(int B, int Hp) {
-  // output-stationary dP0 kernel: (Hp/128)^2 tiles x splits CTAs; aim for >= ~3 waves of 148 SMs
-  int tiles = (Hp / 128) * (Hp / 128);
-  int want = (148 * 3 + tiles - 1) / tiles;
-  int maxs = (B + 127) / 128;          // at least one 128-row slab per split
-  int s = want < maxs ? want : maxs;
-  if (s < 1) s = 1;
-  if (s > 64) s = 64;
-  return s;
-}
-
-// `mid_extra` floats (the tensor-core operand copies, icnn_tc.cu) sit between the forward arrays and the backward scratch
-inline WsLayout ws_layout(int B, int d, int H, size_t mid_extra = 0) {
-  WsLayout L;
-  L.d = d; L.H = H; L.Hp = round_up(H, 128);
-  size_t Hp = (size_t)L.Hp;
-  auto up = [](size_t x) { return (x + 63) / 64 * 64; };   // keep every array 256 B aligned
-  size_t o = 0;
-  L.P0 = o; o += up(Hp * Hp);
-  L.P0T = o; o += up(Hp * Hp);
-  L.P1 = o; o += up(Hp);
-  L.A0p = o; o += up(Hp * (d + 1));
-  L.A1p = o; o += up(Hp * (d + 1));
-  L.A2p = o; o += up(16 > d + 1 ? 16 : d + 1);
-  L.fwd_end = o;
-  o += up(mid_extra);
-  L.n_mtiles = (B + 127) / 128;
-  L.splits = bwd_splits(B, L.Hp);
-  L.colpart = o; o += up((size_t)L.n_mtiles * Hp * (2 * d + 3));
-  L.a2part = o; o += up((size_t)L.n_mtiles * (d + 1));
-  L.dP0part = o; o += up((size_t)L.splits * Hp * Hp);
-  L.end = o;
-  return L;
-}
-
 // ---- device helpers -------------------------------------------------------------------------------
 __device__ __forceinline__ float slope_of(float h) { return h > 0.f ? 1.f : kSlope; }
 

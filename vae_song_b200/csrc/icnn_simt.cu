@@ -5,7 +5,7 @@
 // model.py:820-822 / 826-828 (psi + kappa|z|^2 and autograd.grad -> xhat) and the autograd
 // double-backward those create (lipschitz.py:41).
 //
-// Kernels (all operate on the PREPARED workspace, see common.cuh::WsLayout):
+// Kernels (all operate on the PREPARED workspace, see icnn.cuh::WsLayout):
 //   prepare_kernel        P0 = positive(W0) (+ transpose), P1, packed/padded A0,A1,A2
 //   icnn_fwd_kernel<D>    one CTA = 128 samples: GEMM1 h1 = x1.P0^T (+A1 z+b1) -> mask bits, h2 -> psi;
 //                         GEMM2 gx1 = g1.P0 -> g0 -> xhat.   Nothing but z, psi, xhat, masks touches HBM.
@@ -15,6 +15,7 @@
 //   finalize kernels      fixed-order reduction of the partials + chain through exp / clamp
 // All reductions are ordered (no float atomics): results are bit-reproducible run to run.
 #include "gemm_simt.cuh"
+#include "icnn.cuh"
 
 namespace b200vae {
 
@@ -722,35 +723,6 @@ static int launch_bwd(const float* z, const float* v, const float* gpsi, const u
   return rc;
 }
 
-template <int D>
-static int launch_dP0_only(const float* z, const float* v, const uint32_t* mask1, const uint8_t* mask2, int B,
-                           const WsLayout& L, float* ws, cudaStream_t st) {
-  int rows = (B + L.splits - 1) / L.splits;
-  rows = round_up(rows, kBK);
-  dim3 grid(L.Hp / kBN, L.Hp / kBM, L.splits);
-  icnn_bwd_dP0_kernel<D, false><<<grid, kThreads, 0, st>>>(z, v, nullptr, mask1, mask2, B, L.Hp, rows, ws + L.A0p,
-                                                            ws + L.dP0part);
-  return check_launch();
-}
-
-// dW0 only (FP32 SIMT): used by the tensor-core backward until its own dP0 kernel takes over
-int simt_bwd_W0(const float* z, const float* v, const uint32_t* mask1, const uint8_t* mask2, int B, int d, int H,
-                const b200vae_icnn_params* p, int mode, float* gW0, float* ws, size_t mid_extra, cudaStream_t st) {
-  const WsLayout L = ws_layout(B, d, H, mid_extra);
-  int rc;
-  switch (d) {
-    case 1: rc = launch_dP0_only<1>(z, v, mask1, mask2, B, L, ws, st); break;
-    case 2: rc = launch_dP0_only<2>(z, v, mask1, mask2, B, L, ws, st); break;
-    case 3: rc = launch_dP0_only<3>(z, v, mask1, mask2, B, L, ws, st); break;
-    case 4: rc = launch_dP0_only<4>(z, v, mask1, mask2, B, L, ws, st); break;
-    default: return B200VAE_EUNSUP;
-  }
-  if (rc) return rc;
-  dim3 grid((H + 255) / 256, H);
-  finalize_W0_kernel<<<grid, 256, 0, st>>>(ws + L.dP0part, L.splits, H, L.Hp, L.Hp, ws + L.P0, ws + L.P1, p->W0, mode, 1.f, gW0);
-  return check_launch();
-}
-
 int finalize_W0_launch(const float* part, int splits, int H, int Hp, int ldp, const float* P0, const float* P1,
                        const float* W0raw, int mode, float scale, float* dW0, cudaStream_t st) {
   dim3 grid((H + 255) / 256, H);
@@ -758,18 +730,17 @@ int finalize_W0_launch(const float* part, int splits, int H, int Hp, int ldp, co
   return check_launch();
 }
 
-int simt_prepare(const b200vae_icnn_params* p, int d, int H, int mode, float* ws, cudaStream_t st) {
-  const WsLayout L = ws_layout(128, d, H);
+int simt_prepare(const b200vae_icnn_params* p, const WsLayout& L, int mode, float* ws, cudaStream_t st) {
   dim3 grid(L.Hp / 32, L.Hp / 32), block(32, 8);
-  prepare_kernel<<<grid, block, 0, st>>>(p->W0, p->W1, p->A0w, p->A0b, p->A1w, p->A1b, p->A2w, p->A2b, d, H, L.Hp,
+  prepare_kernel<<<grid, block, 0, st>>>(p->W0, p->W1, p->A0w, p->A0b, p->A1w, p->A1b, p->A2w, p->A2b, L.d, L.H, L.Hp,
                                          mode, ws + L.P0, ws + L.P0T, ws + L.P1, ws + L.A0p, ws + L.A1p, ws + L.A2p);
   return check_launch();
 }
 
-int simt_fwd(const float* z, int B, int d, int H, float kappa, float* psi, float* xhat, uint32_t* mask1,
-             uint8_t* mask2, const float* ws, cudaStream_t st) {
-  const WsLayout L = ws_layout(B, d, H);
-  switch (d) {
+int simt_fwd(const float* z, const WsLayout& L, float kappa, float* psi, float* xhat, uint32_t* mask1, uint8_t* mask2,
+             const float* ws, cudaStream_t st) {
+  const int B = L.B;
+  switch (L.d) {
     case 1: return launch_fwd<1>(z, B, L, ws, kappa, psi, xhat, mask1, mask2, st);
     case 2: return launch_fwd<2>(z, B, L, ws, kappa, psi, xhat, mask1, mask2, st);
     case 3: return launch_fwd<3>(z, B, L, ws, kappa, psi, xhat, mask1, mask2, st);
@@ -778,10 +749,10 @@ int simt_fwd(const float* z, int B, int d, int H, float kappa, float* psi, float
   }
 }
 
-int simt_bwd(const float* z, const float* v, const float* gpsi, const uint32_t* mask1, const uint8_t* mask2,
-             int B, int d, int H, const b200vae_icnn_params* p, int mode, float kappa,
-             const b200vae_icnn_grads* g, float* dz, float* ws, size_t mid_extra, cudaStream_t st) {
-  const WsLayout L = ws_layout(B, d, H, mid_extra);
+int simt_bwd(const float* z, const float* v, const float* gpsi, const uint32_t* mask1, const uint8_t* mask2, const WsLayout& L,
+             const b200vae_icnn_params* p, int mode, float kappa, const b200vae_icnn_grads* g, float* dz, float* ws,
+             cudaStream_t st) {
+  const int B = L.B, d = L.d, H = L.H;
   const bool need_W0 = g && g->W0;
   int rc;
 #define B200VAE_BWD(DD)                                                                                   \

@@ -17,12 +17,12 @@
 //     through an L2-resident scratch; a per-(tile, rank) counter orders GEMM2 after GEMM1 and elects the last
 //     unit of a tile to combine the partials in a FIXED order (bit-reproducible, no float atomics).
 // Reference lines replaced: module.py:142-148 (ICNN.forward) and model.py:820-822 / 826-828 (grad of psi).
-#include <cstdlib>
 #include <mutex>
 #include <unordered_map>
 
 #include <cuda_fp16.h>
 
+#include "icnn.cuh"
 #include "tc_common.cuh"
 
 namespace b200vae {
@@ -44,8 +44,9 @@ constexpr int k3Rows = 128;                       // sample rows per CTA
 constexpr int k3Threads = 18 * 32;                // 8 epilogue warps, 8 generator warps, TMA warp, MMA warp
 constexpr int k3TileBytes = k3Rows * 64;          // 128 rows x 64 B = 8 KB (A tile, and this CTA's half of a B tile)
 constexpr int k3MaskStride = 36;                  // words per row of the shared mask buffer (16 B aligned, conflict free)
-constexpr int kTc3MaxHq = 1024;                   // a mask row must fit the buffer (Hq / 32 <= 36, Hq a multiple of 256): wider
-                                                  // ICNNs are refused (B200VAE_EUNSUP): FP32 kernels only
+static_assert(kTc3MaxHq / 32 <= k3MaskStride, "a row of mask bits must fit the shared mask buffer");
+constexpr int kTc3ChunkK = 512;                   // K per accumulation chunk of the hi/lo modes (WsLayout::cscr, icnn.cuh)
+constexpr uint32_t k3ParkNs = 2000;               // suspend-time hint of the epilogue warps' accumulator waits
 constexpr uint32_t k3Idesc = (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)(256 >> 3) << 17) | ((uint32_t)(256 >> 4) << 24);
 
 __device__ __forceinline__ uint32_t cluster_rank3() {
@@ -290,8 +291,8 @@ struct alignas(64) Tc3Args {
   CUtensorMap b1hi, b1lo, b2hi, b2lo;             // boxes of 16 x 128 (this CTA's half of a 256-row B tile)
   const float* z;
   const float4 *A0g, *E1, *A0q;
-  const float4* A1q;                              // FP16 mode: (A1w0, A1w1, A1w2 | spare, A1b) per unit (TcLayout::A1q)
-  const float* P1q;                               // FP16 mode: P1 per unit (TcLayout::P1q)
+  const float4* A1q;                              // FP16 mode: (A1w0, A1w1, A1w2 | spare, A1b) per unit (WsLayout::A1q)
+  const float* P1q;                               // FP16 mode: P1 per unit (WsLayout::P1q)
   const float *sumV, *A2p;                        // sumV[16..19] = (s1, 1/s1, s2, 1/s2), sumV[24..27] = max |A0| (FP16 mode)
   float *psi, *xhat;
   uint32_t* maskg;                                // mask1 of the caller or the internal scratch (null: psi-only, no masks)
@@ -303,10 +304,9 @@ struct alignas(64) Tc3Args {
                                                   // rows] (k3SaveBlock): the TMEM-native order, so that a warp's store of one
                                                   // column is ONE 128-byte line (row-major rows made every 256-bit store touch 32
                                                   // lines: a quarter of the LSU's time during a GEMM2 unit)
-  float4* cscr;                                   // K-chunk running sums (Tc3Layout::cscr), used when NC > 1
+  float4* cscr;                                   // K-chunk running sums (WsLayout::cscr), used when NC > 1
   int B, Hq, T, NP, mask_stride, mask_rows, want_x;
   int NC;                                         // K-chunks per unit (hi/lo modes: Hq / kTc3ChunkK; 1 = plain accumulation)
-  uint32_t park_ns;                               // suspend-time hint of the epilogue warps' accumulator waits
   float kappa;
 };
 
@@ -324,11 +324,14 @@ struct Tc3Cfg {
   static constexpr int kOffAlo = k3TileBytes, kOffB = (HL ? 2 : 1) * k3TileBytes, kOffBlo = 3 * k3TileBytes;
 };
 template <int MODE>
-static size_t tc3_smem_bytes(int Hq) {
+constexpr size_t tc3_smem_bytes(int Hq) {
   using C = Tc3Cfg<MODE>;
   return (size_t)C::S * C::kStageBytes + (size_t)Hq * (C::F16 ? 52 : 48) + 2 * k3Rows * k3MaskStride * 4 + (2 * C::S + 4) * 8 +
          64 + 1024;
 }
+static_assert(tc3_smem_bytes<kTf32>(kTc3MaxHq) <= 227 * 1024 && tc3_smem_bytes<kX3>(kTc3MaxHq) <= 227 * 1024 &&
+                  tc3_smem_bytes<kF16>(kTc3MaxHq) <= 227 * 1024,
+              "pair kernels: the per-unit tables of every mode fit in shared memory up to kTc3MaxHq");
 
 struct Unit { int g, t, p; };
 __device__ __forceinline__ Unit decode_unit(int u, int T, int NP) {
@@ -412,7 +415,7 @@ icnn_tc3_fwd_kernel(const __grid_constant__ Tc3Args a) {
       const int nck = un.g ? 1 : NC;
       for (int ck = 0; ck + 1 < nck; ++ck, ++i) {
         const int pbuf = i & 1;
-        mbar_wait_parked(accfull0 + 8 * pbuf, (i >> 1) & 1, a.park_ns);
+        mbar_wait_parked(accfull0 + 8 * pbuf, (i >> 1) & 1, k3ParkNs);
         tc_fence_after();
 #pragma unroll 1
         for (int cc = 0; cc < 4; ++cc) {
@@ -456,7 +459,7 @@ icnn_tc3_fwd_kernel(const __grid_constant__ Tc3Args a) {
         row_scale_x1<D>(zr, amax, t_r, inv_x);
         cinv = inv_x * inv_s1;
       }
-      mbar_wait_parked(accfull0 + 8 * buf, (i >> 1) & 1, a.park_ns);
+      mbar_wait_parked(accfull0 + 8 * buf, (i >> 1) & 1, k3ParkNs);
       tc_fence_after();
       // r = TMEM accumulator columns [32 cc, 32 cc + 32) of my row (+ the running sums of the earlier chunks)
       auto load_acc = [&](uint32_t (&r)[32], int cc) {
@@ -920,7 +923,7 @@ icnn_tc3_fwd_kernel(const __grid_constant__ Tc3Args a) {
 // of every 32-column chunk, so per-column parameters are loaded once per 4 rows and a column sum needs 3 in-thread
 // adds plus a 3-step transposing shuffle reduction over the 8 lanes that share the columns (instead of 5 steps over
 // 32 lanes).  Column partials go to ordered slots part[(tile*8 + rank*4 + quarter)][f][Hq] (summed in fixed order by
-// tc_finalize_small_kernel, icnn_tc.cu); dz partials per (row, pass, column half) are combined by tc3_bwd_dz_kernel.
+// tc_finalize_small_kernel); dz partials per (row, pass, column half) are combined by tc3_bwd_dz_kernel.
 struct alignas(64) Tc3BwdArgs {
   CUtensorMap b1hi, b1lo, b2hi, b2lo;
   const float *z, *v;
@@ -1081,7 +1084,7 @@ icnn_tc3_bwd_kernel(const __grid_constant__ Tc3BwdArgs a) {
           s2x2p[pr] = __fmul2_rn(s2p[pr], make_float2(k2, k2));
         }
         if (!from_global) {
-          mbar_wait_parked(accfull0 + 8 * buf, (i >> 1) & 1, 2000);
+          mbar_wait_parked(accfull0 + 8 * buf, (i >> 1) & 1, k3ParkNs);
           tc_fence_after();
         }
 #pragma unroll 1
@@ -1548,14 +1551,84 @@ tc3_bwd_dz_kernel(const float4* __restrict__ dzpart, const float* __restrict__ v
   }
 }
 
+// one thread per hidden unit: (A0w, A0b), (A1w | P1 in the spare lane, A1b), P1 in natural unit order, zero padded to Hq
+__global__ void tc_prepare_kernel(const float* __restrict__ P1, const float* __restrict__ A0p, const float* __restrict__ A1p,
+                                  int d, int Hp, int Hq, float4* __restrict__ A0q, float4* __restrict__ A1q,
+                                  float* __restrict__ P1q) {
+  const int c = blockIdx.x * blockDim.x + threadIdx.x;
+  if (c >= Hq) return;
+  const bool inr = c < Hp;
+  float w[4] = {0.f, 0.f, 0.f, 0.f}, u[4] = {0.f, 0.f, 0.f, 0.f};
+  if (inr) {
+    for (int j = 0; j < d; ++j) { w[j] = A0p[(size_t)c * (d + 1) + j]; u[j] = A1p[(size_t)c * (d + 1) + j]; }
+    w[3] = A0p[(size_t)c * (d + 1) + d]; u[3] = A1p[(size_t)c * (d + 1) + d];
+  }
+  if (d <= 2) u[2] = inr ? P1[c] : 0.f;     // spare lane of the float4: P1 rides along
+  A0q[c] = make_float4(w[0], w[1], w[2], w[3]);
+  A1q[c] = make_float4(u[0], u[1], u[2], u[3]);
+  P1q[c] = inr ? P1[c] : 0.f;
+}
+
+// ordered reduction of the row-kernel partials + chain through the positive reparam for W1.
+// grid (Hq/32, NF, 2): one block of 1024 threads sums all `nslots` partial rows of 32 columns (32 slot lanes x 32 columns,
+// coalesced 128-byte reads, fixed summation order -> deterministic).
+__global__ void __launch_bounds__(1024)
+tc_finalize_small_kernel(const float* __restrict__ partA, const float* __restrict__ partB,
+                         const float* __restrict__ a2part, int nslots, int nmt, int d, int H, int Hq,
+                         const float* __restrict__ P1, const float* __restrict__ W1raw, int mode, b200vae_icnn_grads g) {
+  __shared__ float red[32][33];
+  const int NF = d + 1;
+  const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;
+  const int n = blockIdx.x * 32 + tx, f = blockIdx.y, which = blockIdx.z;
+  const float* part = (which ? partB : partA) + (size_t)f * Hq + n;
+  // 16 independent partial sums per thread, 32 slot lanes per block: the kernel is latency bound (2048 slots x 128-byte
+  // rows per block at B = 65536), so the number of loads in flight is what sets its duration (8 slot lanes: 21 us)
+  float acc[16];
+#pragma unroll
+  for (int i = 0; i < 16; ++i) acc[i] = 0.f;
+  int sl = ty;
+  const size_t stride = (size_t)NF * Hq;
+  for (; sl + 480 < nslots; sl += 512) {
+#pragma unroll
+    for (int i = 0; i < 16; ++i) acc[i] += part[(size_t)(sl + 32 * i) * stride];
+  }
+  for (; sl < nslots; sl += 32) acc[0] += part[(size_t)sl * stride];
+#pragma unroll
+  for (int w = 8; w >= 1; w >>= 1)
+#pragma unroll
+    for (int i = 0; i < w; ++i) acc[i] += acc[i + w];
+  red[ty][tx] = acc[0];
+  __syncthreads();
+  if (ty == 0 && n < H) {
+    float s = 0.f;
+#pragma unroll
+    for (int q = 0; q < 32; ++q) s += red[q][tx];
+    if (!which) {
+      if (f < d) { if (g.A0w) g.A0w[(size_t)n * d + f] = s; }
+      else if (g.A0b) g.A0b[n] = s;
+    } else {
+      if (f < d) { if (g.A1w) g.A1w[(size_t)n * d + f] = s; }
+      else if (g.W1) g.W1[n] = (mode == B200VAE_WEIGHT_EXP) ? s * P1[n] : (W1raw[n] >= kClampMin ? s : 0.f);
+      if (f == 0 && g.A1b) g.A1b[n] = 0.f;                   // exact zeros on the <v, xhat> path (Appendix A)
+    }
+  }
+  if (blockIdx.x == 0 && blockIdx.y == 0 && blockIdx.z == 0) {
+    if (threadIdx.x < d) {
+      float s = 0.f;
+      for (int mt = 0; mt < nmt; ++mt) s += a2part[(size_t)mt * d + threadIdx.x];
+      if (g.A2w) g.A2w[threadIdx.x] = s;
+    }
+    if (threadIdx.x == 0 && g.A2b) g.A2b[0] = 0.f;
+  }
+}
+
 // ------------------------------------------------------------------------------------ host side
 typedef CUresult (*EncodeTiledFn3)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
                                    const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
                                    CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-// arithmetic of the pair kernels for an ABI precision id: FP16 hi/lo where its tables fit in shared memory (Hq <= 1024)
-static int tc3_mode(int precision, int Hq) {
-  if (precision == B200VAE_PREC_F16X3) return (Hq <= kTc3MaxHq && tc3_smem_bytes<kF16>(Hq) <= (size_t)227 * 1024) ? kF16 : kX3;
-  return precision == B200VAE_PREC_TF32X3 ? kX3 : kTf32;
+// arithmetic of the pair kernels for an ABI precision id
+static int tc3_mode(int precision) {
+  return precision == B200VAE_PREC_F16X3 ? kF16 : precision == B200VAE_PREC_TF32X3 ? kX3 : kTf32;
 }
 static int make_map3(CUtensorMap* m, const float* base, int K, int rows, bool f16 = false) {
   static EncodeTiledFn3 fn = nullptr;
@@ -1578,57 +1651,57 @@ static int make_map3(CUtensorMap* m, const float* base, int K, int rows, bool f1
   return B200VAE_OK;
 }
 
-int tc3_prepare(int d, int H, int precision, float* ws, cudaStream_t st) {
-  if (d > 3) return B200VAE_EUNSUP;
-  const WsLayout L = ws_layout(1, d, H);
-  const TcLayout T = tc_layout(d, H);
-  const Tc3Layout T3 = tc3_layout(1, d, H);
-  float* t3 = tc_base(ws, d, H) + T.end;
-  const int mode = tc3_mode(precision, T3.Hq);
-  int rc;
+// the per-unit tables and the pair kernels' operands, from the FP32 arrays simt_prepare wrote
+int tc3_prepare(const WsLayout& L, int precision, float* ws, cudaStream_t st) {
+  tc_prepare_kernel<<<(L.Hq + 255) / 256, 256, 0, st>>>(ws + L.P1, ws + L.A0p, ws + L.A1p, L.d, L.Hp, L.Hq,
+                                                       reinterpret_cast<float4*>(ws + L.A0q),
+                                                       reinterpret_cast<float4*>(ws + L.A1q), ws + L.P1q);
+  int rc = check_launch();
+  if (rc) return rc;
+  const int mode = tc3_mode(precision);
   if (mode == kF16) {
     // the fp16 copies live in the (larger) fp32 operand regions: hi/lo of B1 [Hq][Hq], hi/lo of B2g [Hq][Hq]
-    uint32_t* mx = reinterpret_cast<uint32_t*>(t3 + T3.sumV + 8);
+    uint32_t* mx = reinterpret_cast<uint32_t*>(ws + L.sumV + 8);
     if (cudaMemsetAsync(mx, 0, 2 * sizeof(uint32_t), st) != cudaSuccess) return B200VAE_ECUDA;
     tc3_rowmax_kernel<<<L.Hp, 256, 0, st>>>(ws + L.P0, ws + L.P1, L.Hp, mx);
     rc = check_launch();
     if (rc) return rc;
-    dim3 grid((T3.Hq + 255) / 256, T3.Hq);
+    dim3 grid((L.Hq + 255) / 256, L.Hq);
     tc3_prepare_f16_kernel<<<grid, 256, 0, st>>>(
-        ws + L.P0, ws + L.P0T, ws + L.P1, ws + L.A0p, ws + L.A1p, d, L.Hp, T3.Hq, mx, reinterpret_cast<__half*>(t3 + T3.B1ahi),
-        reinterpret_cast<__half*>(t3 + T3.B1alo), reinterpret_cast<__half*>(t3 + T3.B2ghi), reinterpret_cast<__half*>(t3 + T3.B2glo),
-        reinterpret_cast<float4*>(t3 + T3.A0g), reinterpret_cast<float4*>(t3 + T3.E1), t3 + T3.sumV + 16);
+        ws + L.P0, ws + L.P0T, ws + L.P1, ws + L.A0p, ws + L.A1p, L.d, L.Hp, L.Hq, mx, reinterpret_cast<__half*>(ws + L.B1ahi),
+        reinterpret_cast<__half*>(ws + L.B1alo), reinterpret_cast<__half*>(ws + L.B2ghi), reinterpret_cast<__half*>(ws + L.B2glo),
+        reinterpret_cast<float4*>(ws + L.A0g), reinterpret_cast<float4*>(ws + L.E1), ws + L.sumV + 16);
   } else {
-    dim3 grid((T3.K1 + 255) / 256, T3.Hq);
-    tc3_prepare_kernel<<<grid, 256, 0, st>>>(ws + L.P0, ws + L.P0T, ws + L.P1, ws + L.A0p, ws + L.A1p, d, L.Hp, T3.Hq, T3.K1,
-                                             mode == kX3 ? 1 : 0, t3 + T3.B1ahi, t3 + T3.B1alo, t3 + T3.B2ghi, t3 + T3.B2glo,
-                                             reinterpret_cast<float4*>(t3 + T3.A0g), reinterpret_cast<float4*>(t3 + T3.E1));
+    dim3 grid((L.K1 + 255) / 256, L.Hq);
+    tc3_prepare_kernel<<<grid, 256, 0, st>>>(ws + L.P0, ws + L.P0T, ws + L.P1, ws + L.A0p, ws + L.A1p, L.d, L.Hp, L.Hq, L.K1,
+                                             mode == kX3 ? 1 : 0, ws + L.B1ahi, ws + L.B1alo, ws + L.B2ghi, ws + L.B2glo,
+                                             reinterpret_cast<float4*>(ws + L.A0g), reinterpret_cast<float4*>(ws + L.E1));
   }
   rc = check_launch();
   if (rc) return rc;
-  tc3_sumv_kernel<<<1, 32, 0, st>>>(reinterpret_cast<const float4*>(t3 + T3.E1), reinterpret_cast<const float4*>(t3 + T3.A0g),
-                                    T3.Hq, t3 + T3.sumV);
+  tc3_sumv_kernel<<<1, 32, 0, st>>>(reinterpret_cast<const float4*>(ws + L.E1), reinterpret_cast<const float4*>(ws + L.A0g),
+                                    L.Hq, ws + L.sumV);
   rc = check_launch();
   if (rc) return rc;
-  if (cudaMemsetAsync(t3 + T3.cnt, 0, (size_t)2 * kTc3MaxTiles * sizeof(uint32_t), st) != cudaSuccess) return B200VAE_ECUDA;
+  if (cudaMemsetAsync(ws + L.cnt, 0, (size_t)2 * kTc3MaxTiles * sizeof(uint32_t), st) != cudaSuccess) return B200VAE_ECUDA;
   return B200VAE_OK;
 }
 
 struct Tc3Maps { CUtensorMap b1hi, b1lo, b2hi, b2lo; };
-static int get_maps3(const float* t3, const Tc3Layout& T3, int mode, Tc3Maps* out) {
+static int get_maps3(const float* ws, const WsLayout& L, int mode, Tc3Maps* out) {
   static std::mutex mu;
   static std::unordered_map<uint64_t, Tc3Maps> cache;       // tensor maps only encode (address, shape, element type)
   std::lock_guard<std::mutex> lk(mu);
-  const uint64_t key = reinterpret_cast<uint64_t>(t3) ^ ((uint64_t)T3.Hq << 48) ^ ((uint64_t)mode << 62);
+  const uint64_t key = reinterpret_cast<uint64_t>(ws + L.B1ahi) ^ ((uint64_t)L.Hq << 48) ^ ((uint64_t)mode << 62);
   auto itc = cache.find(key);
   if (itc != cache.end()) { *out = itc->second; return B200VAE_OK; }
   Tc3Maps mp;
   const bool hl = mode != kTf32, f16 = mode == kF16;
-  const int K1 = f16 ? T3.Hq : T3.K1;
-  int rc = make_map3(&mp.b1hi, t3 + T3.B1ahi, K1, T3.Hq, f16);
-  if (!rc) rc = make_map3(&mp.b1lo, t3 + (hl ? T3.B1alo : T3.B1ahi), K1, T3.Hq, f16);
-  if (!rc) rc = make_map3(&mp.b2hi, t3 + T3.B2ghi, T3.Hq, T3.Hq, f16);
-  if (!rc) rc = make_map3(&mp.b2lo, t3 + (hl ? T3.B2glo : T3.B2ghi), T3.Hq, T3.Hq, f16);
+  const int K1 = f16 ? L.Hq : L.K1;
+  int rc = make_map3(&mp.b1hi, ws + L.B1ahi, K1, L.Hq, f16);
+  if (!rc) rc = make_map3(&mp.b1lo, ws + (hl ? L.B1alo : L.B1ahi), K1, L.Hq, f16);
+  if (!rc) rc = make_map3(&mp.b2hi, ws + L.B2ghi, L.Hq, L.Hq, f16);
+  if (!rc) rc = make_map3(&mp.b2lo, ws + (hl ? L.B2glo : L.B2ghi), L.Hq, L.Hq, f16);
   if (rc) return rc;
   if (cache.size() > 256) cache.clear();
   cache.emplace(key, mp);
@@ -1831,7 +1904,7 @@ icnn_tc3_dP0_kernel(const float* __restrict__ z, const float* __restrict__ v, co
     if (two || cg < 2) {
       float* out = dP0part + ((size_t)split * Hq + o0 + cg * 128) * Hq + n;
       if (NKB > 0) {
-        mbar_wait_parked(accfull, 0, 2000);
+        mbar_wait_parked(accfull, 0, k3ParkNs);
         tc_fence_after();
 #pragma unroll 1
         for (int cc = 0; cc < 4; ++cc) {
@@ -2083,7 +2156,7 @@ icnn_tc3_dP0_f16_kernel(const float* __restrict__ z, const float* __restrict__ v
     if (two || cg < 2) {
       float* out = dP0part + ((size_t)split * Hq + o0 + cg * 128) * Hq + n;
       if (NSG > 0) {
-        mbar_wait_parked(accfull, 0, 2000);
+        mbar_wait_parked(accfull, 0, k3ParkNs);
         tc_fence_after();
 #pragma unroll 1
         for (int cc = 0; cc < 4; ++cc) {
@@ -2133,10 +2206,11 @@ icnn_tc3_dP0_f16_kernel(const float* __restrict__ z, const float* __restrict__ v
   }
 }
 
-static int max_clusters_for(const void* fn, size_t smem) {
+// clusters of two CTAs of `fn` that can be resident at once
+static int max_clusters_for(const void* fn, size_t smem, int threads) {
   cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
   cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3(2 * 74); cfg.blockDim = dim3(k3Threads); cfg.dynamicSmemBytes = smem;
+  cfg.gridDim = dim3(2 * 74); cfg.blockDim = dim3(threads); cfg.dynamicSmemBytes = smem;
   cudaLaunchAttribute at;
   at.id = cudaLaunchAttributeClusterDimension;
   at.val.clusterDim.x = 2; at.val.clusterDim.y = 1; at.val.clusterDim.z = 1;
@@ -2149,81 +2223,60 @@ static int max_clusters_for(const void* fn, size_t smem) {
   return n;
 }
 
-static int max_clusters_dp(const void* fn, size_t smem) {
-  cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3(2 * 74); cfg.blockDim = dim3(kDpThreads3); cfg.dynamicSmemBytes = smem;
-  cudaLaunchAttribute at;
-  at.id = cudaLaunchAttributeClusterDimension;
-  at.val.clusterDim.x = 2; at.val.clusterDim.y = 1; at.val.clusterDim.z = 1;
-  cfg.attrs = &at; cfg.numAttrs = 1;
-  int n = 0;
-  if (cudaOccupancyMaxActiveClusters(&n, fn, &cfg) != cudaSuccess || n <= 0) {
-    (void)cudaGetLastError();
-    n = sm_count() / 2;
-  }
-  return n;
-}
+// dP0 launches: one wave of long-running clusters, never more slabs than the workspace holds
 template <int D, bool X3>
-static int launch_tc3_dp0(const float* z, const float* v, const uint32_t* mask1, const uint8_t* mask2, int B, int Hq,
-                          int Hw_in, const float4* A0q, int max_splits, float* part, int* splits_out, cudaStream_t st) {
+static int launch_tc3_dp0(const float* z, const float* v, const uint32_t* mask1, const uint8_t* mask2, const WsLayout& L,
+                          const float4* A0q, float* part, int* splits_out, cudaStream_t st) {
   constexpr size_t smem = dp3_smem_bytes<D, X3>();
   static_assert(smem <= 227 * 1024, "dP0 pair kernel: shared memory");
   static int max_clusters = 0;
-  if (max_clusters == 0) max_clusters = max_clusters_dp(reinterpret_cast<const void*>(icnn_tc3_dP0_kernel<D, X3>), smem);
-  const int tn = Hq / 256, to = (Hq + 511) / 512;
-  int splits = max_clusters / (tn * to);                     // one wave of long-running clusters
-  if (splits > max_splits) splits = max_splits;              // (workspace slabs, and at least 256 samples per split)
-  if (splits < 1) splits = 1;
-  int rows = (B + splits - 1) / splits;
-  rows = round_up(rows, kKB);
-  dim3 grid(2 * tn, to, splits);
-  icnn_tc3_dP0_kernel<D, X3><<<grid, kDpThreads3, smem, st>>>(z, v, mask1, mask2, B, Hq, Hw_in, rows, A0q, part);
+  if (max_clusters == 0)
+    max_clusters = max_clusters_for(reinterpret_cast<const void*>(icnn_tc3_dP0_kernel<D, X3>), smem, kDpThreads3);
+  int splits = dp0_splits(L.B, L.Hq, max_clusters);
+  if (splits > L.dp0_splits) splits = L.dp0_splits;
+  const int rows = round_up((L.B + splits - 1) / splits, kKB);
+  dim3 grid(2 * (L.Hq / 256), (L.Hq + 511) / 512, splits);
+  icnn_tc3_dP0_kernel<D, X3><<<grid, kDpThreads3, smem, st>>>(z, v, mask1, mask2, L.B, L.Hq, L.Hp / 32, rows, A0q, part);
   *splits_out = splits;
   return check_launch();
 }
 template <int D>
-static int launch_tc3_dp0_f16(const float* z, const float* v, const uint32_t* mask1, const uint8_t* mask2, int B, int Hq,
-                              int Hw_in, const float4* A0q, const float* sumV, int max_splits, float* part, int* splits_out,
-                              cudaStream_t st) {
+static int launch_tc3_dp0_f16(const float* z, const float* v, const uint32_t* mask1, const uint8_t* mask2, const WsLayout& L,
+                              const float4* A0q, const float* sumV, float* part, int* splits_out, cudaStream_t st) {
   constexpr size_t smem = dp3_f16_smem_bytes<D>();
   static_assert(smem <= 227 * 1024, "dP0 pair kernel (fp16): shared memory");
   static int max_clusters = 0;
-  if (max_clusters == 0) max_clusters = max_clusters_dp(reinterpret_cast<const void*>(icnn_tc3_dP0_f16_kernel<D>), smem);
-  const int tn = Hq / 256, to = (Hq + 511) / 512;
-  int splits = max_clusters / (tn * to);                     // one wave of long-running clusters
-  if (splits > max_splits) splits = max_splits;
-  if (splits < 1) splits = 1;
-  int rows = (B + splits - 1) / splits;
-  rows = round_up(rows, 32);
-  dim3 grid(2 * tn, to, splits);
-  icnn_tc3_dP0_f16_kernel<D><<<grid, kDpThreads3, smem, st>>>(z, v, mask1, mask2, B, Hq, Hw_in, rows, A0q, sumV, part);
+  if (max_clusters == 0)
+    max_clusters = max_clusters_for(reinterpret_cast<const void*>(icnn_tc3_dP0_f16_kernel<D>), smem, kDpThreads3);
+  int splits = dp0_splits(L.B, L.Hq, max_clusters);
+  if (splits > L.dp0_splits) splits = L.dp0_splits;
+  const int rows = round_up((L.B + splits - 1) / splits, 32);
+  dim3 grid(2 * (L.Hq / 256), (L.Hq + 511) / 512, splits);
+  icnn_tc3_dP0_f16_kernel<D><<<grid, kDpThreads3, smem, st>>>(z, v, mask1, mask2, L.B, L.Hq, L.Hp / 32, rows, A0q, sumV, part);
   *splits_out = splits;
   return check_launch();
 }
-// part: [splits][Hq][Hq] ordered split-K slabs (reduced by finalize_W0_kernel); *splits_out <= max_splits.
-// sumV: Tc3Layout::sumV of the prepared workspace (max |A0| for the FP16 mode's scale)
-int tc3_dp0(const float* z, const float* v, const uint32_t* mask1, const uint8_t* mask2, int B, int d, int Hq, int Hw_in,
-            const float* A0q, const float* sumV, int precision, int max_splits, float* part, int* splits_out, cudaStream_t st) {
-  if (precision == 2 /* reserved */ || d > 3) return B200VAE_EUNSUP;
-  const float4* q = reinterpret_cast<const float4*>(A0q);
-  static const int dp_f16 = [] { const char* e = getenv("B200VAE_DP0_F16"); return e ? atoi(e) : 1; }();
-  if (precision == B200VAE_PREC_F16X3 && dp_f16) {
-    switch (d) {
-      case 1: return launch_tc3_dp0_f16<1>(z, v, mask1, mask2, B, Hq, Hw_in, q, sumV, max_splits, part, splits_out, st);
-      case 2: return launch_tc3_dp0_f16<2>(z, v, mask1, mask2, B, Hq, Hw_in, q, sumV, max_splits, part, splits_out, st);
-      default: return launch_tc3_dp0_f16<3>(z, v, mask1, mask2, B, Hq, Hw_in, q, sumV, max_splits, part, splits_out, st);
+// dP0part_tc: [splits][Hq][Hq] ordered split-K slabs (reduced by finalize_W0_kernel)
+static int tc3_dp0(const float* z, const float* v, const uint32_t* mask1, const uint8_t* mask2, const WsLayout& L, int precision,
+                   float* ws, int* splits_out, cudaStream_t st) {
+  const float4* q = reinterpret_cast<const float4*>(ws + L.A0q);
+  float* part = ws + L.dP0part_tc;
+  if (precision == B200VAE_PREC_F16X3) {
+    const float* sumV = ws + L.sumV;                         // max |A0| for the FP16 mode's scale
+    switch (L.d) {
+      case 1: return launch_tc3_dp0_f16<1>(z, v, mask1, mask2, L, q, sumV, part, splits_out, st);
+      case 2: return launch_tc3_dp0_f16<2>(z, v, mask1, mask2, L, q, sumV, part, splits_out, st);
+      default: return launch_tc3_dp0_f16<3>(z, v, mask1, mask2, L, q, sumV, part, splits_out, st);
     }
   }
-  const bool x3 = (precision == B200VAE_PREC_TF32X3 || precision == B200VAE_PREC_F16X3);
-#define B200VAE_TC3D(DD)                                                                                             \
-  return x3 ? launch_tc3_dp0<DD, true>(z, v, mask1, mask2, B, Hq, Hw_in, q, max_splits, part, splits_out, st)         \
-            : launch_tc3_dp0<DD, false>(z, v, mask1, mask2, B, Hq, Hw_in, q, max_splits, part, splits_out, st)
-  switch (d) {
+  const bool x3 = precision == B200VAE_PREC_TF32X3;
+#define B200VAE_TC3D(DD)                                                                          \
+  return x3 ? launch_tc3_dp0<DD, true>(z, v, mask1, mask2, L, q, part, splits_out, st)            \
+            : launch_tc3_dp0<DD, false>(z, v, mask1, mask2, L, q, part, splits_out, st)
+  switch (L.d) {
     case 1: B200VAE_TC3D(1);
     case 2: B200VAE_TC3D(2);
-    case 3: B200VAE_TC3D(3);
-    default: return B200VAE_EUNSUP;
+    default: B200VAE_TC3D(3);
   }
 #undef B200VAE_TC3D
 }
@@ -2231,131 +2284,128 @@ int tc3_dp0(const float* z, const float* v, const uint32_t* mask1, const uint8_t
 template <int D, int MODE, bool SV>
 static int launch_tc3_bwd(const Tc3BwdArgs& args, cudaStream_t st) {
   const size_t smem = tc3_smem_bytes<MODE>(args.Hq);
-  if (smem > 227 * 1024 || args.Hq > kTc3MaxHq) return B200VAE_EUNSUP;
   static int max_clusters = 0;
-  if (max_clusters == 0) max_clusters = max_clusters_for(reinterpret_cast<const void*>(icnn_tc3_bwd_kernel<D, MODE, SV>), smem);
+  if (max_clusters == 0)
+    max_clusters = max_clusters_for(reinterpret_cast<const void*>(icnn_tc3_bwd_kernel<D, MODE, SV>), smem, k3Threads);
   const int units = (SV ? 1 : 2) * args.T * args.NP;
   const int G = units < max_clusters ? units : max_clusters;
   icnn_tc3_bwd_kernel<D, MODE, SV><<<2 * G, k3Threads, smem, st>>>(args);
   return check_launch();
 }
 
-// rows part of the backward: fills partA/partB [T*8][d+1][Hq], a2part [T][d], dz [B,d] (layouts of icnn_tc.cu's tc_bwd)
-int tc3_bwd_rows(const float* z, const float* v, const uint32_t* mask1, const uint8_t* mask2, int B, int d, int H, float kappa,
-                 float* dz, float* partA, float* partB, float* a2part, float* dzpart, int precision, float* ws,
-                 const float* accsave, cudaStream_t st) {
-  if (precision == 2 /* reserved */ || d > 3) return B200VAE_EUNSUP;
-  const WsLayout L = ws_layout(1, d, H);
-  const TcLayout T = tc_layout(d, H);
-  const Tc3Layout T3 = tc3_layout(B, d, H);
-  float* tb = tc_base(ws, d, H);
-  float* t3 = tb + T.end;
-  const int mode = tc3_mode(precision, T3.Hq);
+// rows part of the backward: fills partA / partB [T*8][d+1][Hq], a2part_tc [T][d], dz [B,d]
+static int tc3_bwd_rows(const float* z, const float* v, const uint32_t* mask1, const uint8_t* mask2, const WsLayout& L,
+                        float kappa, float* dz, int precision, float* ws, const float* accsave, cudaStream_t st) {
+  const int mode = tc3_mode(precision);
   Tc3Maps mp;
-  int rc = get_maps3(t3, T3, mode, &mp);
+  int rc = get_maps3(ws, L, mode, &mp);
   if (rc) return rc;
   Tc3BwdArgs args;
   args.b1hi = mp.b1hi; args.b1lo = mp.b1lo; args.b2hi = mp.b2hi; args.b2lo = mp.b2lo;
   args.z = z; args.v = v; args.mask1 = mask1; args.mask2 = mask2;
-  args.A0g = reinterpret_cast<const float4*>(t3 + T3.A0g);
-  args.E1 = reinterpret_cast<const float4*>(t3 + T3.E1);
-  args.A0q = reinterpret_cast<const float4*>(tb + T.A0q);
-  args.A1q = reinterpret_cast<const float4*>(tb + T.A1q);
-  args.sumV = t3 + T3.sumV;
-  args.partA = partA; args.partB = partB;
-  args.dzpart = reinterpret_cast<float4*>(dzpart);
+  args.A0g = reinterpret_cast<const float4*>(ws + L.A0g);
+  args.E1 = reinterpret_cast<const float4*>(ws + L.E1);
+  args.A0q = reinterpret_cast<const float4*>(ws + L.A0q);
+  args.A1q = reinterpret_cast<const float4*>(ws + L.A1q);
+  args.sumV = ws + L.sumV;
+  args.partA = ws + L.partA; args.partB = ws + L.partB;
+  args.dzpart = reinterpret_cast<float4*>(ws + L.dzpart);
   args.accsave = accsave;
-  args.B = B; args.Hq = T3.Hq; args.T = T3.Bp / 256; args.NP = T3.NP; args.Hw_in = L.Hp / 32;
+  args.B = L.B; args.Hq = L.Hq; args.T = L.Bp / 256; args.NP = L.NP; args.Hw_in = L.Hp / 32;
   // the saved-accumulator kernels pay off where the kernel is tensor bound (3xTF32); at 1xTF32 the epilogue warps are the
   // bottleneck either way and recomputing GEMM2 is free
 #define B200VAE_TC3B(DD)                                                                                                  \
   rc = mode == kF16 ? (accsave ? launch_tc3_bwd<DD, kF16, true>(args, st) : launch_tc3_bwd<DD, kF16, false>(args, st))    \
        : mode == kX3 ? (accsave ? launch_tc3_bwd<DD, kX3, true>(args, st) : launch_tc3_bwd<DD, kX3, false>(args, st))     \
                      : launch_tc3_bwd<DD, kTf32, false>(args, st)
-  switch (d) {
+  switch (L.d) {
     case 1: B200VAE_TC3B(1); break;
     case 2: B200VAE_TC3B(2); break;
-    case 3: B200VAE_TC3B(3); break;
-    default: return B200VAE_EUNSUP;
+    default: B200VAE_TC3B(3); break;
   }
 #undef B200VAE_TC3B
   if (rc) return rc;
-  tc3_bwd_dz_kernel<<<args.T, 256, 0, st>>>(reinterpret_cast<const float4*>(dzpart), v, mask2, B, args.NP, d, kappa, dz, a2part);
+  tc3_bwd_dz_kernel<<<args.T, 256, 0, st>>>(args.dzpart, v, mask2, L.B, args.NP, L.d, kappa, dz, ws + L.a2part_tc);
   return check_launch();
 }
-size_t tc3_bwd_ws_floats(int B, int d, int H) {
-  const Tc3Layout T3 = tc3_layout(B, d, H);
-  return (size_t)T3.Bp * T3.NP * 2 * 4 + 64;
+
+// phase 0: everything; 1: the rows part only (dz + the ordered column partials in the workspace); 2: the parameter
+// gradients only (dP0 + the finalize kernels), from the partials a phase-1 call left in the SAME workspace
+int tc_bwd(const float* z, const float* v, const uint32_t* mask1, const uint8_t* mask2, const WsLayout& L,
+           const b200vae_icnn_params* p, int mode, float kappa, const b200vae_icnn_grads* g, float* dz, int precision,
+           float* ws, const float* accsave, int phase, cudaStream_t st) {
+  int rc = B200VAE_OK;
+  if (phase != 2) rc = tc3_bwd_rows(z, v, mask1, mask2, L, kappa, dz, precision, ws, accsave, st);
+  if (rc || !g || phase == 1) return rc;
+  if (g->W0) {
+    int splits = 0;
+    rc = tc3_dp0(z, v, mask1, mask2, L, precision, ws, &splits, st);
+    if (rc) return rc;
+    rc = finalize_W0_launch(ws + L.dP0part_tc, splits, L.H, L.Hp, L.Hq, ws + L.P0, ws + L.P1, p->W0, mode, kSlope, g->W0, st);
+    if (rc) return rc;
+  }
+  const int T = L.Bp / 256;
+  dim3 fgrid(L.Hq / 32, L.d + 1, 2);
+  tc_finalize_small_kernel<<<fgrid, 1024, 0, st>>>(ws + L.partA, ws + L.partB, ws + L.a2part_tc, T * 8, T, L.d, L.H, L.Hq,
+                                                  ws + L.P1, p->W1, mode, *g);
+  return check_launch();
 }
 
 template <int D, int MODE>
 static int launch_tc3(const Tc3Args& args, int units, cudaStream_t st) {
   const size_t smem = tc3_smem_bytes<MODE>(args.Hq);
-  if (smem > 227 * 1024 || args.Hq > kTc3MaxHq) return B200VAE_EUNSUP;
   static int max_clusters = 0;
-  if (max_clusters == 0) max_clusters = max_clusters_for(reinterpret_cast<const void*>(icnn_tc3_fwd_kernel<D, MODE>), smem);
+  if (max_clusters == 0)
+    max_clusters = max_clusters_for(reinterpret_cast<const void*>(icnn_tc3_fwd_kernel<D, MODE>), smem, k3Threads);
   // every cluster must be resident (GEMM2 units wait for GEMM1 units of other clusters): never exceed one wave
   const int G = units < max_clusters ? units : max_clusters;
   icnn_tc3_fwd_kernel<D, MODE><<<2 * G, k3Threads, smem, st>>>(args);
   return check_launch();
 }
 
-int tc3_fwd(const float* z, int B, int d, int H, float kappa, float* psi, float* xhat, uint32_t* mask1, uint8_t* mask2,
+int tc3_fwd(const float* z, const WsLayout& L, float kappa, float* psi, float* xhat, uint32_t* mask1, uint8_t* mask2,
             int precision, float* ws, float* accsave, cudaStream_t st) {
-  if (precision == 2 /* reserved */ || d > 3) return B200VAE_EUNSUP;
-  const WsLayout L = ws_layout(1, d, H);
-  const TcLayout T = tc_layout(d, H);
-  const Tc3Layout T3 = tc3_layout(B, d, H);
-  if (T3.Bp / 256 > kTc3MaxTiles) return B200VAE_EUNSUP;
-  float* tb = tc_base(ws, d, H);
-  float* t3 = tb + T.end;
-  const int mode = tc3_mode(precision, T3.Hq);
-  const bool x3 = mode != kTf32;
+  if (L.Bp / 256 > kTc3MaxTiles) return B200VAE_EUNSUP;
+  const int mode = tc3_mode(precision);
   Tc3Args args;
   {
     Tc3Maps mp;
-    int rc = get_maps3(t3, T3, mode, &mp);
+    int rc = get_maps3(ws, L, mode, &mp);
     if (rc) return rc;
     args.b1hi = mp.b1hi; args.b1lo = mp.b1lo; args.b2hi = mp.b2hi; args.b2lo = mp.b2lo;
   }
   args.z = z;
-  args.A0g = reinterpret_cast<const float4*>(t3 + T3.A0g);
-  args.E1 = reinterpret_cast<const float4*>(t3 + T3.E1);
-  args.A0q = reinterpret_cast<const float4*>(tb + T.A0q);
-  args.A1q = reinterpret_cast<const float4*>(tb + T.A1q);
-  args.P1q = tb + T.P1q;
-  args.sumV = t3 + T3.sumV;
+  args.A0g = reinterpret_cast<const float4*>(ws + L.A0g);
+  args.E1 = reinterpret_cast<const float4*>(ws + L.E1);
+  args.A0q = reinterpret_cast<const float4*>(ws + L.A0q);
+  args.A1q = reinterpret_cast<const float4*>(ws + L.A1q);
+  args.P1q = ws + L.P1q;
+  args.sumV = ws + L.sumV;
   args.A2p = ws + L.A2p;
   args.psi = psi; args.xhat = xhat; args.mask2 = mask2;
   args.want_x = xhat != nullptr ? 1 : 0;
-  if (mask1) { args.maskg = mask1; args.mask_stride = L.Hp / 32; args.mask_rows = B; }
-  else if (args.want_x) { args.maskg = reinterpret_cast<uint32_t*>(t3 + T3.imask); args.mask_stride = T3.Hq / 32; args.mask_rows = T3.Bp; }
+  if (mask1) { args.maskg = mask1; args.mask_stride = L.Hp / 32; args.mask_rows = L.B; }
+  else if (args.want_x) { args.maskg = reinterpret_cast<uint32_t*>(ws + L.imask); args.mask_stride = L.Hq / 32; args.mask_rows = L.Bp; }
   else { args.maskg = nullptr; args.mask_stride = 0; args.mask_rows = 0; }
-  args.scr1 = reinterpret_cast<float4*>(t3 + T3.scr1);
-  args.scr2 = reinterpret_cast<float4*>(t3 + T3.scr2);
-  args.cnt = reinterpret_cast<uint32_t*>(t3 + T3.cnt);
+  args.scr1 = reinterpret_cast<float4*>(ws + L.scr1);
+  args.scr2 = reinterpret_cast<float4*>(ws + L.scr2);
+  args.cnt = reinterpret_cast<uint32_t*>(ws + L.cnt);
   args.accsave = args.want_x ? accsave : nullptr;
-  args.B = B; args.Hq = T3.Hq; args.T = T3.Bp / 256; args.NP = T3.NP; args.kappa = kappa;
-  // hi/lo modes: accumulate K in chunks of kTc3ChunkK (B200VAE_KCHUNK overrides: a multiple of 64 dividing Hq; 0 = one
-  // chunk).  FP16 mode at H = 1024, default-init weights: psi error 8.7e-6 in one piece (0.453 ms), 4.0e-6 in two chunks
-  // (0.474 ms, wherever the split point lies -- 512 ... 768 measured; the 21 us are the drain's L2 traffic: 14 us its
-  // stores, 6 us the loads of the last chunk's epilogue -- measured by leaving each out), 2.0e-6 in four (0.544 ms)
-  static const int chunk_env = [] { const char* e = getenv("B200VAE_KCHUNK"); return e ? atoi(e) : -1; }();
-  const int chunk_k = chunk_env >= 0 ? chunk_env : kTc3ChunkK;
-  static const int park_ns = [] { const char* e = getenv("B200VAE_PARK_NS"); return e ? atoi(e) : 2000; }();
-  args.cscr = reinterpret_cast<float4*>(t3 + T3.cscr);
-  args.park_ns = (uint32_t)park_ns;
-  args.NC = 1;
-  if (x3 && chunk_k >= 64 && chunk_k % 64 == 0 && T3.Hq % chunk_k == 0) args.NC = T3.Hq / chunk_k;
+  args.B = L.B; args.Hq = L.Hq; args.T = L.Bp / 256; args.NP = L.NP; args.kappa = kappa;
+  // hi/lo modes: accumulate K in chunks of kTc3ChunkK where it divides Hq.  FP16 mode at H = 1024, default-init weights: psi
+  // error 8.7e-6 in one piece (0.453 ms), 4.0e-6 in two chunks (0.474 ms, wherever the split point lies -- 512 ... 768
+  // measured; the 21 us are the drain's L2 traffic: 14 us its stores, 6 us the loads of the last chunk's epilogue --
+  // measured by leaving each out), 2.0e-6 in four (0.544 ms)
+  args.cscr = reinterpret_cast<float4*>(ws + L.cscr);
+  args.NC = (mode != kTf32 && L.Hq % kTc3ChunkK == 0) ? L.Hq / kTc3ChunkK : 1;
   const int units = (args.want_x ? 2 : 1) * args.T * args.NP;
 #define B200VAE_TC3(DD)                                                       \
   return mode == kF16 ? launch_tc3<DD, kF16>(args, units, st)                 \
          : mode == kX3 ? launch_tc3<DD, kX3>(args, units, st) : launch_tc3<DD, kTf32>(args, units, st)
-  switch (d) {
+  switch (L.d) {
     case 1: B200VAE_TC3(1);
     case 2: B200VAE_TC3(2);
-    case 3: B200VAE_TC3(3);
-    default: return B200VAE_EUNSUP;
+    default: B200VAE_TC3(3);
   }
 #undef B200VAE_TC3
 }

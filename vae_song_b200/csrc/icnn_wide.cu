@@ -16,8 +16,6 @@
 //             out : dz = t0 A0 + 2 kappa v
 //             tn  : dA0 = g0^T v + t0^T z,  dA1 = g1^T v,  dP0 = g1^T q1     (split over the batch, ordered slabs)
 // Algebra: SURVEY.md Appendix A (oracle/icnn_oracle.py).  All reductions are ordered: bit-reproducible.
-#include <cstdlib>
-
 #include "gemm_simt.cuh"
 
 namespace b200vae {
@@ -623,8 +621,7 @@ extern "C" int b200vae_icnn_wide_fwd(const float* z, int B, int d, int nz, int H
   const bool p16 = aligned16(p->A0b) && aligned16(p->A1b) && aligned16(p->A2w);
   cudaStream_t st = (cudaStream_t)stream;
   float* ws = (float*)workspace;
-  static const bool tc_on = [] { const char* e = getenv("B200VAE_WIDE_TC"); return !e || atoi(e) != 0; }();
-  if (precision != B200VAE_PREC_FP32 && tc_on && p16 && wide_tc_supported(d, nz, H, precision)) {   // tcgen05 forward
+  if (precision != B200VAE_PREC_FP32 && p16 && wide_tc_supported(d, nz, H, precision)) {   // tcgen05 forward
     const int rc_tc = wide_tc_fwd(z, B, d, nz, H, p, weight_mode, kappa, psi, xhat, h0, mask1, s2, g0, ws, precision, st);
     if (rc_tc != B200VAE_EUNSUP) return rc_tc;
   }
@@ -669,9 +666,8 @@ extern "C" int b200vae_icnn_wide_bwd(const float* z, const float* v, const float
   int rc = wide_prepare(p, d, H, weight_mode, ws, L, st);
   if (rc) return rc;
   const dim3 gH(L.mt, L.nt), gD(L.mt, (d + 127) / 128);
-  static const bool tc_on = [] { const char* e = getenv("B200VAE_WIDE_TC"); return !e || atoi(e) != 0; }();
   bool rows_done = false;
-  if (precision != B200VAE_PREC_FP32 && tc_on && wide_tc_supported(d, nz, H, precision)) {
+  if (precision != B200VAE_PREC_FP32 && wide_tc_supported(d, nz, H, precision)) {
     // sample-stationary GEMMs on tcgen05 (icnn_wide_tc.cu); the batch-reduction GEMMs below stay FP32
     rc = wide_tc_bwd_rows(v, h0, mask1, s2, B, d, nz, H, p, weight_mode, kappa, dz, u0, q1, g0, t0, g ? g->W1 : nullptr,
                           g ? g->A0b : nullptr, ws + L.end, ws + L.colpart, precision, st);

@@ -1,4 +1,4 @@
-// tc_common.cuh -- PTX wrappers (mbarrier, TMA, tcgen05, TMEM) and workspace layout shared by the tensor-core kernels.
+// tc_common.cuh -- PTX wrappers (mbarrier, TMA, tcgen05, TMEM) and small helpers shared by the tensor-core kernels.
 #pragma once
 #include <cuda.h>
 
@@ -6,11 +6,7 @@
 
 namespace b200vae {
 
-
-constexpr int kTM = 256;          // samples per CTA
-constexpr int kTN = 256;          // accumulator columns per pass
 constexpr int kKB = 16;           // K elements per block (64 B rows, SWIZZLE_64B)
-constexpr int kTileBytes = 256 * 64;   // one 256-row x 64-byte operand tile = 16 KB
 
 // ------------------------------------------------------------------------------------ PTX helpers
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
@@ -90,11 +86,7 @@ __device__ __forceinline__ float to_tf32(float x) {
 }
 
 // round-to-nearest (ties away) to tf32 in one integer add: tcgen05 kind::tf32 ignores the 13 low mantissa bits
-#ifdef B200VAE_MASKED_RN
-__device__ __forceinline__ float rn_tf32_fast(float x) { return __uint_as_float((__float_as_uint(x) + 0x1000u) & 0xFFFFE000u); }
-#else
 __device__ __forceinline__ float rn_tf32_fast(float x) { return __uint_as_float(__float_as_uint(x) + 0x1000u); }
-#endif
 __device__ __forceinline__ float rn_tf32_masked(float x) { return __uint_as_float((__float_as_uint(x) + 0x1000u) & 0xFFFFE000u); }
 
 // K-major, SWIZZLE_64B shared-memory matrix descriptor (cute::UMMA::SmemDescriptor): start>>4 | LBO(1)<<16 |
@@ -103,88 +95,6 @@ __device__ __forceinline__ uint64_t make_desc_sw64(uint32_t saddr) {
   return (uint64_t)((saddr & 0x3FFFFu) >> 4) | ((uint64_t)1 << 16) | ((uint64_t)(512 >> 4) << 32) | ((uint64_t)1 << 46) |
          ((uint64_t)4 << 61);
 }
-// kind::tf32 instruction descriptor: D=F32 (1<<4), A=B=TF32 (2<<7, 2<<10), K-major both, N>>3 at 17, M>>4 at 24
-constexpr uint32_t kIdescTf32 = (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)(kTN >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);
-
-// byte offset of 16-byte chunk c (0..3) of row r (0..255) inside a 256-row x 64 B SWIZZLE_64B tile
-__device__ __forceinline__ uint32_t sw64_off(int r, int c) { return (uint32_t)(r * 64 + ((c ^ ((r >> 1) & 3)) << 4)); }
-
-// ------------------------------------------------------------------------------------ TC workspace
-// (floats, after the SIMT layout's `end`)  Hq = H rounded up to 256.  Per-unit parameter tables in natural unit order:
-//   A0q, A1q  float4[Hq] = (w0, w1, w2, bias)   P1q [Hq]
-struct TcLayout {
-  int Hq;
-  size_t A0q, A1q, P1q, end;
-};
-inline TcLayout tc_layout(int d, int H) {
-  (void)d;
-  TcLayout T;
-  T.Hq = round_up(H, 256);
-  size_t o = 0;
-  T.A0q = o; o += (size_t)4 * T.Hq; T.A1q = o; o += (size_t)4 * T.Hq; T.P1q = o; o += T.Hq;
-  T.end = o + 64;
-  return T;
-}
-inline float* tc_base(float* ws, int d, int H) {
-  // TC arrays start after the largest SIMT layout we might share the buffer with; use a fixed, B-independent
-  // offset: the forward part of the SIMT layout (the backward scratch is placed AFTER the TC arrays, see api.cu)
-  return ws + ws_layout(1, d, H).fwd_end;
-}
-
-
-// ------------------------------------------------------------------------------------ persistent pair kernel (icnn_tc3.cu)
-// Placed after the TcLayout arrays (floats from tc_base + TcLayout::end).  K1 = Hq + 16: GEMM1's B operand carries one
-// extra 16-wide K-block holding A1/b1 (split hi/lo) so that the affine part of h1 is accumulated by the tensor core.
-//   B1a hi,lo [Hq][K1]   B1a[o][i] = P[o][i] (i < Hq);  B1a[o][Hq + m] = lin-block column m (see tc3_prepare_kernel)
-//   B2g hi,lo [Hq][Hq]   B2g[i][o] = 0.2 * P1[o] * P[o][i]        (GEMM2: A operand = 1 + 4*maskbit, exact in tf32)
-//   A0g float4[Hq]       (A0w0, A0w1, A0w2, A0b) in generator order: unit 16*kb + 4*c + e sits at 16*kb + 4*e + c
-//   E1  float4[Hq]       (P1[o], P1[o]*A1w[o][0..2])
-//   sumV [4]             sum_o P1[o]*A1w[o][j]
-//   cnt  [2*kTc3MaxTiles] u32 per-(tile, cta rank) unit counters: zeroed by prepare, left zero by every launch
-//   -- B dependent --
-//   scr1 float4 [Bp][NP][2]  (h2 partial, tpos_0..2) per (row, pass, column half);  scr2 float4 same shape (X_0..2)
-//   imask u32 [Bp][Hq/32]    LeakyReLU bits of h1 when the caller does not ask for mask1
-//   cscr float4 [clusters][2 CTAs][2 halves][32][128 rows]   3xTF32 only: running sums of the K-chunked accumulation.  The
-//                            tensor core adds into its fp32 accumulator with truncation, a downward bias that grows with the
-//                            SQUARE of the accumulated K (measured on psi at H = 1024: 7.8e-6 / 1.2e-5 in one piece, 4.3e-6 /
-//                            5.6e-6 in chunks of 512, 2.1e-6 / 2.8e-6 in chunks of 256 -- "mixed" / "default" weights); the
-//                            forward therefore accumulates K in chunks of kTc3ChunkK, each in a fresh accumulator, and the
-//                            epilogue warps add the chunks with round-to-nearest FP32 adds.  A thread re-reads only what it
-//                            wrote itself; 256 KB per cluster, L2 resident.  Cost: the drain is a read-modify-write with
-//                            dependent L2 round trips (~8 us per chunk) and the MMA warp runs at most one chunk ahead, so a
-//                            chunk must outlast its predecessor's drain: 512-wide GEMM1 chunks do (12.5 us, +1 %), 256-wide
-//                            ones do not (+16 %).  Hence 512 (north_star's 1e-5 is met with 1.8x margin), GEMM1 only.
-constexpr int kTc3MaxTiles = 16384;
-constexpr int kTc3MaxClusters = 80;
-constexpr size_t k3ScrFloatsPerCta = (size_t)128 * 256;
-constexpr int kTc3ChunkK = 512;
-struct Tc3Layout {
-  int Hq, K1, NP, Bp;
-  size_t B1ahi, B1alo, B2ghi, B2glo, A0g, E1, sumV, cnt, fixed_end, scr1, scr2, imask, cscr, end;
-};
-inline Tc3Layout tc3_layout(int B, int d, int H) {
-  (void)d;
-  Tc3Layout T;
-  T.Hq = round_up(H, 256); T.K1 = T.Hq + 16; T.NP = T.Hq / 256; T.Bp = round_up(B, 256);
-  auto up = [](size_t x) { return (x + 63) / 64 * 64; };
-  size_t o = 0;
-  T.B1ahi = o; o += up((size_t)T.Hq * T.K1); T.B1alo = o; o += up((size_t)T.Hq * T.K1);
-  T.B2ghi = o; o += up((size_t)T.Hq * T.Hq); T.B2glo = o; o += up((size_t)T.Hq * T.Hq);
-  T.A0g = o; o += (size_t)4 * T.Hq; T.E1 = o; o += (size_t)4 * T.Hq;
-  T.sumV = o; o += 64;
-  T.cnt = o; o += (size_t)2 * kTc3MaxTiles;
-  T.fixed_end = o;
-  T.scr1 = o; o += (size_t)T.Bp * T.NP * 2 * 4;
-  T.scr2 = o; o += (size_t)T.Bp * T.NP * 2 * 4;
-  T.imask = o; o += (size_t)T.Bp * (T.Hq / 32);
-  {
-    const size_t units = (size_t)2 * (T.Bp / 256) * T.NP;
-    const size_t cl = units < (size_t)kTc3MaxClusters ? units : (size_t)kTc3MaxClusters;
-    T.cscr = o; o += cl * 2 * k3ScrFloatsPerCta;
-  }
-  T.end = o + 64;
-  return T;
-}
 
 template <int D>
 __device__ __forceinline__ float lin_of(const float4 q, const float (&z)[D]) {
@@ -192,13 +102,6 @@ __device__ __forceinline__ float lin_of(const float4 q, const float (&z)[D]) {
   h = fmaf(q.x, z[0], h);
   if (D > 1) h = fmaf(q.y, z[D > 1 ? 1 : 0], h);
   if (D > 2) h = fmaf(q.z, z[D > 2 ? 2 : 0], h);
-  return h;
-}
-template <int D>
-__device__ __forceinline__ float dot_of(const float4 q, const float (&v)[D]) {
-  float h = q.x * v[0];
-  if (D > 1) h = fmaf(q.y, v[D > 1 ? 1 : 0], h);
-  if (D > 2) h = fmaf(q.z, v[D > 2 ? 2 : 0], h);
   return h;
 }
 __device__ __forceinline__ float comp(const float4 q, int j) { return j == 0 ? q.x : (j == 1 ? q.y : q.z); }

@@ -14,7 +14,6 @@ image datasets, forward() accepts and ignores L, decode() needs no autograd grap
 from __future__ import annotations
 
 import math
-import os
 
 import torch
 import torch.nn.functional as F
@@ -436,7 +435,7 @@ class LIDVAE(VAE):
                 continue
             ops.icnn_prepare_early(params, ic.in_channel, ic.hidden_channel, ic._mode(), prec, input.shape[0], True, slot)
 
-    early_prepare = os.environ.get("B200VAE_EARLY_PREPARE", "1") != "0"      # A/B switch
+    early_prepare = True          # False: prepare inside the decoder call (the bit-identical reference arm of the tests)
 
     def _B_is_eye(self):
         v = self.__dict__.get("_b_eye_cache")

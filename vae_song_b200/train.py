@@ -9,8 +9,6 @@ DataParallelTrainer   one process per GPU: batch sharded by rank, parameters and
 """
 from __future__ import annotations
 
-import os
-
 import torch
 import torch.distributed as dist
 from torch import nn
@@ -216,7 +214,7 @@ class DataParallelTrainer:
         # step still captures into one CUDA graph (the reference's LR-VAE loop is otherwise host bound at its batch sizes)
         self.staged = bool(staged_backward)
         self.forward_kwargs = dict(forward_kwargs or {})       # e.g. {"L": 4}: num_mc_samples of main.py:259
-        self.defer_param_grads = os.environ.get("B200VAE_DEFER_PARAM_GRADS", "1") != "0"      # A/B switch
+        self.defer_param_grads = True  # False: one-call ICNN backward (the bit-identical reference arm of the tests)
         self._staged = None            # (host tensor, staging slot, copy-done event) of a prefetched batch (step_graphed)
         self._stage = None
         # lr_schedule = ("cosine", T_max): CosineAnnealingLR stepped after every optimiser step (main.py:201-203, 287),
