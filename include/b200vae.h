@@ -179,7 +179,8 @@ int b200vae_adam_step_sched(float* param, const float* grad, float* m, float* v,
  * LeakyReLU(BN(.)) is applied while loading.  `*_stats` == NULL means "raw input, no BN/activation".
  * `scratch`: b200vae_mlp_scratch_bytes(B) bytes of caller-owned device memory -- ordered per-CTA partials plus, in its last
  * 256 bytes, the ticket with which the LAST CTA of a layer kernel finalises the layer's statistics / sums / weight gradient
- * itself (no separate finalize launch on one GPU).  The ticket must be ZERO before the first call and is left zero by
+ * itself (no separate finalize launch on one GPU), and the grid-barrier counters of the stack entries below.  They must be
+ * ZERO before the first call and are left zero by
  * every call: zero-initialise the buffer once and reuse it (per stream). */
 size_t b200vae_mlp_scratch_bytes(int B);
 /* y_out [B,wo] = act(in) W^T + bias, W [wo,wi]; if stats_out != NULL also the batch statistics of y_out (and, when
@@ -199,6 +200,39 @@ int b200vae_mlp_layer_bwd(const float* dyhat, const float* y, const float* stats
                           const float* beta, const float* sums, float inv_n, float slope, const float* W,
                           const float* prev_y, const float* prev_stats, const float* prev_gamma,
                           const float* prev_beta, int B, int wo, int wi, float* da_prev, float* dW,
+                          void* scratch, void* stream);
+
+/* ---- a whole narrow stack in one launch per direction -----------------------------------------------------------------
+ * Layer l: y_l = act_{l-1}(y_{l-1}) W_l^T + bias_l with act = LeakyReLU(slope) . BatchNorm_l (y_{-1} = x, no act); every
+ * layer but the last feeds a BatchNorm.  Every wi, wo <= 8, 1 <= nl <= 16.  The kernels are cooperative (all CTAs
+ * co-resident; capturable into a CUDA graph) and use the same `scratch` as the layer entries above.  In training the
+ * forward gives the same bits as the layer entries at the same batch. */
+typedef struct {
+  const float* W;                 /* [wo][wi] */
+  const float* bias;              /* [wo] */
+  const float* gamma;             /* [wo] BatchNorm affine (not read for the last layer) */
+  const float* beta;
+  float* y;                       /* [B][wo] pre-BatchNorm output: written by the forward, read by the backward */
+  float* stats;                   /* [4][wo] (mean, biased var, invstd, count): training writes it, eval reads it */
+  float* running_mean;            /* training: momentum update (may be NULL) */
+  float* running_var;
+  long long* num_batches_tracked; /* training: += 1 (may be NULL) */
+  float eps, momentum;
+  int wi, wo;
+} b200vae_mlp_layer_t;
+typedef struct {
+  float* dW;                      /* [wo][wi] */
+  float* db;                      /* [wo]: exactly zero for a layer that feeds a BatchNorm */
+  float* dgamma;                  /* [wo] (not written for the last layer) */
+  float* dbeta;
+} b200vae_mlp_grad_t;
+/* head > 0 (2 head == last wo): mu [B][head] = y_last[:, :head] and lv [B][head] = softplus(y_last[:, head:]) as well. */
+int b200vae_mlp_stack_fwd(const b200vae_mlp_layer_t* layers, int nl, const float* x, int B, float slope, int training,
+                          int head, float* mu, float* lv, void* scratch, void* stream);
+/* Gradients of every parameter and (dx != NULL) of x.  head > 0: g0 = dL/dmu, g1 = dL/dlv [B][head] (NULL = zero), the
+ * softplus derivative is applied inside; head == 0: g0 = dL/dy_last [B][wo]. */
+int b200vae_mlp_stack_bwd(const b200vae_mlp_layer_t* layers, const b200vae_mlp_grad_t* grads, int nl, const float* x,
+                          int B, float slope, int training, int head, const float* g0, const float* g1, float* dx,
                           void* scratch, void* stream);
 
 /* ---- nearest-neighbour squared distances (chamfer_distance, model.py:896-912; SURVEY.md 8(f) rank 2) -------------------

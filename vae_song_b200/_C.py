@@ -33,7 +33,8 @@ EXPORTS = [
     "b200vae_peer_close", "b200vae_peer_free", "b200vae_peer_timed_out", "b200vae_peer_allgather", "b200vae_mlp_layer_fwd_peer",
     "b200vae_mlp_layer_bwd_reduce_peer", "b200vae_peer_allreduce_adam",
     "b200vae_icnn_wide_workspace_bytes", "b200vae_icnn_wide_fwd", "b200vae_icnn_wide_bwd", "b200vae_icnn_wide_bwd_psi",
-    "b200vae_mi_logqz", "b200vae_nll_iw_lse", "b200vae_nll_iw_scratch_bytes",
+    "b200vae_mi_logqz", "b200vae_nll_iw_lse", "b200vae_nll_iw_scratch_bytes", "b200vae_mlp_stack_fwd",
+    "b200vae_mlp_stack_bwd",
 ]
 PEER_MAX_WORLD, PEER_HANDLE_BYTES = 16, 64
 
@@ -53,6 +54,18 @@ class IcnnGrads(C.Structure):
 class PeerStruct(C.Structure):
     """b200vae_peer_t"""
     _fields_ = [("world", C.c_int), ("rank", C.c_int), ("buf", C.c_void_p * 16)]
+
+
+class MlpLayer(C.Structure):
+    """b200vae_mlp_layer_t"""
+    _fields_ = [(k, C.c_void_p) for k in ("W", "bias", "gamma", "beta", "y", "stats", "running_mean", "running_var",
+                                          "num_batches_tracked")] + \
+        [("eps", C.c_float), ("momentum", C.c_float), ("wi", C.c_int), ("wo", C.c_int)]
+
+
+class MlpGrad(C.Structure):
+    """b200vae_mlp_grad_t"""
+    _fields_ = [(k, C.c_void_p) for k in ("dW", "db", "dgamma", "dbeta")]
 
 
 PARAM_FIELDS = ("A0w", "A0b", "A1w", "A1b", "A2w", "A2b", "W0", "W1")
@@ -119,6 +132,10 @@ def load():
     lib.b200vae_mlp_layer_bwd_reduce.argtypes = [vp, vp, vp, vp, vp, f, i, i, vp, vp, vp, vp]
     lib.b200vae_mlp_layer_bwd.restype = i
     lib.b200vae_mlp_layer_bwd.argtypes = [vp, vp, vp, vp, vp, vp, f, f, vp, vp, vp, vp, vp, i, i, i, vp, vp, vp, vp]
+    lib.b200vae_mlp_stack_fwd.restype = i
+    lib.b200vae_mlp_stack_fwd.argtypes = [C.POINTER(MlpLayer), i, vp, i, f, i, i, vp, vp, vp, vp]
+    lib.b200vae_mlp_stack_bwd.restype = i
+    lib.b200vae_mlp_stack_bwd.argtypes = [C.POINTER(MlpLayer), C.POINTER(MlpGrad), i, vp, i, f, i, i, vp, vp, vp, vp, vp]
     lib.b200vae_nn_sqdist_fwd.restype = i
     lib.b200vae_nn_sqdist_fwd.argtypes = [vp, vp, i, i, i, i, vp, vp, vp]
     lib.b200vae_nn_sqdist_bwd.restype = i

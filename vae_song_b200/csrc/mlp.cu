@@ -876,8 +876,373 @@ mlp_rows_bwd_kernel(DyCtx c, ActSrc prev, const float* __restrict__ W, int B, fl
   }
 }
 
-static int narrow_class(int w) { return w <= 2 ? 2 : (w <= 4 ? 4 : (w <= 8 ? 8 : 0)); }
+__host__ __device__ __forceinline__ int narrow_class(int w) { return w <= 2 ? 2 : (w <= 4 ? 4 : (w <= 8 ? 8 : 0)); }
 static int narrow_grid(int B) { int g = (B + 255) / 256; return g > 592 ? 592 : (g < 1 ? 1 : g); }
+
+// ----------------------------------------------------------------------------------------- narrow stacks, one launch
+// When every layer of a stack is narrow the per-layer kernels above are bound by their chain of dependent launches (one
+// or two per layer and direction, each ending in a last-block finalize), not by the few MFLOP they do.  The stack kernels
+// run all layers in ONE cooperative launch: rows keep the thread mapping of mlp_narrow_*_kernel (row = blockIdx*256 +
+// tid, stride gridDim*256), and where the per-layer path finalises in the last block, every CTA waits at a grid barrier
+// and then combines the same ordered per-CTA partials itself, in the same fixed order, so all CTAs hold identical
+// statistics and the forward results are bit-identical to the per-layer path at the same grid.
+constexpr int kStackMaxLayers = 16;
+constexpr int kStackMaxGrid = 592;
+constexpr size_t kStackPartFloats = (size_t)2 * kStackMaxGrid * 128 * 3;      // two alternating partial buffers
+constexpr size_t kStackDwFloats = (size_t)kStackMaxGrid * 64 * kStackMaxLayers; // per-CTA dW partials of every layer
+constexpr size_t kStackDbFloats = (size_t)kStackMaxGrid * 8;                    // per-CTA bias-gradient partials, last layer
+static size_t stack_scratch_floats(int B) { return kStackPartFloats + kStackDwFloats + kStackDbFloats + (size_t)B * 8; }
+
+struct StackArgs {
+  b200vae_mlp_layer_t L[kStackMaxLayers];
+  b200vae_mlp_grad_t G[kStackMaxLayers];
+  int nl, B, training, head;   // head > 0: the last layer's output is (mu = cols [0, head), softplus(cols [head, 2 head)))
+  float slope;
+  const float* x;              // [B][L[0].wi]
+  float* out0; float* out1;    // forward: mu, lv (head) ; backward: unused
+  const float* g0; const float* g1;   // backward: g_mu, g_lv (head; either may be null = zero) or g_out in g0
+  float* dx;                   // backward: [B][L[0].wi] or null
+  float* scratch;
+  unsigned* bar;               // [0] barrier arrivals, [1] exit ticket: zero before the launch, left zero
+};
+
+__device__ __forceinline__ unsigned ld_acquire_gpu(const unsigned* p) {
+  unsigned v;
+  asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
+  return v;
+}
+// Grid-wide barrier.  Only valid in a cooperative launch (all CTAs co-resident).  The arrival counter only grows during a
+// launch (`epoch` = arrivals expected so far); stack_exit() resets it once every CTA is past its last barrier.
+__device__ __forceinline__ void grid_barrier(unsigned* count, unsigned& epoch) {
+  __syncthreads();
+  epoch += gridDim.x;
+  if (threadIdx.x == 0) {
+    __threadfence();
+    atomicAdd(count, 1u);
+    while (ld_acquire_gpu(count) < epoch) __nanosleep(32);
+    __threadfence();
+  }
+  __syncthreads();
+}
+__device__ __forceinline__ bool stack_exit(unsigned* bar) {
+  const bool last = last_block_arrives(bar + 1);
+  if (last && threadIdx.x == 0) bar[0] = 0u;
+  return last;
+}
+
+// layer input a[k] for row `row`: raw input or LeakyReLU(BN(previous y)) -- the arithmetic of mlp_narrow_*_kernel
+template <int WI>
+__device__ __forceinline__ void stack_act(float (&a)[WI], const ActSmem& am, bool has_bn, float slope, const float* y,
+                                          int wi, int row) {
+#pragma unroll
+  for (int k = 0; k < WI; ++k) a[k] = (k < wi) ? am.act(has_bn, slope, y[(size_t)row * wi + k], k) : 0.f;
+}
+
+template <int WI, int WO>
+__device__ __forceinline__ void stack_fwd_layer(const StackArgs& A, int l, const ActSmem& am, bool in_bn,
+                                                const float (*Ws)[8], const float* bs, bool do_stats,
+                                                float (*red)[8][3], float* part) {
+  const b200vae_mlp_layer_t& L = A.L[l];
+  const int wi = L.wi, wo = L.wo;
+  const float* src = l == 0 ? A.x : A.L[l - 1].y;
+  const bool last = l == A.nl - 1, head = last && A.head > 0;
+  float cnt = 0.f, mean[WO], m2[WO];
+#pragma unroll
+  for (int o = 0; o < WO; ++o) { mean[o] = 0.f; m2[o] = 0.f; }
+  for (int row = blockIdx.x * 256 + threadIdx.x; row < A.B; row += gridDim.x * 256) {
+    float a[WI];
+    stack_act<WI>(a, am, in_bn, A.slope, src, wi, row);
+    cnt += 1.f;
+#pragma unroll
+    for (int o = 0; o < WO; ++o) {
+      float yv = bs[o];
+#pragma unroll
+      for (int k = 0; k < WI; ++k) yv = fmaf(a[k], Ws[o][k], yv);
+      if (o < wo) {
+        L.y[(size_t)row * wo + o] = yv;
+        if (head) {      // torch.nn.functional.softplus (beta 1, threshold 20), the same expression as ATen's kernel
+          if (o < A.head) A.out0[(size_t)row * A.head + o] = yv;
+          else A.out1[(size_t)row * A.head + o - A.head] = yv > 20.f ? yv : log1pf(expf(yv));
+        }
+      }
+      const float dlt = yv - mean[o];                    // Welford
+      mean[o] += dlt / cnt;
+      m2[o] = fmaf(dlt, yv - mean[o], m2[o]);
+    }
+  }
+  if (!do_stats) return;
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+#pragma unroll
+  for (int o = 0; o < WO; ++o) {
+    float c = cnt, mu = mean[o], q = m2[o];
+#pragma unroll
+    for (int off = 16; off >= 1; off >>= 1) {
+      const float nb = __shfl_down_sync(0xffffffffu, c, off), mb = __shfl_down_sync(0xffffffffu, mu, off),
+                  qb = __shfl_down_sync(0xffffffffu, q, off);
+      chan_merge(c, mu, q, nb, mb, qb);
+    }
+    if (lane == 0) { red[warp][o][0] = c; red[warp][o][1] = mu; red[warp][o][2] = q; }
+  }
+  __syncthreads();
+  if (threadIdx.x < wo) {
+    float c = 0.f, mu = 0.f, q = 0.f;
+    for (int w8 = 0; w8 < 8; ++w8) chan_merge(c, mu, q, red[w8][threadIdx.x][0], red[w8][threadIdx.x][1], red[w8][threadIdx.x][2]);
+    float* o = part + ((size_t)blockIdx.x * 128 + threadIdx.x) * 3;
+    o[0] = c; o[1] = mu; o[2] = q;
+  }
+}
+
+// kMaxC: the widest layer class the kernel instantiation serves (4: only (2|4) x (2|4) bodies are compiled, which keeps
+// the register count -- and what the kernel leaves to concurrent kernels -- low)
+#define B200VAE_STACK_DISPATCH(kMaxC, FN, ci, co, ...)                                                     \
+  do {                                                                                                      \
+    if (ci == 2 && co == 2) FN<2, 2>(__VA_ARGS__); else if (ci == 2 && co == 4) FN<2, 4>(__VA_ARGS__);     \
+    else if (ci == 4 && co == 2) FN<4, 2>(__VA_ARGS__); else if (ci == 4 && co == 4) FN<4, 4>(__VA_ARGS__); \
+    else if constexpr (kMaxC == 8) {                                                                        \
+      if (ci == 2) FN<2, 8>(__VA_ARGS__); else if (ci == 4) FN<4, 8>(__VA_ARGS__);                          \
+      else if (co == 2) FN<8, 2>(__VA_ARGS__); else if (co == 4) FN<8, 4>(__VA_ARGS__);                     \
+      else FN<8, 8>(__VA_ARGS__);                                                                           \
+    }                                                                                                       \
+  } while (0)
+
+// Forward of a whole narrow stack.  Training: per BatchNorm layer one grid barrier, then every CTA combines the layer's
+// (count, mean, M2) partials with stats_finalize_block (the per-layer path's last-block code) into shared memory; CTA 0
+// also stores the statistics and updates running_mean / running_var / num_batches_tracked.  Eval: the statistics are read
+// from L[l].stats and no CTA waits for another.
+template <int kMaxC>
+__global__ void __launch_bounds__(256, kMaxC == 8 ? 2 : 4) mlp_stack_fwd_kernel(const StackArgs A) {
+  __shared__ ActSmem am;
+  __shared__ float Ws[kStackMaxLayers][8][8], bs[kStackMaxLayers][8];
+  __shared__ float red[8][8][3];
+  __shared__ float st[4 * 8];
+  for (int e = threadIdx.x; e < A.nl * 64; e += 256) {      // every layer's weights, zero-padded to 8 x 8
+    const int l = e >> 6, o = (e >> 3) & 7, k = e & 7;
+    const b200vae_mlp_layer_t& L = A.L[l];
+    Ws[l][o][k] = (o < L.wo && k < L.wi) ? L.W[o * L.wi + k] : 0.f;
+    if (k == 0) bs[l][o] = o < L.wo ? L.bias[o] : 0.f;
+  }
+  unsigned epoch = 0;
+  for (int l = 0; l < A.nl; ++l) {
+    const b200vae_mlp_layer_t& L = A.L[l];
+    const bool in_bn = l > 0;
+    __syncthreads();                                          // weights loaded / previous layer's ActSmem in place
+    const bool do_stats = A.training && l < A.nl - 1;
+    float* part = A.scratch + (size_t)(l & 1) * kStackMaxGrid * 128 * 3;
+    B200VAE_STACK_DISPATCH(kMaxC, stack_fwd_layer, narrow_class(L.wi), narrow_class(L.wo), A, l, am, in_bn, Ws[l], bs[l],
+                           do_stats, red, part);
+    if (l == A.nl - 1) break;
+    const int wo = L.wo;
+    if (do_stats) {
+      grid_barrier(A.bar, epoch);
+      StatsFin f;
+      f.stats = st; f.eps = L.eps; f.momentum = L.momentum; f.peer = 0;
+      f.running_mean = blockIdx.x == 0 ? L.running_mean : nullptr;
+      f.running_var = blockIdx.x == 0 ? L.running_var : nullptr;
+      stats_finalize_block(part, (int)gridDim.x, wo, f);
+      __syncthreads();
+      if (blockIdx.x == 0) {
+        if (threadIdx.x < 4 * wo) L.stats[threadIdx.x] = st[threadIdx.x];
+        if (threadIdx.x == 0 && L.num_batches_tracked) *L.num_batches_tracked += 1;
+      }
+    } else if (threadIdx.x < 4 * wo) {
+      st[threadIdx.x] = L.stats[threadIdx.x];
+    }
+    __syncthreads();
+    if (threadIdx.x < 128) {                                  // the next layer's input transform
+      const int k = threadIdx.x;
+      const bool in = k < wo;
+      am.mean[k] = in ? st[k] : 0.f; am.invstd[k] = in ? st[2 * wo + k] : 0.f;
+      am.gamma[k] = in ? L.gamma[k] : 0.f; am.beta[k] = in ? L.beta[k] : 0.f;
+    }
+  }
+  if (A.training) stack_exit(A.bar);
+}
+
+// Backward, phase 1 of layer l: dyhat = da * lrelu'(.) and the per-CTA (S1, S2) partials.  da of the last layer comes
+// from the caller's gradients (softplus' applied to the lv half, the expression of ATen's softplus_backward); the
+// others from the rows buffer that phase 2 of layer l + 1 filled (each thread only touches its own rows).
+template <int WO>
+__device__ __forceinline__ void stack_dyhat(const StackArgs& A, int l, const ActSmem& am, int row, float (&g)[WO],
+                                            float (&xh)[WO]) {
+  const b200vae_mlp_layer_t& L = A.L[l];
+  const int wo = L.wo;
+  const bool has_bn = l < A.nl - 1;
+  const float* da_rows = A.scratch + kStackPartFloats + kStackDwFloats + kStackDbFloats;
+#pragma unroll
+  for (int o = 0; o < WO; ++o) {
+    float d = 0.f, yv = 0.f;
+    if (o < wo) {
+      if (has_bn) yv = L.y[(size_t)row * wo + o];
+      if (l < A.nl - 1) {
+        d = da_rows[(size_t)row * 8 + o];
+      } else if (A.head == 0) {
+        d = A.g0[(size_t)row * wo + o];
+      } else if (o < A.head) {
+        d = A.g0 ? A.g0[(size_t)row * A.head + o] : 0.f;
+      } else {
+        const float gl = A.g1 ? A.g1[(size_t)row * A.head + o - A.head] : 0.f;
+        const float x = L.y[(size_t)row * wo + o], z = expf(x);
+        d = x > 20.f ? gl : gl * z / (z + 1.f);
+      }
+    }
+    xh[o] = 0.f;
+    if (has_bn) {
+      xh[o] = am.xhat(yv, o);
+      const float t = fmaf(xh[o], am.gamma[o], am.beta[o]);
+      d = t > 0.f ? d : A.slope * d;
+    }
+    g[o] = d;
+  }
+}
+
+template <int WO>
+__device__ __forceinline__ void stack_bwd_sums(const StackArgs& A, int l, const ActSmem& am, float (*red)[8][2],
+                                               float* part) {
+  const int wo = A.L[l].wo;
+  float s1[WO], s2[WO];
+#pragma unroll
+  for (int o = 0; o < WO; ++o) { s1[o] = 0.f; s2[o] = 0.f; }
+  for (int row = blockIdx.x * 256 + threadIdx.x; row < A.B; row += gridDim.x * 256) {
+    float g[WO], xh[WO];
+    stack_dyhat<WO>(A, l, am, row, g, xh);
+#pragma unroll
+    for (int o = 0; o < WO; ++o) { s1[o] += g[o]; s2[o] = fmaf(g[o], xh[o], s2[o]); }
+  }
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+#pragma unroll
+  for (int o = 0; o < WO; ++o) {
+    const float a = warp_sum(s1[o]), b = warp_sum(s2[o]);
+    if (lane == 0) { red[warp][o][0] = a; red[warp][o][1] = b; }
+  }
+  __syncthreads();
+  if (threadIdx.x < wo) {
+    float a = 0.f, b = 0.f;
+    for (int w8 = 0; w8 < 8; ++w8) { a += red[w8][threadIdx.x][0]; b += red[w8][threadIdx.x][1]; }
+    part[((size_t)blockIdx.x * 128 + threadIdx.x) * 2 + 0] = a;
+    part[((size_t)blockIdx.x * 128 + threadIdx.x) * 2 + 1] = b;
+  }
+}
+
+// Backward, phase 2 of layer l: dy from dyhat and the global sums, da_prev = dy W into the rows buffer (or dx), and the
+// per-CTA dW partial (warp -> block, fixed order)
+template <int WI, int WO>
+__device__ __forceinline__ void stack_bwd_layer(const StackArgs& A, int l, const ActSmem& am, const ActSmem& pm,
+                                                const float (*Ws)[8], const float* s1, const float* s2, float invN,
+                                                float* red) {
+  const b200vae_mlp_layer_t& L = A.L[l];
+  const int wo = L.wo, wi = L.wi;
+  const bool has_bn = l < A.nl - 1;
+  const float* src = l == 0 ? A.x : A.L[l - 1].y;
+  float* da_rows = A.scratch + kStackPartFloats + kStackDwFloats + kStackDbFloats;
+  float acc[WO][WI];
+#pragma unroll
+  for (int o = 0; o < WO; ++o)
+#pragma unroll
+    for (int k = 0; k < WI; ++k) acc[o][k] = 0.f;
+  for (int row = blockIdx.x * 256 + threadIdx.x; row < A.B; row += gridDim.x * 256) {
+    float g[WO], xh[WO], dy[WO], a[WI], dap[WI];
+    stack_dyhat<WO>(A, l, am, row, g, xh);
+#pragma unroll
+    for (int o = 0; o < WO; ++o)
+      dy[o] = (o < wo && has_bn) ? am.gamma[o] * am.invstd[o] * (g[o] - s1[o] * invN - xh[o] * (s2[o] * invN)) : g[o];
+    stack_act<WI>(a, pm, l > 0, A.slope, src, wi, row);
+#pragma unroll
+    for (int k = 0; k < WI; ++k) dap[k] = 0.f;
+#pragma unroll
+    for (int o = 0; o < WO; ++o)
+#pragma unroll
+      for (int k = 0; k < WI; ++k) { dap[k] = fmaf(dy[o], Ws[o][k], dap[k]); acc[o][k] = fmaf(dy[o], a[k], acc[o][k]); }
+    if (l > 0) {
+#pragma unroll
+      for (int k = 0; k < WI; ++k) if (k < wi) da_rows[(size_t)row * 8 + k] = dap[k];
+    } else if (A.dx) {
+#pragma unroll
+      for (int k = 0; k < WI; ++k) if (k < wi) A.dx[(size_t)row * wi + k] = dap[k];
+    }
+  }
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+#pragma unroll
+  for (int o = 0; o < WO; ++o)
+#pragma unroll
+    for (int k = 0; k < WI; ++k) {
+      const float v = warp_sum(acc[o][k]);
+      if (lane == 0) red[warp * 64 + o * WI + k] = v;
+    }
+  __syncthreads();
+  if (threadIdx.x < WO * WI) {
+    const int o = threadIdx.x / WI, k = threadIdx.x % WI;
+    float v = 0.f;
+    for (int w8 = 0; w8 < 8; ++w8) v += red[w8 * 64 + threadIdx.x];
+    float* part = A.scratch + kStackPartFloats + (size_t)l * kStackMaxGrid * 64;
+    if (o < wo && k < wi) part[(size_t)blockIdx.x * wo * wi + o * wi + k] = v;
+  }
+}
+
+__device__ __forceinline__ void stack_load_act(ActSmem& s, const b200vae_mlp_layer_t& L) {
+  if (threadIdx.x < 128) {
+    const int k = threadIdx.x, w = L.wo;
+    const bool in = k < w;
+    s.mean[k] = in ? L.stats[k] : 0.f; s.invstd[k] = in ? L.stats[2 * w + k] : 0.f;
+    s.gamma[k] = in ? L.gamma[k] : 0.f; s.beta[k] = in ? L.beta[k] : 0.f;
+  }
+}
+
+// Backward of a whole narrow stack, layers in reverse.  Per BatchNorm layer one grid barrier between the (S1, S2)
+// partials and their fixed-order combine (sums_finalize_column, in every CTA); CTA 0 stores dbeta = S1, dgamma = S2 and
+// the exactly-zero gradient of the bias that feeds the BatchNorm.  dW of every layer and the last layer's bias gradient
+// are reduced once, by the last CTA to leave, in fixed order (dw_finalize_block).
+template <int kMaxC>
+__global__ void __launch_bounds__(256, kMaxC == 8 ? 2 : 4) mlp_stack_bwd_kernel(const StackArgs A) {
+  __shared__ ActSmem am, pm;
+  __shared__ float Ws[8][8], s1[8], s2[8], sums[2 * 8];
+  __shared__ float red[8 * 64];
+  unsigned epoch = 0;
+  const float invN = 1.f / (float)A.B;
+  float* dbpart = A.scratch + kStackPartFloats + kStackDwFloats;
+  for (int l = A.nl - 1; l >= 0; --l) {
+    const b200vae_mlp_layer_t& L = A.L[l];
+    const int wo = L.wo, wi = L.wi;
+    const bool has_bn = l < A.nl - 1;
+    __syncthreads();                                          // the previous layer is done with the shared arrays
+    if (has_bn) stack_load_act(am, L);
+    if (l > 0) stack_load_act(pm, A.L[l - 1]);
+    if (threadIdx.x < 64) {
+      const int o = threadIdx.x >> 3, k = threadIdx.x & 7;
+      Ws[o][k] = (o < wo && k < wi) ? L.W[o * wi + k] : 0.f;
+    }
+    __syncthreads();
+    float* part = A.scratch + (size_t)(l & 1) * kStackMaxGrid * 128 * 2;
+    const int co = narrow_class(wo);
+    float (*red2)[8][2] = reinterpret_cast<float (*)[8][2]>(red);
+    if (co == 2) stack_bwd_sums<2>(A, l, am, red2, part);
+    else if (co == 4) stack_bwd_sums<4>(A, l, am, red2, part);
+    else if constexpr (kMaxC == 8) stack_bwd_sums<8>(A, l, am, red2, part);
+    if (has_bn) {
+      grid_barrier(A.bar, epoch);
+      for (int n = threadIdx.x >> 5; n < wo; n += 8) sums_finalize_column(part, (int)gridDim.x, wo, n, sums);
+      __syncthreads();
+      if (threadIdx.x < wo) {
+        const int n = threadIdx.x;
+        if (blockIdx.x == 0) { A.G[l].dbeta[n] = sums[n]; A.G[l].dgamma[n] = sums[wo + n]; A.G[l].db[n] = 0.f; }
+        s1[n] = A.training ? sums[n] : 0.f;          // eval-mode BatchNorm is affine: dy = gamma*invstd*dyhat
+        s2[n] = A.training ? sums[wo + n] : 0.f;
+      }
+    } else {
+      __syncthreads();
+      if (threadIdx.x < wo) dbpart[(size_t)blockIdx.x * wo + threadIdx.x] = part[((size_t)blockIdx.x * 128 + threadIdx.x) * 2];
+    }
+    __syncthreads();
+    B200VAE_STACK_DISPATCH(kMaxC, stack_bwd_layer, narrow_class(wi), co, A, l, am, pm, Ws, s1, s2, invN, red);
+  }
+  if (stack_exit(A.bar)) {
+    for (int l = 0; l < A.nl; ++l) {
+      const float* part = A.scratch + kStackPartFloats + (size_t)l * kStackMaxGrid * 64;
+      dw_finalize_block(part, (int)gridDim.x, A.L[l].wo * A.L[l].wi, A.G[l].dW);
+    }
+    const int wo = A.L[A.nl - 1].wo;
+    dw_finalize_block(dbpart, (int)gridDim.x, wo, A.G[A.nl - 1].db);
+  }
+}
 
 template <int WI, int WO>
 static void narrow_fwd_launch(const ActSrc& src, const float* W, const float* bias, int B, int wo, float* y, float* part,
@@ -915,7 +1280,8 @@ static size_t mlp_scratch_floats(int B) {
   const size_t a = (ncta > 592 ? ncta : 592) * 128 * 3, b = (size_t)296 * 128 * 2, c = (size_t)296 * 128 * 128;
   size_t m = a > b ? a : b;
   if (c > m) m = c;
-  return m;
+  const size_t s = stack_scratch_floats(B);
+  return s > m ? s : m;
 }
 // partials, then 64 floats holding the last-block ticket (must be zero before the first call; every call leaves it zero),
 // then the staging area of the fused cross-rank exchange (this rank's values + every rank's)
@@ -1080,4 +1446,83 @@ extern "C" int b200vae_mlp_layer_bwd(const float* dyhat, const float* y, const f
     rc = check_launch();
   }
   return rc;
+}
+
+// ----------------------------------------------------------------------------------------- narrow stacks
+static bool stack_shape_ok(const b200vae_mlp_layer_t* L, int nl, int B, bool need_stats) {
+  if (!L || nl < 1 || nl > kStackMaxLayers || B <= 0) return false;
+  for (int l = 0; l < nl; ++l) {
+    if (L[l].wi < 1 || L[l].wi > 8 || L[l].wo < 1 || L[l].wo > 8) return false;
+    if (l > 0 && L[l].wi != L[l - 1].wo) return false;
+    if (!L[l].W || !L[l].bias || !L[l].y) return false;
+    if (l < nl - 1 && (!L[l].gamma || !L[l].beta || (need_stats && !L[l].stats))) return false;
+  }
+  return true;
+}
+static int stack_max_class(const b200vae_mlp_layer_t* L, int nl) {
+  int c = 2;
+  for (int l = 0; l < nl; ++l) c = max(c, max(narrow_class(L[l].wi), narrow_class(L[l].wo)));
+  return c;
+}
+// The grid of the per-layer narrow kernels (so the statistics are combined from the same partials), clamped to what
+// the occupancy API says fits co-resident: the grid barrier needs every CTA running at once.
+template <int kMaxC>
+static int stack_grid(int B) {
+  static int cap = 0;
+  if (cap == 0) {
+    int f = 0, b = 0;
+    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&f, mlp_stack_fwd_kernel<kMaxC>, 256, 0);
+    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&b, mlp_stack_bwd_kernel<kMaxC>, 256, 0);
+    cap = (f < b ? f : b) * sm_count();
+    if (cap <= 0) return 0;
+  }
+  const int g = narrow_grid(B);
+  return g < cap ? g : cap;
+}
+template <typename Kernel>
+static int stack_launch(Kernel kernel, const StackArgs& A, int grid, void* stream) {
+  if (grid <= 0) return B200VAE_ECUDA;
+  cudaLaunchConfig_t cfg = {};
+  cfg.gridDim = dim3(grid); cfg.blockDim = dim3(256); cfg.dynamicSmemBytes = 0; cfg.stream = (cudaStream_t)stream;
+  cudaLaunchAttribute attr[1];
+  attr[0].id = cudaLaunchAttributeCooperative; attr[0].val.cooperative = 1;
+  cfg.attrs = attr; cfg.numAttrs = 1;
+  const cudaError_t e = cudaLaunchKernelEx(&cfg, kernel, A);
+  if (e != cudaSuccess) { g_last_cuda_error = (int)e; ++g_launch_count; return B200VAE_ECUDA; }
+  return check_launch();
+}
+static StackArgs stack_args(const b200vae_mlp_layer_t* layers, int nl, const float* x, int B, float slope, int training,
+                            int head, void* scratch) {
+  StackArgs A;
+  memset(&A, 0, sizeof(A));
+  for (int l = 0; l < nl; ++l) A.L[l] = layers[l];
+  A.nl = nl; A.B = B; A.training = training ? 1 : 0; A.head = head; A.slope = slope; A.x = x;
+  A.scratch = (float*)scratch; A.bar = mlp_ticket(scratch, B) + 1;    // [0] stays the layer kernels' last-block ticket
+  return A;
+}
+
+extern "C" int b200vae_mlp_stack_fwd(const b200vae_mlp_layer_t* layers, int nl, const float* x, int B, float slope,
+                                     int training, int head, float* mu, float* lv, void* scratch, void* stream) {
+  if (!x || !scratch) return B200VAE_EALIGN;
+  if (!stack_shape_ok(layers, nl, B, !training)) return B200VAE_ESHAPE;
+  if (head < 0 || (head > 0 && (2 * head != layers[nl - 1].wo || !mu || !lv))) return B200VAE_ESHAPE;
+  StackArgs A = stack_args(layers, nl, x, B, slope, training, head, scratch);
+  A.out0 = mu; A.out1 = lv;
+  if (stack_max_class(layers, nl) == 8) return stack_launch(mlp_stack_fwd_kernel<8>, A, stack_grid<8>(B), stream);
+  return stack_launch(mlp_stack_fwd_kernel<4>, A, stack_grid<4>(B), stream);
+}
+
+extern "C" int b200vae_mlp_stack_bwd(const b200vae_mlp_layer_t* layers, const b200vae_mlp_grad_t* grads, int nl,
+                                     const float* x, int B, float slope, int training, int head, const float* g0,
+                                     const float* g1, float* dx, void* scratch, void* stream) {
+  if (!x || !scratch || !grads) return B200VAE_EALIGN;
+  if (!stack_shape_ok(layers, nl, B, true)) return B200VAE_ESHAPE;
+  if (head < 0 || (head > 0 && 2 * head != layers[nl - 1].wo) || (head == 0 && !g0)) return B200VAE_ESHAPE;
+  for (int l = 0; l < nl; ++l)
+    if (!grads[l].dW || !grads[l].db || (l < nl - 1 && (!grads[l].dgamma || !grads[l].dbeta))) return B200VAE_EALIGN;
+  StackArgs A = stack_args(layers, nl, x, B, slope, training, head, scratch);
+  for (int l = 0; l < nl; ++l) A.G[l] = grads[l];
+  A.g0 = g0; A.g1 = g1; A.dx = dx;
+  if (stack_max_class(layers, nl) == 8) return stack_launch(mlp_stack_bwd_kernel<8>, A, stack_grid<8>(B), stream);
+  return stack_launch(mlp_stack_bwd_kernel<4>, A, stack_grid<4>(B), stream);
 }

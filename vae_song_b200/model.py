@@ -401,7 +401,9 @@ class LIDVAE(VAE):
         # the plan caches module references: rebuild it if BatchNorms were swapped (e.g. SyncBatchNorm conversion)
         if plan is not None and any(b is not blk[1] for b, blk in zip(plan.bns, self.encoder)):
             self.__dict__["_mlp_plan"] = plan = ops.MlpPlan.from_sequential(self.encoder)
-        ret = ops.fused_mlp(plan, input, self.training) if plan is not None else self.encoder(input)
+        if plan is not None:
+            return ops.fused_mlp(plan, input, self.training, softplus_head=True)
+        ret = self.encoder(input)
         mu, var = ret.split(ret.shape[1] // 2, 1)
         return mu, F.softplus(var)
 

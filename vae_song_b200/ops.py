@@ -842,13 +842,126 @@ class FusedMlpFn(torch.autograd.Function):
         return (da if ctx.needs_input_grad[0] else None, None, None, *flat)
 
 
-def fused_mlp(plan, x, training):
+STACK_MAX_WIDTH, STACK_MAX_LAYERS = 8, 16
+
+
+def _stack_ok(plan, training):
+    """Every layer narrow and no cross-rank BatchNorm: the whole stack runs as one launch per direction."""
+    lin = plan.linears
+    if len(lin) > STACK_MAX_LAYERS or any(l.in_features > STACK_MAX_WIDTH or l.out_features > STACK_MAX_WIDTH for l in lin):
+        return False
+    return not (training and any(_bn_group(b) is not None for b in plan.bns))
+
+
+def _stack_layers(plan, ys, stats, Ws, bs, gs, bes, training):
+    nl = len(Ws)
+    arr = (_C.MlpLayer * nl)()
+    for i in range(nl):
+        L = arr[i]
+        wo, wi = Ws[i].shape
+        L.W, L.bias, L.y, L.wi, L.wo = _ptr(Ws[i]), _ptr(bs[i]), _ptr(ys[i]), wi, wo
+        if i < nl - 1:
+            bn = plan.bns[i]
+            L.gamma, L.beta, L.stats, L.eps, L.momentum = _ptr(gs[i]), _ptr(bes[i]), _ptr(stats[i]), float(bn.eps), float(bn.momentum)
+            if training:
+                L.running_mean, L.running_var = _ptr(bn.running_mean), _ptr(bn.running_var)
+                L.num_batches_tracked = _ptr(bn.num_batches_tracked)
+    return arr
+
+
+class FusedMlpStackFn(torch.autograd.Function):
+    """FusedMlpFn for a stack whose layers are all at most 8 wide: one cooperative launch per direction
+    (b200vae_mlp_stack_fwd / _bwd).  head > 0: returns (mu, softplus(var)) -- the two halves of the last layer's output,
+    the second through F.softplus -- instead of the output itself."""
+
+    @staticmethod
+    def forward(ctx, x, plan, training, head, *params):
+        lib = _C.load()
+        x = _req(x, "x")
+        B, dev = x.shape[0], x.device
+        nl = len(plan.linears)
+        Ws = [_req(params[2 * i], "W") for i in range(nl)]
+        bs = [_req(params[2 * i + 1], "b") for i in range(nl)]
+        gs = [_req(params[2 * nl + 2 * i], "gamma") for i in range(nl - 1)]
+        bes = [_req(params[2 * nl + 2 * i + 1], "beta") for i in range(nl - 1)]
+        scratch = _mlp_scratch(lib.b200vae_mlp_scratch_bytes(B), dev)
+        ys = [torch.empty(B, W.shape[0], dtype=torch.float32, device=dev) for W in Ws]
+        stats = [torch.empty(4, W.shape[0], dtype=torch.float32, device=dev) for W in Ws[:nl - 1]]
+        if not training:                  # eval: running statistics are constants
+            for st, bn in zip(stats, plan.bns):
+                st[0].copy_(bn.running_mean); st[1].copy_(bn.running_var)
+                st[2].copy_(torch.rsqrt(bn.running_var + bn.eps)); st[3].fill_(float(B))
+        layers = _stack_layers(plan, ys, stats, Ws, bs, gs, bes, training)
+        mu = lv = None
+        if head:
+            mu = torch.empty(B, head, dtype=torch.float32, device=dev)
+            lv = torch.empty(B, head, dtype=torch.float32, device=dev)
+        _C.check(lib.b200vae_mlp_stack_fwd(layers, nl, _ptr(x), B, plan.slope, int(training), head, _ptr(mu), _ptr(lv),
+                                           _ptr(scratch), _stream()), "mlp_stack_fwd")
+        ctx.plan, ctx.training, ctx.nl, ctx.head = plan, training, nl, head
+        ctx.save_for_backward(x, *ys, *stats, *Ws, *bs, *gs, *bes)
+        ctx.scratch = scratch
+        ctx.set_materialize_grads(False)
+        return (mu, lv) if head else ys[-1]
+
+    @staticmethod
+    @torch.autograd.function.once_differentiable
+    def backward(ctx, *grads):
+        lib = _C.load()
+        plan, training, nl, head = ctx.plan, ctx.training, ctx.nl, ctx.head
+        sv = ctx.saved_tensors
+        x = sv[0]; ys = sv[1:1 + nl]; stats = sv[1 + nl:2 * nl]; Ws = sv[2 * nl:3 * nl]; bs = sv[3 * nl:4 * nl]
+        gs = sv[4 * nl:5 * nl - 1]; bes = sv[5 * nl - 1:6 * nl - 2]
+        B = x.shape[0]
+        g0 = _req(grads[0], "grad_out") if grads[0] is not None else None
+        g1 = _req(grads[1], "grad_out") if head and grads[1] is not None else None
+        if not head and g0 is None:
+            g0 = torch.zeros_like(ys[-1])
+        # every parameter gradient in one buffer, written completely by the kernel (zeros included)
+        sizes = []
+        for i in range(nl):
+            wo, wi = Ws[i].shape
+            sizes += [wo * wi, wo] + ([wo, wo] if i < nl - 1 else [])
+        flat = torch.empty(sum(sizes), dtype=torch.float32, device=x.device)
+        parts = list(flat.split(sizes))
+        garr = (_C.MlpGrad * nl)()
+        dWs, dbs, dgs, dbes = [], [], [], []
+        for i in range(nl):
+            wo, wi = Ws[i].shape
+            dW, db = parts.pop(0).view(wo, wi), parts.pop(0)
+            garr[i].dW, garr[i].db = _ptr(dW), _ptr(db)
+            dWs.append(dW); dbs.append(db)
+            if i < nl - 1:
+                dg, dbe = parts.pop(0), parts.pop(0)
+                garr[i].dgamma, garr[i].dbeta = _ptr(dg), _ptr(dbe)
+                dgs.append(dg); dbes.append(dbe)
+        dx = torch.empty_like(x) if ctx.needs_input_grad[0] else None
+        layers = _stack_layers(plan, ys, stats, Ws, bs, gs, bes, False)
+        _C.check(lib.b200vae_mlp_stack_bwd(layers, garr, nl, _ptr(x), B, plan.slope, int(training), head, _ptr(g0),
+                                           _ptr(g1), _ptr(dx), _ptr(ctx.scratch), _stream()), "mlp_stack_bwd")
+        out = []
+        for i in range(nl):
+            out += [dWs[i], dbs[i]]
+        for i in range(nl - 1):
+            out += [dgs[i], dbes[i]]
+        return (dx, None, None, None, *out)
+
+
+def fused_mlp(plan, x, training, softplus_head=False):
+    """Output of the stack; softplus_head: (mu, softplus(var)) of its two halves (LIDVAE.encode)."""
     params = []
     for l in plan.linears:
         params += [l.weight, l.bias]
     for b in plan.bns:
         params += [b.weight, b.bias]
-    return FusedMlpFn.apply(x, plan, training, *params)
+    if _stack_ok(plan, training):
+        head = plan.linears[-1].out_features // 2 if softplus_head else 0
+        return FusedMlpStackFn.apply(x, plan, training, head, *params)
+    out = FusedMlpFn.apply(x, plan, training, *params)
+    if not softplus_head:
+        return out
+    mu, var = out.split(out.shape[1] // 2, 1)
+    return mu, torch.nn.functional.softplus(var)
 
 
 # ------------------------------------------------------------------------------------------ chamfer
