@@ -28,6 +28,14 @@ struct ActSrc {          // how a layer input a[b][k] is obtained from the previ
   float slope;
 };
 
+__host__ __device__ __forceinline__ ActSrc make_src(const float* y, const float* stats, const float* gamma,
+                                                    const float* beta, int w, float slope) {
+  ActSrc s;
+  s.y = y; s.w = w; s.slope = slope;
+  s.mean = stats; s.invstd = stats ? stats + 2 * w : nullptr; s.gamma = gamma; s.beta = beta;
+  return s;
+}
+
 struct ActSmem {
   float mean[128], invstd[128], gamma[128], beta[128];
   __device__ __forceinline__ void load(const ActSrc& s) {
@@ -116,6 +124,19 @@ struct StatsFin {      // stats == nullptr: no fused finalize (a finalize kernel
 struct SumsFin { float* sums; unsigned* ticket; int peer, slot; float* sums_global; float* stage; PeerComm comm; };
 struct DwFin { float* dW; unsigned* ticket; };
 
+// The merged (count, mean, M2) of column n -> stats[4][w] = mean, biased var, invstd, count, and (with running_mean) the
+// momentum update of the running statistics.  The update is written with explicit roundings: left to the compiler, the
+// products were contracted into an FMA differently depending on the kernel this is inlined into.
+__device__ __forceinline__ void stats_store(const StatsFin& f, int w, int n, float cnt, float mean, float m2) {
+  const float var = m2 / cnt;
+  f.stats[n] = mean; f.stats[w + n] = var; f.stats[2 * w + n] = rsqrtf(var + f.eps); f.stats[3 * w + n] = cnt;
+  if (f.running_mean) {
+    const float keep = __fsub_rn(1.f, f.momentum);
+    f.running_mean[n] = __fmaf_rn(f.momentum, mean, __fmul_rn(keep, f.running_mean[n]));
+    f.running_var[n] = __fmaf_rn(f.momentum, m2 / fmaxf(cnt - 1.f, 1.f), __fmul_rn(keep, f.running_var[n]));
+  }
+}
+
 // ----------------------------------------------------------------------------------------- forward
 // part: [nCTA][128][3] = (count, mean, M2) of this CTA's rows per output column
 __device__ __forceinline__ void chan_merge(float& cnt, float& mean, float& m2, float nb, float mb, float m2b);
@@ -177,10 +198,18 @@ __device__ __forceinline__ void chan_merge(float& cnt, float& mean, float& m2, f
   }
   cnt = tot;
 }
+// the fixed-order shuffle tree: lane 0 ends with the merge of the warp's 32 triples
+__device__ __forceinline__ void chan_warp_merge(float& cnt, float& mean, float& m2) {
+#pragma unroll
+  for (int off = 16; off >= 1; off >>= 1) {
+    const float nb = __shfl_down_sync(0xffffffffu, cnt, off), mb = __shfl_down_sync(0xffffffffu, mean, off),
+                m2b = __shfl_down_sync(0xffffffffu, m2, off);
+    chan_merge(cnt, mean, m2, nb, mb, m2b);
+  }
+}
 // column n by one warp: lanes stride over the CTAs' partials (L2 loads), fixed-order shuffle tree
-__device__ __forceinline__ void stats_finalize_column(const float* __restrict__ part, int ncta, int w, int n, float eps,
-                                                      float* __restrict__ stats, float* __restrict__ running_mean,
-                                                      float* __restrict__ running_var, float momentum) {
+__device__ __forceinline__ void stats_finalize_column(const float* __restrict__ part, int ncta, int w, int n,
+                                                      const StatsFin& f) {
   const int lane = threadIdx.x & 31;
   float cnt = 0.f, mean = 0.f, m2 = 0.f;
   for (int c0 = lane; c0 < ncta; c0 += 4 * 32) {   // 4 partial triples per lane in flight per L2 round trip, merged in order
@@ -195,29 +224,17 @@ __device__ __forceinline__ void stats_finalize_column(const float* __restrict__ 
 #pragma unroll
     for (int j = 0; j < 4; ++j) chan_merge(cnt, mean, m2, pc[j], pm[j], pq[j]);     // a zero count is the identity
   }
-#pragma unroll
-  for (int off = 16; off >= 1; off >>= 1) {
-    const float nb = __shfl_down_sync(0xffffffffu, cnt, off), mb = __shfl_down_sync(0xffffffffu, mean, off),
-                m2b = __shfl_down_sync(0xffffffffu, m2, off);
-    chan_merge(cnt, mean, m2, nb, mb, m2b);
-  }
-  if (lane == 0) {
-    const float var = m2 / cnt;
-    stats[n] = mean; stats[w + n] = var; stats[2 * w + n] = rsqrtf(var + eps); stats[3 * w + n] = cnt;
-    if (running_mean) {
-      running_mean[n] = (1.f - momentum) * running_mean[n] + momentum * mean;
-      running_var[n] = (1.f - momentum) * running_var[n] + momentum * (m2 / fmaxf(cnt - 1.f, 1.f));
-    }
-  }
+  chan_warp_merge(cnt, mean, m2);
+  if (lane == 0) stats_store(f, w, n, cnt, mean, m2);
 }
 __global__ void __launch_bounds__(256)
-mlp_stats_finalize_kernel(const float* __restrict__ part, int ncta, int w, float eps, float* __restrict__ stats,
-                          float* __restrict__ running_mean, float* __restrict__ running_var, float momentum) {
+mlp_stats_finalize_kernel(const float* __restrict__ part, int ncta, int w, StatsFin fin) {
   const int n = blockIdx.x * 8 + (threadIdx.x >> 5);
   if (n >= w) return;
-  stats_finalize_column(part, ncta, w, n, eps, stats, running_mean, running_var, momentum);
+  stats_finalize_column(part, ncta, w, n, fin);
 }
-// the same, executed by the last CTA of the producing kernel (all its warps, columns round-robin)
+// the same, executed by ONE CTA (all its warps, columns round-robin): the last CTA of the producing kernel, or the
+// stand-alone cross-rank finalize below
 __device__ __forceinline__ void stats_finalize_block(const float* __restrict__ part, int ncta, int w, const StatsFin& f) {
   if (f.peer) {                // cross-rank: local (count, mean, M2) per column -> exchange -> Chan merge in rank order
     float* mine = f.stage;
@@ -229,12 +246,7 @@ __device__ __forceinline__ void stats_finalize_block(const float* __restrict__ p
         const float* p = part + ((size_t)c * 128 + n) * 3;
         chan_merge(cnt, mean, m2, __ldcg(p), __ldcg(p + 1), __ldcg(p + 2));
       }
-#pragma unroll
-      for (int off = 16; off >= 1; off >>= 1) {
-        const float nb = __shfl_down_sync(0xffffffffu, cnt, off), mb = __shfl_down_sync(0xffffffffu, mean, off),
-                    m2b = __shfl_down_sync(0xffffffffu, m2, off);
-        chan_merge(cnt, mean, m2, nb, mb, m2b);
-      }
+      chan_warp_merge(cnt, mean, m2);
       if (lane == 0) { mine[n] = cnt; mine[w + n] = mean; mine[2 * w + n] = m2; }
     }
     __syncthreads();
@@ -245,12 +257,7 @@ __device__ __forceinline__ void stats_finalize_block(const float* __restrict__ p
         const float* a = all + (size_t)r * 3 * w;
         chan_merge(cnt, mean, m2, a[n], a[w + n], a[2 * w + n]);
       }
-      const float var = m2 / cnt;
-      f.stats[n] = mean; f.stats[w + n] = var; f.stats[2 * w + n] = rsqrtf(var + f.eps); f.stats[3 * w + n] = cnt;
-      if (f.running_mean) {
-        f.running_mean[n] = (1.f - f.momentum) * f.running_mean[n] + f.momentum * mean;
-        f.running_var[n] = (1.f - f.momentum) * f.running_var[n] + f.momentum * (m2 / fmaxf(cnt - 1.f, 1.f));
-      }
+      stats_store(f, w, n, cnt, mean, m2);
     }
     return;
   }
@@ -268,58 +275,17 @@ __device__ __forceinline__ void stats_finalize_block(const float* __restrict__ p
 #pragma unroll
         for (int j = 0; j < 8; ++j) chan_merge(cnt, mean, m2, pc[j], pm[j], pq[j]);   // a zero count is the identity
       }
-      const float var = m2 / cnt;
-      f.stats[n] = mean; f.stats[w + n] = var; f.stats[2 * w + n] = rsqrtf(var + f.eps); f.stats[3 * w + n] = cnt;
-      if (f.running_mean) {
-        f.running_mean[n] = (1.f - f.momentum) * f.running_mean[n] + f.momentum * mean;
-        f.running_var[n] = (1.f - f.momentum) * f.running_var[n] + f.momentum * (m2 / fmaxf(cnt - 1.f, 1.f));
-      }
+      stats_store(f, w, n, cnt, mean, m2);
     }
     return;
   }
-  for (int n = threadIdx.x >> 5; n < w; n += (int)(blockDim.x >> 5))
-    stats_finalize_column(part, ncta, w, n, f.eps, f.stats, f.running_mean, f.running_var, f.momentum);
+  for (int n = threadIdx.x >> 5; n < w; n += (int)(blockDim.x >> 5)) stats_finalize_column(part, ncta, w, n, f);
 }
 
-// Cross-rank variant: ONE CTA of 32 warps.  Local (count, mean, M2) per column -> peer exchange -> Chan merge of the
-// ranks' triples in rank order (identical on every rank).
+// Cross-rank finalize when it is not fused into the producing kernel: ONE CTA of 32 warps, staging in f.stage.
 __global__ void __launch_bounds__(1024)
-mlp_stats_finalize_peer_kernel(const float* __restrict__ part, int ncta, int w, float eps, float* __restrict__ stats,
-                               float* __restrict__ running_mean, float* __restrict__ running_var, float momentum,
-                               PeerComm comm, int slot) {
-  __shared__ float mine[3 * 128];
-  __shared__ float all[kPeerMaxWorld * 3 * 128];
-  const int lane = threadIdx.x & 31, wp = threadIdx.x >> 5;
-  for (int n = wp; n < w; n += 32) {
-    float cnt = 0.f, mean = 0.f, m2 = 0.f;
-    for (int c = lane; c < ncta; c += 32) {
-      const float* p = part + ((size_t)c * 128 + n) * 3;
-      chan_merge(cnt, mean, m2, p[0], p[1], p[2]);
-    }
-#pragma unroll
-    for (int off = 16; off >= 1; off >>= 1) {
-      const float nb = __shfl_down_sync(0xffffffffu, cnt, off), mb = __shfl_down_sync(0xffffffffu, mean, off),
-                  m2b = __shfl_down_sync(0xffffffffu, m2, off);
-      chan_merge(cnt, mean, m2, nb, mb, m2b);
-    }
-    if (lane == 0) { mine[n] = cnt; mine[w + n] = mean; mine[2 * w + n] = m2; }
-  }
-  __syncthreads();
-  peer_exchange(comm, slot, mine, 3 * w, all);
-  const int n = threadIdx.x;
-  if (n < w) {
-    float cnt = 0.f, mean = 0.f, m2 = 0.f;
-    for (int r = 0; r < comm.world; ++r) {
-      const float* a = all + (size_t)r * 3 * w;
-      chan_merge(cnt, mean, m2, a[n], a[w + n], a[2 * w + n]);
-    }
-    const float var = m2 / cnt;
-    stats[n] = mean; stats[w + n] = var; stats[2 * w + n] = rsqrtf(var + eps); stats[3 * w + n] = cnt;
-    if (running_mean) {
-      running_mean[n] = (1.f - momentum) * running_mean[n] + momentum * mean;
-      running_var[n] = (1.f - momentum) * running_var[n] + momentum * (m2 / fmaxf(cnt - 1.f, 1.f));
-    }
-  }
+mlp_stats_finalize_peer_kernel(const float* __restrict__ part, int ncta, int w, StatsFin fin) {
+  stats_finalize_block(part, ncta, w, fin);
 }
 
 // column n of the (S1, S2) sums by one warp (lanes stride over the blocks' partials, fixed shuffle tree)
@@ -385,7 +351,7 @@ mlp_bwd_reduce_kernel(const float* __restrict__ da, ActSrc cur, int has_bn, long
       fin.sums_global[i] = sacc;
       if (fin.sums) fin.sums[i] = mine[i];
     }
-  } else if (!fin.peer && fin.sums && last_block_arrives(fin.ticket)) {
+  } else if (!fin.peer && last_block_arrives(fin.ticket)) {
     const int nblk = (int)gridDim.x;
     if (nblk <= 64) {          // few partials: a thread per column, block order
       if (threadIdx.x < w) {
@@ -399,36 +365,6 @@ mlp_bwd_reduce_kernel(const float* __restrict__ da, ActSrc cur, int has_bn, long
     } else {
       for (int n = threadIdx.x >> 5; n < w; n += 8) sums_finalize_column(part, nblk, w, n, fin.sums);
     }
-  }
-}
-__global__ void __launch_bounds__(256)
-mlp_sum_finalize_kernel(const float* __restrict__ part, int nblk, int w, float* __restrict__ sums /*[2][w]*/) {
-  const int n = blockIdx.x * 8 + (threadIdx.x >> 5);
-  if (n >= w) return;
-  sums_finalize_column(part, nblk, w, n, sums);
-}
-
-// Cross-rank variant: local sums (parameter gradients of gamma/beta) and the rank-ordered global sums (for dy).
-__global__ void __launch_bounds__(1024)
-mlp_sum_finalize_peer_kernel(const float* __restrict__ part, int nblk, int w, float* __restrict__ sums_local,
-                             float* __restrict__ sums_global, PeerComm comm, int slot) {
-  __shared__ float mine[2 * 128];
-  __shared__ float all[kPeerMaxWorld * 2 * 128];
-  const int lane = threadIdx.x & 31, wp = threadIdx.x >> 5;
-  for (int n = wp; n < w; n += 32) {
-    float a = 0.f, b = 0.f;
-    for (int c = lane; c < nblk; c += 32) { a += part[((size_t)c * 128 + n) * 2]; b += part[((size_t)c * 128 + n) * 2 + 1]; }
-    a = warp_sum(a); b = warp_sum(b);
-    if (lane == 0) { mine[n] = a; mine[w + n] = b; }
-  }
-  __syncthreads();
-  peer_exchange(comm, slot, mine, 2 * w, all);
-  const int i = threadIdx.x;
-  if (i < 2 * w) {
-    float s = 0.f;
-    for (int r = 0; r < comm.world; ++r) s += all[(size_t)r * 2 * w + i];
-    sums_global[i] = s;
-    if (sums_local) sums_local[i] = mine[i];
   }
 }
 
@@ -602,23 +538,48 @@ mlp_dw_finalize_kernel(const float* __restrict__ part, int nsplit, int n, float*
 
 // ----------------------------------------------------------------------------------------- narrow layers (w <= 8)
 // The default LID-VAE encoder is 2-2-2-2-2-4-4 wide: a 128x128 tile per 128 rows wastes >99 % of its FMAs and is
-// latency bound.  For wi, wo <= 8 one THREAD owns a row: vector load, BN+LeakyReLU, wo x wi FMAs, vector store;
-// statistics / weight gradients are Chan- / sum-reduced warp -> block -> ordered per-block partials.
-template <int WI, int WO>
-__global__ void __launch_bounds__(256)
-mlp_narrow_fwd_kernel(ActSrc src, const float* __restrict__ W, const float* __restrict__ bias, int B, int wo,
-                      float* __restrict__ y_out, float* __restrict__ part, int do_stats, StatsFin fin) {
-  __shared__ ActSmem am;
-  __shared__ float Ws[WO][WI], bs[WO];
-  __shared__ float red[8][WO][3];
-  am.load(src);
-  const int wi = src.w;
-  if (threadIdx.x < WO * WI) {
-    const int o = threadIdx.x / WI, k = threadIdx.x % WI;
-    Ws[o][k] = (o < wo && k < wi) ? W[o * wi + k] : 0.f;
-  }
-  if (threadIdx.x < WO) bs[threadIdx.x] = (threadIdx.x < wo && bias) ? bias[threadIdx.x] : 0.f;
+// latency bound.  For wi, wo <= 8 one THREAD owns a row (row = blockIdx*256 + tid, stride gridDim*256): vector load,
+// BN+LeakyReLU, wo x wi FMAs, vector store; statistics / weight gradients are Chan- / sum-reduced warp -> block -> ordered
+// per-block partials.  The bodies below serve both the per-layer kernels and the whole-stack kernels, so the two paths
+// compute the same bits from the same partition of the rows.  Weights are staged zero-padded to 8 x 8.
+__device__ __forceinline__ void stage_w8(float (*Ws)[8], float* bs, const float* W, const float* bias, int wi, int wo, int e) {
+  const int o = e >> 3, k = e & 7;
+  Ws[o][k] = (o < wo && k < wi) ? W[o * wi + k] : 0.f;
+  if (bs && k == 0) bs[o] = (o < wo && bias) ? bias[o] : 0.f;
+}
+
+// per-CTA sums of v[R][C] over the 256 threads: warp_sum, then warps 0..7 in order.  Thread i < R*C returns the sum of
+// element i (row-major).
+template <int R, int C>
+__device__ __forceinline__ float cta_sum(const float (&v)[R][C], float* red /*[8][R*C]*/) {
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+#pragma unroll
+  for (int i = 0; i < R; ++i)
+#pragma unroll
+    for (int j = 0; j < C; ++j) {
+      const float s = warp_sum(v[i][j]);
+      if (lane == 0) red[(warp * R + i) * C + j] = s;
+    }
   __syncthreads();
+  float s = 0.f;
+  if (threadIdx.x < R * C)
+    for (int w8 = 0; w8 < 8; ++w8) s += red[w8 * R * C + threadIdx.x];
+  return s;
+}
+
+// ro_in: the layer input is not written by the launch that runs the body, so it may be read through the read-only
+// cache (the stack kernel reads rows it wrote itself for the previous layer).
+__device__ __forceinline__ float ld_in(bool ro_in, const float* p) { return ro_in ? __ldg(p) : *p; }
+
+// Forward rows: y = act(src) W^T + b.  head > 0: the layer's output is also split into mu = cols [0, head) and
+// softplus(cols [head, 2 head)) (torch.nn.functional.softplus, beta 1, threshold 20, ATen's expression).  do_stats: this
+// CTA's (count, mean, M2) per column -> part[blockIdx][128][3].
+template <int WI, int WO>
+__device__ __forceinline__ void narrow_fwd_rows(const ActSrc& src, bool ro_in, const ActSmem& am, int B, int wo,
+                                                const float (*Ws)[8],
+                                                const float* bs, float* y, bool head, int nh, float* mu, float* lv,
+                                                bool do_stats, float (*red)[8][3], float* part) {
+  const int wi = src.w;
   const bool has_bn = src.mean != nullptr;
   float cnt = 0.f, mean[WO], m2[WO];
 #pragma unroll
@@ -626,14 +587,20 @@ mlp_narrow_fwd_kernel(ActSrc src, const float* __restrict__ W, const float* __re
   for (int row = blockIdx.x * 256 + threadIdx.x; row < B; row += gridDim.x * 256) {
     float a[WI];
 #pragma unroll
-    for (int k = 0; k < WI; ++k) a[k] = (k < wi) ? am.act(has_bn, src.slope, __ldg(src.y + (size_t)row * wi + k), k) : 0.f;
+    for (int k = 0; k < WI; ++k) a[k] = (k < wi) ? am.act(has_bn, src.slope, ld_in(ro_in, src.y + (size_t)row * wi + k), k) : 0.f;
     cnt += 1.f;
 #pragma unroll
     for (int o = 0; o < WO; ++o) {
       float yv = bs[o];
 #pragma unroll
       for (int k = 0; k < WI; ++k) yv = fmaf(a[k], Ws[o][k], yv);
-      if (o < wo) y_out[(size_t)row * wo + o] = yv;
+      if (o < wo) {
+        y[(size_t)row * wo + o] = yv;
+        if (head) {
+          if (o < nh) mu[(size_t)row * nh + o] = yv;
+          else lv[(size_t)row * nh + o - nh] = yv > 20.f ? yv : log1pf(expf(yv));
+        }
+      }
       const float dlt = yv - mean[o];                    // Welford
       mean[o] += dlt / cnt;
       m2[o] = fmaf(dlt, yv - mean[o], m2[o]);
@@ -643,33 +610,43 @@ mlp_narrow_fwd_kernel(ActSrc src, const float* __restrict__ W, const float* __re
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
 #pragma unroll
   for (int o = 0; o < WO; ++o) {
-    float c = cnt, mu = mean[o], q = m2[o];
-#pragma unroll
-    for (int off = 16; off >= 1; off >>= 1) {
-      const float nb = __shfl_down_sync(0xffffffffu, c, off), mb = __shfl_down_sync(0xffffffffu, mu, off),
-                  qb = __shfl_down_sync(0xffffffffu, q, off);
-      chan_merge(c, mu, q, nb, mb, qb);
-    }
-    if (lane == 0) { red[warp][o][0] = c; red[warp][o][1] = mu; red[warp][o][2] = q; }
+    float c = cnt, mu_o = mean[o], q = m2[o];
+    chan_warp_merge(c, mu_o, q);
+    if (lane == 0) { red[warp][o][0] = c; red[warp][o][1] = mu_o; red[warp][o][2] = q; }
   }
   __syncthreads();
   if (threadIdx.x < wo) {
-    float c = 0.f, mu = 0.f, q = 0.f;
-    for (int w8 = 0; w8 < 8; ++w8) chan_merge(c, mu, q, red[w8][threadIdx.x][0], red[w8][threadIdx.x][1], red[w8][threadIdx.x][2]);
+    float c = 0.f, mu_o = 0.f, q = 0.f;
+    for (int w8 = 0; w8 < 8; ++w8) chan_merge(c, mu_o, q, red[w8][threadIdx.x][0], red[w8][threadIdx.x][1], red[w8][threadIdx.x][2]);
     float* o = part + ((size_t)blockIdx.x * 128 + threadIdx.x) * 3;
-    o[0] = c; o[1] = mu; o[2] = q;
+    o[0] = c; o[1] = mu_o; o[2] = q;
   }
-  if (fin.stats && last_block_arrives(fin.ticket)) stats_finalize_block(part, (int)gridDim.x, wo, fin);
 }
 
-// da_prev = dy W and per-block partial of dW = dy^T act(prev), one row per thread
+template <int WI, int WO>
+__global__ void __launch_bounds__(256)
+mlp_narrow_fwd_kernel(ActSrc src, const float* __restrict__ W, const float* __restrict__ bias, int B, int wo,
+                      float* __restrict__ y_out, float* __restrict__ part, int do_stats, StatsFin fin) {
+  __shared__ ActSmem am;
+  __shared__ float Ws[8][8], bs[8];
+  __shared__ float red[8][8][3];
+  am.load(src);
+  if (threadIdx.x < 64) stage_w8(Ws, bs, W, bias, src.w, wo, threadIdx.x);
+  __syncthreads();
+  narrow_fwd_rows<WI, WO>(src, true, am, B, wo, Ws, bs, y_out, false, 0, nullptr, nullptr, do_stats, red, part);
+  if (do_stats && fin.stats && last_block_arrives(fin.ticket)) stats_finalize_block(part, (int)gridDim.x, wo, fin);
+}
+
+// da_prev = dy W and per-block partial of dW = dy^T act(prev), one row per thread.  stack_bwd_layer runs the same row
+// loop and reduction; sharing them (cta_sum included) raised the register count here and in the stack kernels (the
+// 8-wide stack kernel spilled).
 template <int WI, int WO>
 __global__ void __launch_bounds__(256)
 mlp_narrow_bwd_kernel(DyCtx c, ActSrc prev, const float* __restrict__ W, int B, float* __restrict__ da_prev,
                       float* __restrict__ part /*[nblk][wo*wi]*/, DwFin fin) {
   __shared__ ActSmem am, pm;
   __shared__ float Ws[WO][WI], s1[WO], s2[WO];
-  __shared__ float red[8][WO * WI];
+  __shared__ float red[8 * WO * WI];
   const int wo = c.cur.w, wi = prev.w;
   am.load(c.cur);
   pm.load(prev);
@@ -720,17 +697,31 @@ mlp_narrow_bwd_kernel(DyCtx c, ActSrc prev, const float* __restrict__ W, int B, 
 #pragma unroll
     for (int k = 0; k < WI; ++k) {
       const float v = warp_sum(acc[o][k]);
-      if (lane == 0) red[warp][o * WI + k] = v;
+      if (lane == 0) red[warp * WO * WI + o * WI + k] = v;
     }
   __syncthreads();
   if (threadIdx.x < WO * WI) {
     const int o = threadIdx.x / WI, k = threadIdx.x % WI;
     float v = 0.f;
-    for (int w8 = 0; w8 < 8; ++w8) v += red[w8][threadIdx.x];
+    for (int w8 = 0; w8 < 8; ++w8) v += red[w8 * WO * WI + threadIdx.x];
     if (o < wo && k < wi) part[(size_t)blockIdx.x * wo * wi + o * wi + k] = v;
   }
   if (fin.dW && last_block_arrives(fin.ticket)) dw_finalize_block(part, (int)gridDim.x, wo * wi, fin.dW);
 }
+
+// Calls FN<WI, WO> ARGS for the width classes (ci, co) of a narrow layer; ARGS is an argument list in parentheses, or a
+// kernel launch's <<<...>>>(...).  kMaxC: the widest class compiled (4: only the (2|4) x (2|4) bodies, which keeps the
+// register count of the stack kernels -- and what they leave to concurrent kernels -- low).
+#define B200VAE_NARROW_DISPATCH(kMaxC, FN, ci, co, ...)                                                  \
+  do {                                                                                                    \
+    if (ci == 2 && co == 2) FN<2, 2> __VA_ARGS__; else if (ci == 2 && co == 4) FN<2, 4> __VA_ARGS__;     \
+    else if (ci == 4 && co == 2) FN<4, 2> __VA_ARGS__; else if (ci == 4 && co == 4) FN<4, 4> __VA_ARGS__; \
+    else if constexpr (kMaxC == 8) {                                                                      \
+      if (ci == 2) FN<2, 8> __VA_ARGS__; else if (ci == 4) FN<4, 8> __VA_ARGS__;                          \
+      else if (co == 2) FN<8, 2> __VA_ARGS__; else if (co == 4) FN<8, 4> __VA_ARGS__;                     \
+      else FN<8, 8> __VA_ARGS__;                                                                          \
+    }                                                                                                     \
+  } while (0)
 
 // ----------------------------------------------------------------------------------------- small batches (B <= kRowsMaxB)
 // At the batch sizes of BASELINE configs[2] / [3] (256) the 128x128x16 tile core runs a layer on 2 CTAs that walk up to 8
@@ -930,107 +921,38 @@ __device__ __forceinline__ bool stack_exit(unsigned* bar) {
   return last;
 }
 
-// layer input a[k] for row `row`: raw input or LeakyReLU(BN(previous y)) -- the arithmetic of mlp_narrow_*_kernel
-template <int WI>
-__device__ __forceinline__ void stack_act(float (&a)[WI], const ActSmem& am, bool has_bn, float slope, const float* y,
-                                          int wi, int row) {
-#pragma unroll
-  for (int k = 0; k < WI; ++k) a[k] = (k < wi) ? am.act(has_bn, slope, y[(size_t)row * wi + k], k) : 0.f;
-}
-
-template <int WI, int WO>
-__device__ __forceinline__ void stack_fwd_layer(const StackArgs& A, int l, const ActSmem& am, bool in_bn,
-                                                const float (*Ws)[8], const float* bs, bool do_stats,
-                                                float (*red)[8][3], float* part) {
-  const b200vae_mlp_layer_t& L = A.L[l];
-  const int wi = L.wi, wo = L.wo;
-  const float* src = l == 0 ? A.x : A.L[l - 1].y;
-  const bool last = l == A.nl - 1, head = last && A.head > 0;
-  float cnt = 0.f, mean[WO], m2[WO];
-#pragma unroll
-  for (int o = 0; o < WO; ++o) { mean[o] = 0.f; m2[o] = 0.f; }
-  for (int row = blockIdx.x * 256 + threadIdx.x; row < A.B; row += gridDim.x * 256) {
-    float a[WI];
-    stack_act<WI>(a, am, in_bn, A.slope, src, wi, row);
-    cnt += 1.f;
-#pragma unroll
-    for (int o = 0; o < WO; ++o) {
-      float yv = bs[o];
-#pragma unroll
-      for (int k = 0; k < WI; ++k) yv = fmaf(a[k], Ws[o][k], yv);
-      if (o < wo) {
-        L.y[(size_t)row * wo + o] = yv;
-        if (head) {      // torch.nn.functional.softplus (beta 1, threshold 20), the same expression as ATen's kernel
-          if (o < A.head) A.out0[(size_t)row * A.head + o] = yv;
-          else A.out1[(size_t)row * A.head + o - A.head] = yv > 20.f ? yv : log1pf(expf(yv));
-        }
-      }
-      const float dlt = yv - mean[o];                    // Welford
-      mean[o] += dlt / cnt;
-      m2[o] = fmaf(dlt, yv - mean[o], m2[o]);
-    }
-  }
-  if (!do_stats) return;
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-#pragma unroll
-  for (int o = 0; o < WO; ++o) {
-    float c = cnt, mu = mean[o], q = m2[o];
-#pragma unroll
-    for (int off = 16; off >= 1; off >>= 1) {
-      const float nb = __shfl_down_sync(0xffffffffu, c, off), mb = __shfl_down_sync(0xffffffffu, mu, off),
-                  qb = __shfl_down_sync(0xffffffffu, q, off);
-      chan_merge(c, mu, q, nb, mb, qb);
-    }
-    if (lane == 0) { red[warp][o][0] = c; red[warp][o][1] = mu; red[warp][o][2] = q; }
-  }
-  __syncthreads();
-  if (threadIdx.x < wo) {
-    float c = 0.f, mu = 0.f, q = 0.f;
-    for (int w8 = 0; w8 < 8; ++w8) chan_merge(c, mu, q, red[w8][threadIdx.x][0], red[w8][threadIdx.x][1], red[w8][threadIdx.x][2]);
-    float* o = part + ((size_t)blockIdx.x * 128 + threadIdx.x) * 3;
-    o[0] = c; o[1] = mu; o[2] = q;
-  }
-}
-
-// kMaxC: the widest layer class the kernel instantiation serves (4: only (2|4) x (2|4) bodies are compiled, which keeps
-// the register count -- and what the kernel leaves to concurrent kernels -- low)
-#define B200VAE_STACK_DISPATCH(kMaxC, FN, ci, co, ...)                                                     \
-  do {                                                                                                      \
-    if (ci == 2 && co == 2) FN<2, 2>(__VA_ARGS__); else if (ci == 2 && co == 4) FN<2, 4>(__VA_ARGS__);     \
-    else if (ci == 4 && co == 2) FN<4, 2>(__VA_ARGS__); else if (ci == 4 && co == 4) FN<4, 4>(__VA_ARGS__); \
-    else if constexpr (kMaxC == 8) {                                                                        \
-      if (ci == 2) FN<2, 8>(__VA_ARGS__); else if (ci == 4) FN<4, 8>(__VA_ARGS__);                          \
-      else if (co == 2) FN<8, 2>(__VA_ARGS__); else if (co == 4) FN<8, 4>(__VA_ARGS__);                     \
-      else FN<8, 8>(__VA_ARGS__);                                                                           \
-    }                                                                                                       \
-  } while (0)
-
 // Forward of a whole narrow stack.  Training: per BatchNorm layer one grid barrier, then every CTA combines the layer's
 // (count, mean, M2) partials with stats_finalize_block (the per-layer path's last-block code) into shared memory; CTA 0
 // also stores the statistics and updates running_mean / running_var / num_batches_tracked.  Eval: the statistics are read
 // from L[l].stats and no CTA waits for another.
+// the input of layer l: the raw input, or LeakyReLU(BN(y of layer l - 1)) with that layer's stored statistics
+__device__ __forceinline__ ActSrc stack_in(const StackArgs& A, int l) {
+  if (l == 0) return make_src(A.x, nullptr, nullptr, nullptr, A.L[0].wi, A.slope);
+  const b200vae_mlp_layer_t& P = A.L[l - 1];
+  return make_src(P.y, P.stats, P.gamma, P.beta, P.wo, A.slope);
+}
+
 template <int kMaxC>
 __global__ void __launch_bounds__(256, kMaxC == 8 ? 2 : 4) mlp_stack_fwd_kernel(const StackArgs A) {
   __shared__ ActSmem am;
   __shared__ float Ws[kStackMaxLayers][8][8], bs[kStackMaxLayers][8];
   __shared__ float red[8][8][3];
   __shared__ float st[4 * 8];
-  for (int e = threadIdx.x; e < A.nl * 64; e += 256) {      // every layer's weights, zero-padded to 8 x 8
-    const int l = e >> 6, o = (e >> 3) & 7, k = e & 7;
-    const b200vae_mlp_layer_t& L = A.L[l];
-    Ws[l][o][k] = (o < L.wo && k < L.wi) ? L.W[o * L.wi + k] : 0.f;
-    if (k == 0) bs[l][o] = o < L.wo ? L.bias[o] : 0.f;
+  for (int e = threadIdx.x; e < A.nl * 64; e += 256) {      // every layer's weights
+    const int l = e >> 6;
+    stage_w8(Ws[l], bs[l], A.L[l].W, A.L[l].bias, A.L[l].wi, A.L[l].wo, e & 63);
   }
   unsigned epoch = 0;
   for (int l = 0; l < A.nl; ++l) {
     const b200vae_mlp_layer_t& L = A.L[l];
-    const bool in_bn = l > 0;
+    const bool last = l == A.nl - 1;
     __syncthreads();                                          // weights loaded / previous layer's ActSmem in place
-    const bool do_stats = A.training && l < A.nl - 1;
+    const bool do_stats = A.training && !last;
     float* part = A.scratch + (size_t)(l & 1) * kStackMaxGrid * 128 * 3;
-    B200VAE_STACK_DISPATCH(kMaxC, stack_fwd_layer, narrow_class(L.wi), narrow_class(L.wo), A, l, am, in_bn, Ws[l], bs[l],
-                           do_stats, red, part);
-    if (l == A.nl - 1) break;
+    const ActSrc src = stack_in(A, l);
+    B200VAE_NARROW_DISPATCH(kMaxC, narrow_fwd_rows, narrow_class(L.wi), narrow_class(L.wo),
+                            (src, false, am, A.B, L.wo, Ws[l], bs[l], L.y, last && A.head > 0, A.head, A.out0, A.out1, do_stats, red, part));
+    if (last) break;
     const int wo = L.wo;
     if (do_stats) {
       grid_barrier(A.bar, epoch);
@@ -1048,12 +970,7 @@ __global__ void __launch_bounds__(256, kMaxC == 8 ? 2 : 4) mlp_stack_fwd_kernel(
       st[threadIdx.x] = L.stats[threadIdx.x];
     }
     __syncthreads();
-    if (threadIdx.x < 128) {                                  // the next layer's input transform
-      const int k = threadIdx.x;
-      const bool in = k < wo;
-      am.mean[k] = in ? st[k] : 0.f; am.invstd[k] = in ? st[2 * wo + k] : 0.f;
-      am.gamma[k] = in ? L.gamma[k] : 0.f; am.beta[k] = in ? L.beta[k] : 0.f;
-    }
+    am.load(make_src(L.y, st, L.gamma, L.beta, wo, A.slope));   // the next layer's input transform
   }
   if (A.training) stack_exit(A.bar);
 }
@@ -1096,35 +1013,22 @@ __device__ __forceinline__ void stack_dyhat(const StackArgs& A, int l, const Act
 }
 
 template <int WO>
-__device__ __forceinline__ void stack_bwd_sums(const StackArgs& A, int l, const ActSmem& am, float (*red)[8][2],
-                                               float* part) {
-  const int wo = A.L[l].wo;
-  float s1[WO], s2[WO];
+__device__ __forceinline__ void stack_bwd_sums(const StackArgs& A, int l, const ActSmem& am, float* red, float* part) {
+  float s[WO][2];                                             // S1, S2 of column o
 #pragma unroll
-  for (int o = 0; o < WO; ++o) { s1[o] = 0.f; s2[o] = 0.f; }
+  for (int o = 0; o < WO; ++o) { s[o][0] = 0.f; s[o][1] = 0.f; }
   for (int row = blockIdx.x * 256 + threadIdx.x; row < A.B; row += gridDim.x * 256) {
     float g[WO], xh[WO];
     stack_dyhat<WO>(A, l, am, row, g, xh);
 #pragma unroll
-    for (int o = 0; o < WO; ++o) { s1[o] += g[o]; s2[o] = fmaf(g[o], xh[o], s2[o]); }
+    for (int o = 0; o < WO; ++o) { s[o][0] += g[o]; s[o][1] = fmaf(g[o], xh[o], s[o][1]); }
   }
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-#pragma unroll
-  for (int o = 0; o < WO; ++o) {
-    const float a = warp_sum(s1[o]), b = warp_sum(s2[o]);
-    if (lane == 0) { red[warp][o][0] = a; red[warp][o][1] = b; }
-  }
-  __syncthreads();
-  if (threadIdx.x < wo) {
-    float a = 0.f, b = 0.f;
-    for (int w8 = 0; w8 < 8; ++w8) { a += red[w8][threadIdx.x][0]; b += red[w8][threadIdx.x][1]; }
-    part[((size_t)blockIdx.x * 128 + threadIdx.x) * 2 + 0] = a;
-    part[((size_t)blockIdx.x * 128 + threadIdx.x) * 2 + 1] = b;
-  }
+  const float v = cta_sum(s, red);
+  if (threadIdx.x < 2 * A.L[l].wo) part[(size_t)blockIdx.x * 256 + threadIdx.x] = v;
 }
 
 // Backward, phase 2 of layer l: dy from dyhat and the global sums, da_prev = dy W into the rows buffer (or dx), and the
-// per-CTA dW partial (warp -> block, fixed order)
+// per-CTA dW partial.  The row loop is mlp_narrow_bwd_kernel's, with dy from stack_dyhat.
 template <int WI, int WO>
 __device__ __forceinline__ void stack_bwd_layer(const StackArgs& A, int l, const ActSmem& am, const ActSmem& pm,
                                                 const float (*Ws)[8], const float* s1, const float* s2, float invN,
@@ -1145,9 +1049,11 @@ __device__ __forceinline__ void stack_bwd_layer(const StackArgs& A, int l, const
 #pragma unroll
     for (int o = 0; o < WO; ++o)
       dy[o] = (o < wo && has_bn) ? am.gamma[o] * am.invstd[o] * (g[o] - s1[o] * invN - xh[o] * (s2[o] * invN)) : g[o];
-    stack_act<WI>(a, pm, l > 0, A.slope, src, wi, row);
 #pragma unroll
-    for (int k = 0; k < WI; ++k) dap[k] = 0.f;
+    for (int k = 0; k < WI; ++k) {
+      a[k] = (k < wi) ? pm.act(l > 0, A.slope, src[(size_t)row * wi + k], k) : 0.f;
+      dap[k] = 0.f;
+    }
 #pragma unroll
     for (int o = 0; o < WO; ++o)
 #pragma unroll
@@ -1160,30 +1066,11 @@ __device__ __forceinline__ void stack_bwd_layer(const StackArgs& A, int l, const
       for (int k = 0; k < WI; ++k) if (k < wi) A.dx[(size_t)row * wi + k] = dap[k];
     }
   }
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-#pragma unroll
-  for (int o = 0; o < WO; ++o)
-#pragma unroll
-    for (int k = 0; k < WI; ++k) {
-      const float v = warp_sum(acc[o][k]);
-      if (lane == 0) red[warp * 64 + o * WI + k] = v;
-    }
-  __syncthreads();
+  const float v = cta_sum(acc, red);
   if (threadIdx.x < WO * WI) {
     const int o = threadIdx.x / WI, k = threadIdx.x % WI;
-    float v = 0.f;
-    for (int w8 = 0; w8 < 8; ++w8) v += red[w8 * 64 + threadIdx.x];
     float* part = A.scratch + kStackPartFloats + (size_t)l * kStackMaxGrid * 64;
     if (o < wo && k < wi) part[(size_t)blockIdx.x * wo * wi + o * wi + k] = v;
-  }
-}
-
-__device__ __forceinline__ void stack_load_act(ActSmem& s, const b200vae_mlp_layer_t& L) {
-  if (threadIdx.x < 128) {
-    const int k = threadIdx.x, w = L.wo;
-    const bool in = k < w;
-    s.mean[k] = in ? L.stats[k] : 0.f; s.invstd[k] = in ? L.stats[2 * w + k] : 0.f;
-    s.gamma[k] = in ? L.gamma[k] : 0.f; s.beta[k] = in ? L.beta[k] : 0.f;
   }
 }
 
@@ -1204,19 +1091,15 @@ __global__ void __launch_bounds__(256, kMaxC == 8 ? 2 : 4) mlp_stack_bwd_kernel(
     const int wo = L.wo, wi = L.wi;
     const bool has_bn = l < A.nl - 1;
     __syncthreads();                                          // the previous layer is done with the shared arrays
-    if (has_bn) stack_load_act(am, L);
-    if (l > 0) stack_load_act(pm, A.L[l - 1]);
-    if (threadIdx.x < 64) {
-      const int o = threadIdx.x >> 3, k = threadIdx.x & 7;
-      Ws[o][k] = (o < wo && k < wi) ? L.W[o * wi + k] : 0.f;
-    }
+    if (has_bn) am.load(stack_in(A, l + 1));
+    pm.load(stack_in(A, l));
+    if (threadIdx.x < 64) stage_w8(Ws, nullptr, L.W, nullptr, wi, wo, threadIdx.x);
     __syncthreads();
     float* part = A.scratch + (size_t)(l & 1) * kStackMaxGrid * 128 * 2;
     const int co = narrow_class(wo);
-    float (*red2)[8][2] = reinterpret_cast<float (*)[8][2]>(red);
-    if (co == 2) stack_bwd_sums<2>(A, l, am, red2, part);
-    else if (co == 4) stack_bwd_sums<4>(A, l, am, red2, part);
-    else if constexpr (kMaxC == 8) stack_bwd_sums<8>(A, l, am, red2, part);
+    if (co == 2) stack_bwd_sums<2>(A, l, am, red, part);
+    else if (co == 4) stack_bwd_sums<4>(A, l, am, red, part);
+    else if constexpr (kMaxC == 8) stack_bwd_sums<8>(A, l, am, red, part);
     if (has_bn) {
       grid_barrier(A.bar, epoch);
       for (int n = threadIdx.x >> 5; n < wo; n += 8) sums_finalize_column(part, (int)gridDim.x, wo, n, sums);
@@ -1232,7 +1115,7 @@ __global__ void __launch_bounds__(256, kMaxC == 8 ? 2 : 4) mlp_stack_bwd_kernel(
       if (threadIdx.x < wo) dbpart[(size_t)blockIdx.x * wo + threadIdx.x] = part[((size_t)blockIdx.x * 128 + threadIdx.x) * 2];
     }
     __syncthreads();
-    B200VAE_STACK_DISPATCH(kMaxC, stack_bwd_layer, narrow_class(wi), co, A, l, am, pm, Ws, s1, s2, invN, red);
+    B200VAE_NARROW_DISPATCH(kMaxC, stack_bwd_layer, narrow_class(wi), co, (A, l, am, pm, Ws, s1, s2, invN, red));
   }
   if (stack_exit(A.bar)) {
     for (int l = 0; l < A.nl; ++l) {
@@ -1244,32 +1127,7 @@ __global__ void __launch_bounds__(256, kMaxC == 8 ? 2 : 4) mlp_stack_bwd_kernel(
   }
 }
 
-template <int WI, int WO>
-static void narrow_fwd_launch(const ActSrc& src, const float* W, const float* bias, int B, int wo, float* y, float* part,
-                              int do_stats, const StatsFin& fin, int grid, cudaStream_t st) {
-  mlp_narrow_fwd_kernel<WI, WO><<<grid, 256, 0, st>>>(src, W, bias, B, wo, y, part, do_stats, fin);
-}
-template <int WI, int WO>
-static void narrow_bwd_launch(const DyCtx& c, const ActSrc& prev, const float* W, int B, float* da_prev, float* part,
-                              const DwFin& fin, int grid, cudaStream_t st) {
-  mlp_narrow_bwd_kernel<WI, WO><<<grid, 256, 0, st>>>(c, prev, W, B, da_prev, part, fin);
-}
-#define B200VAE_NARROW_DISPATCH(FN, ci, co, ...)                                   \
-  do {                                                                              \
-    if (ci == 2 && co == 2) FN<2, 2>(__VA_ARGS__); else if (ci == 2 && co == 4) FN<2, 4>(__VA_ARGS__);   \
-    else if (ci == 2 && co == 8) FN<2, 8>(__VA_ARGS__); else if (ci == 4 && co == 2) FN<4, 2>(__VA_ARGS__); \
-    else if (ci == 4 && co == 4) FN<4, 4>(__VA_ARGS__); else if (ci == 4 && co == 8) FN<4, 8>(__VA_ARGS__); \
-    else if (ci == 8 && co == 2) FN<8, 2>(__VA_ARGS__); else if (ci == 8 && co == 4) FN<8, 4>(__VA_ARGS__); \
-    else FN<8, 8>(__VA_ARGS__);                                                     \
-  } while (0)
-
 static bool pow2_le128(int w) { return w >= 1 && w <= 128 && (w & (w - 1)) == 0; }
-static ActSrc make_src(const float* y, const float* stats, const float* gamma, const float* beta, int w, float slope) {
-  ActSrc s;
-  s.y = y; s.w = w; s.slope = slope;
-  s.mean = stats; s.invstd = stats ? stats + 2 * w : nullptr; s.gamma = gamma; s.beta = beta;
-  return s;
-}
 
 }  // namespace b200vae
 
@@ -1313,7 +1171,8 @@ static int mlp_layer_fwd_impl(const float* in_y, const float* in_stats, const fl
   fin.peer = comm ? 1 : 0; fin.slot = slot; fin.stage = mlp_stage(scratch, B);
   if (comm) fin.comm = make_peer(comm); else memset(&fin.comm, 0, sizeof(fin.comm));
   if (ci && co) {
-    B200VAE_NARROW_DISPATCH(narrow_fwd_launch, ci, co, src, W, bias, B, wo, y_out, (float*)scratch, stats_out ? 1 : 0, fin, ncta, st);
+    B200VAE_NARROW_DISPATCH(8, mlp_narrow_fwd_kernel, ci, co,
+                            <<<ncta, 256, 0, st>>>(src, W, bias, B, wo, y_out, (float*)scratch, stats_out ? 1 : 0, fin));
   } else if (rows) {
     static bool attr_done = false;
     if (!attr_done) { cudaFuncSetAttribute(mlp_rows_fwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)rows_smem_bytes(false)); attr_done = true; }
@@ -1323,11 +1182,9 @@ static int mlp_layer_fwd_impl(const float* in_y, const float* in_stats, const fl
   }
   int rc = check_launch();
   if (rc || !stats_out || fused) return rc;
-  if (comm)
-    mlp_stats_finalize_peer_kernel<<<1, 1024, 0, st>>>((const float*)scratch, ncta, wo, eps, stats_out, running_mean,
-                                                      running_var, momentum, make_peer(comm), slot);
-  else
-    mlp_stats_finalize_kernel<<<(wo + 7) / 8, 256, 0, st>>>((const float*)scratch, ncta, wo, eps, stats_out, running_mean, running_var, momentum);
+  fin.stats = stats_out;
+  if (comm) mlp_stats_finalize_peer_kernel<<<1, 1024, 0, st>>>((const float*)scratch, ncta, wo, fin);
+  else mlp_stats_finalize_kernel<<<(wo + 7) / 8, 256, 0, st>>>((const float*)scratch, ncta, wo, fin);
   return check_launch();
 }
 extern "C" int b200vae_mlp_layer_fwd(const float* in_y, const float* in_stats, const float* in_gamma, const float* in_beta,
@@ -1366,12 +1223,6 @@ static int mlp_layer_bwd_reduce_impl(const float* da, const float* y, const floa
   fin.peer = comm ? 1 : 0; fin.slot = slot; fin.sums_global = sums_global; fin.stage = mlp_stage(scratch, B);
   if (comm) fin.comm = make_peer(comm); else memset(&fin.comm, 0, sizeof(fin.comm));
   mlp_bwd_reduce_kernel<<<nblk, 256, 0, st>>>(da, cur, stats ? 1 : 0, n, per, dyhat, (float*)scratch, fin);
-  int rc = check_launch();
-  if (rc || fin.sums || fin.peer) return rc;
-  if (comm)
-    mlp_sum_finalize_peer_kernel<<<1, 1024, 0, st>>>((const float*)scratch, nblk, w, sums, sums_global, make_peer(comm), slot);
-  else
-    mlp_sum_finalize_kernel<<<(w + 7) / 8, 256, 0, st>>>((const float*)scratch, nblk, w, sums);
   return check_launch();
 }
 extern "C" int b200vae_mlp_layer_bwd_reduce(const float* da, const float* y, const float* stats, const float* gamma,
@@ -1407,7 +1258,8 @@ extern "C" int b200vae_mlp_layer_bwd(const float* dyhat, const float* y, const f
     const ActSrc prev = make_src(prev_y, prev_stats, prev_gamma, prev_beta, wi, slope);
     DwFin fin;
     fin.dW = dW; fin.ticket = mlp_ticket(scratch, B);        // <= 64 outputs from <= 592 partials: always fused
-    B200VAE_NARROW_DISPATCH(narrow_bwd_launch, ci, co, c, prev, W, B, da_prev, dW ? (float*)scratch : nullptr, fin, grid, st);
+    B200VAE_NARROW_DISPATCH(8, mlp_narrow_bwd_kernel, ci, co,
+                            <<<grid, 256, 0, st>>>(c, prev, W, B, da_prev, dW ? (float*)scratch : nullptr, fin));
     return check_launch();
   }
   if (B <= kRowsMaxB) {            // small batch: ONE row-tile kernel for da_prev and the dW partials (W in shared memory)
@@ -1449,13 +1301,13 @@ extern "C" int b200vae_mlp_layer_bwd(const float* dyhat, const float* y, const f
 }
 
 // ----------------------------------------------------------------------------------------- narrow stacks
-static bool stack_shape_ok(const b200vae_mlp_layer_t* L, int nl, int B, bool need_stats) {
+static bool stack_shape_ok(const b200vae_mlp_layer_t* L, int nl, int B) {
   if (!L || nl < 1 || nl > kStackMaxLayers || B <= 0) return false;
   for (int l = 0; l < nl; ++l) {
     if (L[l].wi < 1 || L[l].wi > 8 || L[l].wo < 1 || L[l].wo > 8) return false;
     if (l > 0 && L[l].wi != L[l - 1].wo) return false;
     if (!L[l].W || !L[l].bias || !L[l].y) return false;
-    if (l < nl - 1 && (!L[l].gamma || !L[l].beta || (need_stats && !L[l].stats))) return false;
+    if (l < nl - 1 && (!L[l].gamma || !L[l].beta || !L[l].stats)) return false;
   }
   return true;
 }
@@ -1504,7 +1356,7 @@ static StackArgs stack_args(const b200vae_mlp_layer_t* layers, int nl, const flo
 extern "C" int b200vae_mlp_stack_fwd(const b200vae_mlp_layer_t* layers, int nl, const float* x, int B, float slope,
                                      int training, int head, float* mu, float* lv, void* scratch, void* stream) {
   if (!x || !scratch) return B200VAE_EALIGN;
-  if (!stack_shape_ok(layers, nl, B, !training)) return B200VAE_ESHAPE;
+  if (!stack_shape_ok(layers, nl, B)) return B200VAE_ESHAPE;
   if (head < 0 || (head > 0 && (2 * head != layers[nl - 1].wo || !mu || !lv))) return B200VAE_ESHAPE;
   StackArgs A = stack_args(layers, nl, x, B, slope, training, head, scratch);
   A.out0 = mu; A.out1 = lv;
@@ -1516,7 +1368,7 @@ extern "C" int b200vae_mlp_stack_bwd(const b200vae_mlp_layer_t* layers, const b2
                                      const float* x, int B, float slope, int training, int head, const float* g0,
                                      const float* g1, float* dx, void* scratch, void* stream) {
   if (!x || !scratch || !grads) return B200VAE_EALIGN;
-  if (!stack_shape_ok(layers, nl, B, true)) return B200VAE_ESHAPE;
+  if (!stack_shape_ok(layers, nl, B)) return B200VAE_ESHAPE;
   if (head < 0 || (head > 0 && 2 * head != layers[nl - 1].wo) || (head == 0 && !g0)) return B200VAE_ESHAPE;
   for (int l = 0; l < nl; ++l)
     if (!grads[l].dW || !grads[l].db || (l < nl - 1 && (!grads[l].dgamma || !grads[l].dbeta))) return B200VAE_EALIGN;

@@ -261,13 +261,9 @@ class FlexibleVAE(VAE):
 
     def _stack_plan(self, name):
         """Cached ops.MlpPlan of self.encoder / self.decoder, or None when the stack is not a plain MLP chain."""
-        seq = getattr(self, name)
-        cache = self.__dict__.setdefault("_mlp_plans", {})
-        plan = cache.get(name, False)
-        if plan is False or (plan is not None and not ops.mlp_plan_is_current(plan, seq)):
-            plan = ops.mlp_plan_from_modules(seq) if (self.data_type == "1d" and not self.residual_connection) else None
-            cache[name] = plan
-        return plan
+        if self.data_type != "1d" or self.residual_connection:
+            return None
+        return ops.cached_mlp_plan(self, name)
 
     def _run_stack(self, name, input):
         plan = self._stack_plan(name) if (self.fused_mlp and input.is_cuda and input.dim() == 2) else None
@@ -390,17 +386,10 @@ class LIDVAE(VAE):
     fused_encoder = True    # 1-D MLP encoders run through the fused Linear+BN+LeakyReLU layer kernels when they match
 
     def _encoder_plan(self):
-        plan = self.__dict__.get("_mlp_plan", False)
-        if plan is False or (plan is not None and plan.linears[0] is not self.encoder[0][0]):
-            plan = ops.MlpPlan.from_sequential(self.encoder)
-            self.__dict__["_mlp_plan"] = plan
-        return plan
+        return ops.cached_mlp_plan(self, "encoder")
 
     def encode(self, input):
         plan = self._encoder_plan() if (self.fused_encoder and input.is_cuda and input.dim() == 2) else None
-        # the plan caches module references: rebuild it if BatchNorms were swapped (e.g. SyncBatchNorm conversion)
-        if plan is not None and any(b is not blk[1] for b, blk in zip(plan.bns, self.encoder)):
-            self.__dict__["_mlp_plan"] = plan = ops.MlpPlan.from_sequential(self.encoder)
         if plan is not None:
             return ops.fused_mlp(plan, input, self.training, softplus_head=True)
         ret = self.encoder(input)

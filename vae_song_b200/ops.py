@@ -576,41 +576,28 @@ class VaeLossFn(torch.autograd.Function):
 
 
 # ------------------------------------------------------------------------------------------ fused MLP encoder
+def _flat_params(Ws, bs, gs, bes):
+    """The parameter order of FusedMlpFn / FusedMlpStackFn: (W, b) of every Linear, then (gamma, beta) of every BN."""
+    out = []
+    for W, b in zip(Ws, bs):
+        out += [W, b]
+    for g, be in zip(gs, bes):
+        out += [g, be]
+    return out
+
+
 class MlpPlan:
     """Structure of a [Linear -> BatchNorm1d -> LeakyReLU] x n (+ trailing Linear) stack, extracted from stock
-    nn.Modules (which keep owning the parameters / buffers, so state_dict keys do not change)."""
+    nn.Modules (which keep owning the parameters / buffers, so state_dict keys do not change).  `source` holds the
+    identities of the leaf modules it was read from; `identity_tail`: the trailing Linear is an appended identity."""
 
-    def __init__(self, linears, bns, slope):
+    def __init__(self, linears, bns, slope, source=(), identity_tail=False):
         self.linears, self.bns, self.slope = linears, bns, slope       # len(bns) == len(linears) - 1
+        self.source, self.identity_tail = source, identity_tail
 
-    @staticmethod
-    def from_sequential(seq):
-        """Recognise LIDVAE.make_encoder_1d (model.py:711-734): blocks Seq(Linear, BN1d, LeakyReLU) and a last block
-        Seq(Linear, BN1d, LeakyReLU, Linear).  Returns None when the module does not match (stock path is used)."""
-        nn = torch.nn
-        try:
-            blocks = list(seq)
-            lin, bns, slopes = [], [], []
-            for bi, blk in enumerate(blocks):
-                mods = list(blk)
-                last = bi == len(blocks) - 1
-                if len(mods) != (4 if last else 3):
-                    return None
-                if not (isinstance(mods[0], nn.Linear) and isinstance(mods[1], nn.BatchNorm1d) and isinstance(mods[2], nn.LeakyReLU)):
-                    return None
-                lin.append(mods[0]); bns.append(mods[1]); slopes.append(mods[2].negative_slope)
-                if last:
-                    if not isinstance(mods[3], nn.Linear):
-                        return None
-                    lin.append(mods[3])
-        except TypeError:
-            return None
-        ok_w = all(1 <= l.out_features <= 128 and (l.out_features & (l.out_features - 1)) == 0 for l in lin)
-        ok_w = ok_w and 1 <= lin[0].in_features <= 128
-        ok_bn = all(b.affine and b.track_running_stats and b.momentum is not None for b in bns)
-        if not (ok_w and ok_bn and len(set(slopes)) == 1 and all(l.bias is not None for l in lin)):
-            return None
-        return MlpPlan(lin, bns, float(slopes[0]))
+    def params(self):
+        return _flat_params([l.weight for l in self.linears], [l.bias for l in self.linears],
+                            [b.weight for b in self.bns], [b.bias for b in self.bns])
 
 
 def _leaf_modules(mod):
@@ -626,7 +613,7 @@ def _leaf_modules(mod):
 def mlp_plan_from_modules(seq):
     """MlpPlan for ANY nesting of Sequentials whose leaves read (Linear, BatchNorm1d, LeakyReLU)+ [Linear] -- the 1-D MLP
     stacks of FlexibleVAE (model.py:186-208, 360-374: the encoder ENDS in BN + LeakyReLU, the decoder in a bare Linear) as
-    well as LIDVAE's encoder.  A stack without the trailing Linear gets a frozen identity layer appended (not registered
+    well as LIDVAE's encoder (model.py:711-734).  A stack without the trailing Linear gets a frozen identity layer appended (not registered
     anywhere: act(BN(y)) . I + 0 is exact), so that the last BatchNorm + activation is applied by the same layer kernels.
     Returns None when the modules do not match; `plan.source` holds the leaf identities for staleness checks."""
     nn = torch.nn
@@ -655,15 +642,23 @@ def mlp_plan_from_modules(seq):
     ok_bn = all(b.affine and b.track_running_stats and b.momentum is not None for b in bns)
     if not (ok_w and ok_bn and len(set(slopes)) == 1 and all(l.bias is not None for l in lin)):
         return None
-    plan = MlpPlan(lin, bns, float(slopes[0]))
-    plan.source = tuple(id(m) for m in leaves)
-    plan.identity_tail = identity
-    return plan
+    return MlpPlan(lin, bns, float(slopes[0]), tuple(id(m) for m in leaves), identity)
 
 
 def mlp_plan_is_current(plan, seq):
-    return plan is not None and getattr(plan, "source", None) == tuple(id(m) for m in _leaf_modules(seq)) \
+    return plan is not None and plan.source == tuple(id(m) for m in _leaf_modules(seq)) \
         and plan.linears[0].weight.device == plan.linears[-1].weight.device
+
+
+def cached_mlp_plan(module, name):
+    """MlpPlan of module.<name>, cached on the module and rebuilt when its leaf modules are no longer the ones the plan
+    was read from (a SyncBatchNorm conversion, a replaced layer).  None when the stack does not match."""
+    seq = getattr(module, name)
+    cache = module.__dict__.setdefault("_mlp_plans", {})
+    plan = cache.get(name, False)
+    if plan is False or (plan is not None and not mlp_plan_is_current(plan, seq)):
+        plan = cache[name] = mlp_plan_from_modules(seq)
+    return plan
 
 
 def _bn_group(bn):
@@ -672,6 +667,21 @@ def _bn_group(bn):
     if type(bn).__name__ == "SyncBatchNorm1d" and dist.is_available() and dist.is_initialized() and dist.get_world_size(bn.group) > 1:
         return bn.group if bn.group is not None else dist.group.WORLD
     return None
+
+
+def _unpack_params(nl, params):
+    """(Ws, bs, gammas, betas) from the flat order of _flat_params"""
+    Ws = [_req(params[2 * i], "W") for i in range(nl)]
+    bs = [_req(params[2 * i + 1], "b") for i in range(nl)]
+    gs = [_req(params[2 * nl + 2 * i], "gamma") for i in range(nl - 1)]
+    bes = [_req(params[2 * nl + 2 * i + 1], "beta") for i in range(nl - 1)]
+    return Ws, bs, gs, bes
+
+
+def _eval_stats(st, bn, B):
+    """stats [4][w] of an eval-mode BatchNorm: its running statistics are constants"""
+    st[0].copy_(bn.running_mean); st[1].copy_(bn.running_var)
+    st[2].copy_(torch.rsqrt(bn.running_var + bn.eps)); st[3].fill_(float(B))
 
 
 _mlp_scratch_cache = {}
@@ -697,10 +707,7 @@ class FusedMlpFn(torch.autograd.Function):
         x = _req(x, "x")
         B = x.shape[0]
         nl = len(plan.linears)
-        Ws = [_req(params[2 * i], "W") for i in range(nl)]
-        bs = [_req(params[2 * i + 1], "b") for i in range(nl)]
-        gs = [_req(params[2 * nl + 2 * i], "gamma") for i in range(nl - 1)]
-        bes = [_req(params[2 * nl + 2 * i + 1], "beta") for i in range(nl - 1)]
+        Ws, bs, gs, bes = _unpack_params(nl, params)
         scratch = _mlp_scratch(lib.b200vae_mlp_scratch_bytes(B), x.device)
         ys, stats, counts = [], [], []
         ticks = []                # num_batches_tracked counters, advanced by one multi-tensor launch at the end
@@ -735,9 +742,8 @@ class FusedMlpFn(torch.autograd.Function):
             n_glob = float(B)
             if has_bn:
                 bn = plan.bns[i]
-                if not training:          # eval: running statistics are constants
-                    st[0].copy_(bn.running_mean); st[1].copy_(bn.running_var)
-                    st[2].copy_(torch.rsqrt(bn.running_var + bn.eps)); st[3].fill_(float(B))
+                if not training:
+                    _eval_stats(st, bn, B)
                 elif peer is not None:
                     n_glob = None
                 elif grp is not None:     # cross-rank: one all_gather of (mean, var, count), Chan combine, no host sync
@@ -834,12 +840,7 @@ class FusedMlpFn(torch.autograd.Function):
                                                _ptr(scratch), _stream()), "mlp_layer_bwd")
             dWs[i] = dW
             da = da_prev
-        flat = []
-        for i in range(nl):
-            flat += [dWs[i], dbs[i]]
-        for i in range(nl - 1):
-            flat += [dgs[i], dbes[i]]
-        return (da if ctx.needs_input_grad[0] else None, None, None, *flat)
+        return (da if ctx.needs_input_grad[0] else None, None, None, *_flat_params(dWs, dbs, dgs, dbes))
 
 
 STACK_MAX_WIDTH, STACK_MAX_LAYERS = 8, 16
@@ -880,17 +881,13 @@ class FusedMlpStackFn(torch.autograd.Function):
         x = _req(x, "x")
         B, dev = x.shape[0], x.device
         nl = len(plan.linears)
-        Ws = [_req(params[2 * i], "W") for i in range(nl)]
-        bs = [_req(params[2 * i + 1], "b") for i in range(nl)]
-        gs = [_req(params[2 * nl + 2 * i], "gamma") for i in range(nl - 1)]
-        bes = [_req(params[2 * nl + 2 * i + 1], "beta") for i in range(nl - 1)]
+        Ws, bs, gs, bes = _unpack_params(nl, params)
         scratch = _mlp_scratch(lib.b200vae_mlp_scratch_bytes(B), dev)
         ys = [torch.empty(B, W.shape[0], dtype=torch.float32, device=dev) for W in Ws]
         stats = [torch.empty(4, W.shape[0], dtype=torch.float32, device=dev) for W in Ws[:nl - 1]]
-        if not training:                  # eval: running statistics are constants
+        if not training:
             for st, bn in zip(stats, plan.bns):
-                st[0].copy_(bn.running_mean); st[1].copy_(bn.running_var)
-                st[2].copy_(torch.rsqrt(bn.running_var + bn.eps)); st[3].fill_(float(B))
+                _eval_stats(st, bn, B)
         layers = _stack_layers(plan, ys, stats, Ws, bs, gs, bes, training)
         mu = lv = None
         if head:
@@ -939,21 +936,12 @@ class FusedMlpStackFn(torch.autograd.Function):
         layers = _stack_layers(plan, ys, stats, Ws, bs, gs, bes, False)
         _C.check(lib.b200vae_mlp_stack_bwd(layers, garr, nl, _ptr(x), B, plan.slope, int(training), head, _ptr(g0),
                                            _ptr(g1), _ptr(dx), _ptr(ctx.scratch), _stream()), "mlp_stack_bwd")
-        out = []
-        for i in range(nl):
-            out += [dWs[i], dbs[i]]
-        for i in range(nl - 1):
-            out += [dgs[i], dbes[i]]
-        return (dx, None, None, None, *out)
+        return (dx, None, None, None, *_flat_params(dWs, dbs, dgs, dbes))
 
 
 def fused_mlp(plan, x, training, softplus_head=False):
     """Output of the stack; softplus_head: (mu, softplus(var)) of its two halves (LIDVAE.encode)."""
-    params = []
-    for l in plan.linears:
-        params += [l.weight, l.bias]
-    for b in plan.bns:
-        params += [b.weight, b.bias]
+    params = plan.params()
     if _stack_ok(plan, training):
         head = plan.linears[-1].out_features // 2 if softplus_head else 0
         return FusedMlpStackFn.apply(x, plan, training, head, *params)
