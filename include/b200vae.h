@@ -154,6 +154,33 @@ int b200vae_lipschitz_allpairs(const float* X, const float* Y, int N, int dx, in
                                int nbins, float hist_lo, float hist_hi, void* scratch, void* stream);
 long long b200vae_lipschitz_num_tiles(int N);
 
+/* Exact quantiles of the same keys over every pair i<j: the all-pairs version of the reference's figure, utils.py:563-567
+ * (A = quantile(r, q), B = quantile(r, 1-q) of the ratios).  A pair's key is exactly the value the entry above feeds into
+ * its min / max, so quantile 0 / 1 equal its min / max bit for bit.  Quantiles use torch.quantile's "linear" rule with the
+ * rank arithmetic in fp64 (torch does it in the tensor's dtype, which cannot address ranks beyond 2^24):
+ *   n = N(N-1)/2, pos = q (n-1), k = floor(pos), w = pos - k,  v(q) = key[k] + w (key[min(k+1, n-1)] - key[k])  (fp64).
+ * A radix select on the keys' bit patterns in B200VAE_LIPSCHITZ_SELECT_PASSES = 3 passes; per pass p = 0, 1, 2:
+ *   select_count(..., tile_begin, tile_end, p, state, hist)  on every rank (tiles split like the entry above): OVERWRITES
+ *       hist with the counts of its pairs' keys in the bins of pass p (integer atomics only: the same at any grid size);
+ *   sum hist over ranks (uint64 element-wise; skip on one rank);
+ *   select_locate(N, q0, q1, p, hist, state, out)  on every rank: narrows the targets (ranks k and k+1 of q0 and q1) in
+ *       `state`; pass 0 sets them from (N, q0, q1).  After pass 2: out [6] fp64 = (v(q0), v(q1), key[k0], key[k0+1],
+ *       key[k1], key[k1+1]).
+ * No host synchronisation inside, so a one-rank sequence can be captured into a CUDA graph.
+ *   state: b200vae_lipschitz_select_state_bytes(), hist: b200vae_lipschitz_select_hist_bytes() (uint64), both 16-byte
+ *   aligned, caller-owned, no initialisation needed.  Requires N >= 2 and eps > 0; B200VAE_EUNSUP when one CTA would count
+ *   2^32 or more pairs (N above about 2 million points). */
+#define B200VAE_LIPSCHITZ_SELECT_PASSES 3
+size_t b200vae_lipschitz_select_state_bytes(void);
+size_t b200vae_lipschitz_select_hist_bytes(void);
+/* host only: (k, w) of the rule above for n >= 1 keys and q in [0, 1] (else B200VAE_ESHAPE) */
+int b200vae_lipschitz_quantile_ranks(long long n, double q, long long* k, double* w);
+int b200vae_lipschitz_select_count(const float* X, const float* Y, int N, int dx, int dy, float eps,
+                                   long long tile_begin, long long tile_end, int pass, const void* state, uint64_t* hist,
+                                   void* stream);
+int b200vae_lipschitz_select_locate(int N, double q0, double q1, int pass, const uint64_t* hist, void* state, double* out,
+                                    void* stream);
+
 /* Fused Adam step over a flat fp32 parameter buffer (torch.optim.Adam semantics, lipschitz.py:25,43):
  *   m,v moments; step = 1-based step count; grad_scale multiplies g first (e.g. 1/world_size). */
 int b200vae_adam_step(float* param, const float* grad, float* m, float* v, long long n, float lr,

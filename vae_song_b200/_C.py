@@ -34,8 +34,10 @@ EXPORTS = [
     "b200vae_mlp_layer_bwd_reduce_peer", "b200vae_peer_allreduce_adam",
     "b200vae_icnn_wide_workspace_bytes", "b200vae_icnn_wide_fwd", "b200vae_icnn_wide_bwd", "b200vae_icnn_wide_bwd_psi",
     "b200vae_mi_logqz", "b200vae_nll_iw_lse", "b200vae_nll_iw_scratch_bytes", "b200vae_mlp_stack_fwd",
-    "b200vae_mlp_stack_bwd",
+    "b200vae_mlp_stack_bwd", "b200vae_lipschitz_select_state_bytes", "b200vae_lipschitz_select_hist_bytes",
+    "b200vae_lipschitz_quantile_ranks", "b200vae_lipschitz_select_count", "b200vae_lipschitz_select_locate",
 ]
+LIPSCHITZ_SELECT_PASSES = 3
 PEER_MAX_WORLD, PEER_HANDLE_BYTES = 16, 64
 
 
@@ -118,6 +120,17 @@ def load():
     lib.b200vae_lipschitz_scratch_bytes.argtypes = []
     lib.b200vae_lipschitz_num_tiles.restype = ll
     lib.b200vae_lipschitz_num_tiles.argtypes = [i]
+    d = C.c_double
+    lib.b200vae_lipschitz_select_state_bytes.restype = sz
+    lib.b200vae_lipschitz_select_state_bytes.argtypes = []
+    lib.b200vae_lipschitz_select_hist_bytes.restype = sz
+    lib.b200vae_lipschitz_select_hist_bytes.argtypes = []
+    lib.b200vae_lipschitz_quantile_ranks.restype = i
+    lib.b200vae_lipschitz_quantile_ranks.argtypes = [ll, d, C.POINTER(ll), C.POINTER(d)]
+    lib.b200vae_lipschitz_select_count.restype = i
+    lib.b200vae_lipschitz_select_count.argtypes = [vp, vp, i, i, i, f, ll, ll, i, vp, vp, vp]
+    lib.b200vae_lipschitz_select_locate.restype = i
+    lib.b200vae_lipschitz_select_locate.argtypes = [i, d, d, i, vp, vp, vp, vp]
     lib.b200vae_adam_step.restype = i
     lib.b200vae_adam_step.argtypes = [vp, vp, vp, vp, ll, f, f, f, f, f, ll, f, vp]
     lib.b200vae_adam_step_dev.restype = i

@@ -22,7 +22,7 @@ import torch
 
 from . import model as _model
 from .train import train_model  # noqa: F401  (lipschitz.py:23-44, same signature)
-from .utils import estimate_local_lipschitz, estimate_local_lipschitz_batched, reparameterize
+from .utils import estimate_lipschitz_allpairs, estimate_local_lipschitz, estimate_local_lipschitz_batched, reparameterize
 
 DEFAULT_EMPTY_CELL_FILL_VALUE = -5.0     # lipschitz.py:19
 
@@ -114,11 +114,18 @@ def _data_based_samples(model, test_dataset, device, num_samples):
 
 
 def _get_data_based_lipschitz(model, test_dataset, device, num_samples=5000, num_pairs_lips=5000,
-                              empty_cell_fill_value=DEFAULT_EMPTY_CELL_FILL_VALUE):
-    """lipschitz.py:157-194 -> (inverse_lipschitz, lipschitz, bi_lipschitz) floats."""
+                              empty_cell_fill_value=DEFAULT_EMPTY_CELL_FILL_VALUE, pairs="sampled"):
+    """lipschitz.py:157-194 -> (inverse_lipschitz, lipschitz, bi_lipschitz) floats.  pairs="all" (an extension) takes the
+    same triple over every pair of the same `num_samples` points instead of `num_pairs_lips` random pairs: exact
+    quantiles, utils.estimate_lipschitz_allpairs(quantile=0.05)."""
+    if pairs not in ("sampled", "all"):
+        raise ValueError(f"pairs must be 'sampled' or 'all', got {pairs!r}")
     model.eval()
     with torch.no_grad():
         z, _, _ = _data_based_samples(model, test_dataset, device, num_samples)
+        if pairs == "all":
+            r = estimate_lipschitz_allpairs(model.decode, z, quantile=0.05)
+            return r["inverse_lipschitz"], r["lipschitz"], r["bi_lipschitz"]
         return estimate_local_lipschitz(model.decode, z, num_pairs=num_pairs_lips)
 
 
@@ -194,11 +201,16 @@ def build_parser():
     p.add_argument("--wu_repeat_interval", type=int, default=10)
     p.add_argument("--precision", type=str, default="fp32", choices=["fp32", "f16x3", "tf32x3", "tf32"],
                    help="arithmetic of the ICNN contractions (extension; fp32 = the parity path)")
+    p.add_argument("--lipschitz_pairs", type=str, default="sampled", choices=["sampled", "all"],
+                   help="pairs of the data-based Lipschitz estimate (extension): the reference's random pairs, or every "
+                        "pair of the 5000 samples with exact quantiles; the per-cell grids always sample")
     return p
 
 
-def evaluate(model, dataset, K, K_z, z_min, z_max, latent_dim, device, num_pairs_cells=2000, num_pairs_data=5000):
-    """Steps 4-6 of lipschitz.main (lipschitz.py:423-520) without the plots."""
+def evaluate(model, dataset, K, K_z, z_min, z_max, latent_dim, device, num_pairs_cells=2000, num_pairs_data=5000,
+             lipschitz_pairs="sampled"):
+    """Steps 4-6 of lipschitz.main (lipschitz.py:423-520) without the plots; `lipschitz_pairs` as in
+    _get_data_based_lipschitz."""
     out = {}
     kx = _get_kl_and_lipschitz_for_x_cells(model, dataset, K, device, nsamples_z=10, num_pairs_lips=num_pairs_cells)
     out.update(dict(zip(("kl_x", "lips_x", "inv_lips_x", "bi_lips_x"), kx)))
@@ -206,7 +218,8 @@ def evaluate(model, dataset, K, K_z, z_min, z_max, latent_dim, device, num_pairs
         kz = _get_kl_and_lipschitz_for_z_cells(model, K_z, z_min, z_max, latent_dim, device, nsamples_z_per_cell=100,
                                                num_pairs_lips=num_pairs_cells)
         out.update(dict(zip(("kl_z", "lips_z", "inv_lips_z", "bi_lips_z"), kz)))
-    inv_l, l, bi = _get_data_based_lipschitz(model, dataset, device, num_samples=5000, num_pairs_lips=num_pairs_data)
+    inv_l, l, bi = _get_data_based_lipschitz(model, dataset, device, num_samples=5000, num_pairs_lips=num_pairs_data,
+                                             pairs=lipschitz_pairs)
     out["data_inv_lips"], out["data_lips"], out["data_bi_lips"] = inv_l, l, bi
     out["data_kl"] = _get_data_based_kl(model, dataset, device, num_samples=5000)
     return out
@@ -245,12 +258,14 @@ def main(argv=None):
             z_min, z_max = float(zt[:, 0].min()), float(zt[:, 0].max())
     if args.model != "lidvae":
         model.alpha = model.wu_alpha = args.alpha
-    res = evaluate(model, train_dataset, args.K, args.K_z, z_min, z_max, latent_dim, args.device)
+    res = evaluate(model, train_dataset, args.K, args.K_z, z_min, z_max, latent_dim, args.device,
+                   lipschitz_pairs=args.lipschitz_pairs)
     arrays = {k: v for k, v in res.items() if isinstance(v, np.ndarray)}
     scalars = {k: float(v) for k, v in res.items() if not isinstance(v, np.ndarray)}
     np.savez(os.path.join(args.output_dir, "metrics.npz"), **arrays)
     with open(os.path.join(args.output_dir, "summary.json"), "w") as f:
-        json.dump(dict(args=vars(args), z_extent=[z_min, z_max], **scalars), f, indent=1)
+        json.dump(dict(args=vars(args), z_extent=[z_min, z_max], data_lipschitz_pairs=args.lipschitz_pairs, **scalars), f,
+                  indent=1)
     print(json.dumps(scalars))
     return res
 

@@ -1043,6 +1043,69 @@ def lipschitz_num_tiles(N):
     return int(_C.load().b200vae_lipschitz_num_tiles(N))
 
 
+# exact all-pairs quantiles: a 3-pass radix select over the keys of lipschitz_allpairs (include/b200vae.h)
+_select_buffers = {}
+
+
+def lipschitz_select_buffers(device):
+    """(state uint8, hist int64) per (device, stream), allocated on first use; the passes need no initialisation.  Make one
+    call on a stream before capturing it into a CUDA graph, so that the capture allocates nothing."""
+    key = (device, torch.cuda.current_stream().cuda_stream)
+    bufs = _select_buffers.get(key)
+    if bufs is None:
+        if torch.cuda.is_current_stream_capturing():
+            raise _C.B200VaeError("lipschitz_allpairs_quantiles: make one call on this stream before capturing it")
+        lib = _C.load()
+        bufs = _select_buffers[key] = (
+            torch.empty(lib.b200vae_lipschitz_select_state_bytes(), dtype=torch.uint8, device=device),
+            torch.empty(lib.b200vae_lipschitz_select_hist_bytes() // 8, dtype=torch.int64, device=device))
+    return bufs
+
+
+def lipschitz_select_count(X, Y, eps, tile_begin, tile_end, pass_, state, hist):
+    """One count pass over the pairs of tiles [tile_begin, tile_end): OVERWRITES `hist` (int64) with this shard's bins."""
+    X = _req(X.detach().reshape(X.shape[0], -1), "X")
+    Y = _req(Y.detach().reshape(Y.shape[0], -1), "Y")
+    _C.check(_C.load().b200vae_lipschitz_select_count(_ptr(X), _ptr(Y), X.shape[0], X.shape[1], Y.shape[1], float(eps),
+                                                      int(tile_begin), int(tile_end), int(pass_), _ptr(state), _ptr(hist),
+                                                      _stream()), "lipschitz_select_count")
+
+
+def lipschitz_select_locate(N, q0, q1, pass_, hist, state, out):
+    """Narrow the targets with `hist` (summed over every shard); after the last pass out (fp64 [6]) holds
+    (v(q0), v(q1), key[k0], key[k0+1], key[k1], key[k1+1])."""
+    _C.check(_C.load().b200vae_lipschitz_select_locate(int(N), float(q0), float(q1), int(pass_), _ptr(hist), _ptr(state),
+                                                       _ptr(out), _stream()), "lipschitz_select_locate")
+
+
+def lipschitz_quantile_ranks(n, q):
+    """(k, w) of torch.quantile's linear rule for n values, in fp64 (the library owns the rule)."""
+    k, w = C.c_longlong(), C.c_double()
+    _C.check(_C.load().b200vae_lipschitz_quantile_ranks(int(n), float(q), C.byref(k), C.byref(w)), "lipschitz_quantile_ranks")
+    return k.value, w.value
+
+
+def lipschitz_allpairs_quantiles(X, Y, qs, eps=1e-3, tile_begin=0, tile_end=None, reduce_hist=None):
+    """Exact quantiles (torch.quantile's linear rule, ranks in fp64) of the keys of `lipschitz_allpairs` over every pair
+    i<j: one or two quantiles `qs`.  Returns a new fp64 device tensor [6] = (v(qs[0]), v(qs[-1]), the two order statistics
+    behind each).  With shards, every rank passes its tile range and `reduce_hist(hist)` sums the int64 histogram over the
+    ranks in place between count and locate.  No host synchronisation: capturable into a CUDA graph (call once first)."""
+    qs = [float(q) for q in qs]
+    if not 1 <= len(qs) <= 2:
+        raise ValueError("lipschitz_allpairs_quantiles: one or two quantiles")
+    N = X.shape[0]
+    if tile_end is None:
+        tile_end = lipschitz_num_tiles(N)
+    state, hist = lipschitz_select_buffers(X.device)
+    out = torch.empty(6, dtype=torch.float64, device=X.device)
+    for p in range(_C.LIPSCHITZ_SELECT_PASSES):
+        lipschitz_select_count(X, Y, eps, tile_begin, tile_end, p, state, hist)
+        if reduce_hist is not None:
+            reduce_hist(hist)
+        lipschitz_select_locate(N, qs[0], qs[-1], p, hist, state, out)
+    return out
+
+
 # ------------------------------------------------------------------------------------------ Adam
 def adam_step_(param, grad, m, v, step, lr=1e-3, betas=(0.9, 0.999), eps=1e-8, weight_decay=0.0, grad_scale=1.0):
     """In-place fused Adam over flat fp32 buffers (torch.optim.Adam semantics; lipschitz.py:25,43)."""

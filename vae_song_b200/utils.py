@@ -251,12 +251,19 @@ def estimate_local_lipschitz_batched(func, X_list, num_pairs=2000, quantile=0.05
 
 
 def estimate_lipschitz_allpairs(func, X, eps=1e-3, process_group=None, nbins=0, hist_range=(-20.0, 20.0), peer=None,
-                                shard_decode=True):
+                                shard_decode=True, quantile=None):
     """All-pairs max / min / mean of |f(x)-f(y)|/|x-y| over every unordered pair (north_star kernel 4).
     With a process group (X replicated on every rank) BOTH stages shard: rank r decodes rows [r*per, (r+1)*per) and the
     outputs are all-gathered; the 64x64 pair tiles are split by range (`tile_range`) and the per-rank statistics combined
     with ONE exchange -- `peer` (a peer.PeerComm: an own all-gather kernel over NVLink peer memory, ~13 us) or one
-    torch.distributed all_gather.  Returns dict(max, min, mean, count[, hist])."""
+    torch.distributed all_gather.  Returns dict(max, min, mean, count[, hist]).
+
+    `quantile` = q adds the reference's estimate (utils.py:563-567) over EVERY pair instead of sampled ones: the exact
+    quantiles v(q), v(1-q) of the same ratios (ops.lipschitz_allpairs_quantiles: torch.quantile's linear rule, ranks in
+    fp64), A = max(v(q), eps), B = v(1-q) -> keys inverse_lipschitz = 1/A, lipschitz = B, bi_lipschitz = max(1/A, B) and
+    quantiles = (v(q), v(1-q)); (0, 0, 0) for fewer than 2 points.  Sharded like the statistics, each of the three passes'
+    histograms summed with one all_reduce.  One difference from the sampled estimator: its random pairs may draw i == j
+    (ratio 1.0 through both clamps), all pairs i < j never do."""
     import torch.distributed as dist
     rank, world = 0, 1
     if process_group is not None or (dist.is_available() and dist.is_initialized()):
@@ -292,6 +299,16 @@ def estimate_lipschitz_allpairs(func, X, eps=1e-3, process_group=None, nbins=0, 
     out = dict(max=mx, min=mn, mean=sm / max(cnt, 1.0), count=int(cnt))
     if hist is not None:
         out["hist"] = hist
+    if quantile is not None:
+        if N < 2:
+            out.update(inverse_lipschitz=0.0, lipschitz=0.0, bi_lipschitz=0.0, quantiles=(0.0, 0.0))
+            return out
+        reduce_hist = None
+        if world > 1:
+            reduce_hist = lambda h: dist.all_reduce(h, op=dist.ReduceOp.SUM, group=process_group)   # noqa: E731
+        v = ops.lipschitz_allpairs_quantiles(X, Y, (quantile, 1.0 - quantile), eps, lo, hi, reduce_hist)[:2].tolist()
+        inv = 1.0 / max(v[0], eps)
+        out.update(inverse_lipschitz=inv, lipschitz=v[1], bi_lipschitz=max(inv, v[1]), quantiles=(v[0], v[1]))
     return out
 
 
