@@ -279,10 +279,14 @@ int b200vae_nn_sqdist_bwd(const float* A, const float* Bp, const int* argA, cons
  * for the backward; g0 (fwd) and u0,q1,g0,t0 (bwd) are [B,H] fp32 scratch.  psi may be NULL; xhat NULL = psi only.
  * b200vae_icnn_wide_bwd takes v = dL/dxhat (the psi-gradient path is b200vae_icnn_wide_bwd_psi below) and OVERWRITES every
  * non-null field of `g` and dz.
- * `precision` (forward): FP32 = the tile-GEMM chain above; TF32 / TF32X3 = the same chain on tcgen05 (csrc/icnn_wide_tc.cu:
- * TMA-fed 128x256 tiles, transform + hi/lo split of the A tile in shared memory, accumulators in TMEM) when d, nz, H are
- * multiples of 4, else FP32.  Backward with TF32 / TF32X3: the sample-stationary GEMMs (u0, w1, gx1, dz) run on the same
- * tcgen05 kernel, the batch-reduction GEMMs (dA0, dA1, dP0) stay FP32; it works on whatever forward produced h0/mask1/s2.
+ * `precision`: FP32 = the tile-GEMM chain above; TF32 / TF32X3 = every GEMM of the call on tcgen05 (csrc/icnn_wide_tc.cu:
+ * TMA-fed 128x256 tiles, transform + hi/lo split of the A tile in shared memory, accumulators in TMEM) -- in the backward
+ * the sample-stationary GEMMs (u0, w1, gx1, dz) and the batch-reduction GEMMs (dA0, dA1, dP0) alike; F16X3 runs as
+ * TF32X3 (the operands come from HBM: there is no fp16 variant).  A tensor-core precision falls back to the FP32 chain
+ * when d, nz or H is not a multiple of 4, and in the forward also when A0b, A1b or A2w is not 16-byte aligned (the
+ * tensor-core epilogues read them with 16-byte loads).  Either backward works on whatever forward produced h0/mask1/s2.
+ * b200vae_icnn_wide_workspace_bytes returns 0 for a shape or precision the entries refuse; for a tensor-core precision
+ * it is the larger of the two paths' workspaces, since it sees neither nz nor the parameters' alignment.
  * `nz` (1 <= nz <= d): z is [B,nz] and the ICNN input is z ZERO-PADDED to d columns -- the x = x1 B^T step of
  * model.py:824 with B = eye(Dx, D) fused away (nz = D = 32, d = Dx = 784): products with z run over nz columns only,
  * xhat is [B,d], v is [B,d], dz is [B,nz].  nz = d is the plain case. */

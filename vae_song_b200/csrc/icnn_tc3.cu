@@ -1623,34 +1623,10 @@ tc_finalize_small_kernel(const float* __restrict__ partA, const float* __restric
 }
 
 // ------------------------------------------------------------------------------------ host side
-typedef CUresult (*EncodeTiledFn3)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                   const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
-                                   CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
 // arithmetic of the pair kernels for an ABI precision id
 static int tc3_mode(int precision) {
   return precision == B200VAE_PREC_F16X3 ? kF16 : precision == B200VAE_PREC_TF32X3 ? kX3 : kTf32;
 }
-static int make_map3(CUtensorMap* m, const float* base, int K, int rows, bool f16 = false) {
-  static EncodeTiledFn3 fn = nullptr;
-  if (!fn) {
-    void* p = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess && p)
-      fn = reinterpret_cast<EncodeTiledFn3>(p);
-  }
-  if (!fn) return B200VAE_ECUDA;
-  // 64-byte rows either way: 16 fp32 / 32 fp16 K elements x this CTA's 128 rows
-  const cuuint64_t dims[2] = {(cuuint64_t)K, (cuuint64_t)rows};
-  const cuuint64_t strides[1] = {(cuuint64_t)K * (f16 ? sizeof(__half) : sizeof(float))};
-  const cuuint32_t box[2] = {(cuuint32_t)(f16 ? 32 : kKB), (cuuint32_t)k3Rows};
-  const cuuint32_t estr[2] = {1, 1};
-  CUresult r = fn(m, f16 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, const_cast<float*>(base), dims, strides, box, estr,
-                  CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                  CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) { g_last_cuda_error = 100000 + (int)r; return B200VAE_ECUDA; }
-  return B200VAE_OK;
-}
-
 // the per-unit tables and the pair kernels' operands, from the FP32 arrays simt_prepare wrote
 int tc3_prepare(const WsLayout& L, int precision, float* ws, cudaStream_t st) {
   tc_prepare_kernel<<<(L.Hq + 255) / 256, 256, 0, st>>>(ws + L.P1, ws + L.A0p, ws + L.A1p, L.d, L.Hp, L.Hq,
@@ -1698,10 +1674,10 @@ static int get_maps3(const float* ws, const WsLayout& L, int mode, Tc3Maps* out)
   Tc3Maps mp;
   const bool hl = mode != kTf32, f16 = mode == kF16;
   const int K1 = f16 ? L.Hq : L.K1;
-  int rc = make_map3(&mp.b1hi, ws + L.B1ahi, K1, L.Hq, f16);
-  if (!rc) rc = make_map3(&mp.b1lo, ws + (hl ? L.B1alo : L.B1ahi), K1, L.Hq, f16);
-  if (!rc) rc = make_map3(&mp.b2hi, ws + L.B2ghi, L.Hq, L.Hq, f16);
-  if (!rc) rc = make_map3(&mp.b2lo, ws + (hl ? L.B2glo : L.B2ghi), L.Hq, L.Hq, f16);
+  int rc = tma_map_2d(&mp.b1hi, ws + L.B1ahi, K1, L.Hq, K1, k3Rows, f16);
+  if (!rc) rc = tma_map_2d(&mp.b1lo, ws + (hl ? L.B1alo : L.B1ahi), K1, L.Hq, K1, k3Rows, f16);
+  if (!rc) rc = tma_map_2d(&mp.b2hi, ws + L.B2ghi, L.Hq, L.Hq, L.Hq, k3Rows, f16);
+  if (!rc) rc = tma_map_2d(&mp.b2lo, ws + (hl ? L.B2glo : L.B2ghi), L.Hq, L.Hq, L.Hq, k3Rows, f16);
   if (rc) return rc;
   if (cache.size() > 256) cache.clear();
   cache.emplace(key, mp);

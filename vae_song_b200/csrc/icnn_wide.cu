@@ -1,5 +1,6 @@
 // icnn_wide.cu -- fused FP32 kernels for WIDE-input ICNNs (d > 4): the MNIST-shaped LIDVAE decoder of BASELINE
-// configs[3], ICNN(32,512) + ICNN(784,1024) (model.py:766-805, module.py:117-148).
+// configs[3], ICNN(32,512) + ICNN(784,1024) (model.py:766-805, module.py:117-148).  Also the b200vae_icnn_wide_* entries:
+// validation, the workspace size, and the choice between these kernels and the tcgen05 drivers of icnn_wide_tc.cu.
 //
 // For wide inputs the thin products A.z are dense [B,d]x[d,H] contractions too, so per-sample activations no longer fit in
 // registers.  The path is a short chain of 128x128x16 FP32 tile GEMMs (gemm_simt.cuh) whose A operands are GENERATED while
@@ -17,6 +18,7 @@
 //             tn  : dA0 = g0^T v + t0^T z,  dA1 = g1^T v,  dP0 = g1^T q1     (split over the batch, ordered slabs)
 // Algebra: SURVEY.md Appendix A (oracle/icnn_oracle.py).  All reductions are ordered: bit-reproducible.
 #include "gemm_simt.cuh"
+#include "icnn_wide.cuh"
 
 namespace b200vae {
 
@@ -168,38 +170,6 @@ __device__ __forceinline__ BMat make_bmat(const float* Mx, int ld, int kbeg, int
 __device__ __forceinline__ int ktiles(int K) { return (K + kBK - 1) / kBK; }
 
 // ---- prepare: P0, P0^T, P1, A0^T, A1^T (unpadded; the generators guard the edges) ------------------------------------------------
-struct WideWs {
-  size_t P0, P0T, P1, A0T, A1T, part, colpart, slabs, end;
-  int mt, nt, splits;
-};
-__host__ __device__ inline size_t up64(size_t x) { return (x + 63) / 64 * 64; }
-inline int wide_splits(int B, int tiles) {
-  int want = (148 * 2 + tiles - 1) / tiles, maxs = (B + 127) / 128;
-  int s = want < maxs ? want : maxs;
-  return s < 1 ? 1 : (s > 32 ? 32 : s);
-}
-inline WideWs wide_layout(int B, int d, int H, bool bwd) {
-  WideWs L;
-  size_t o = 0;
-  L.mt = (B + 127) / 128; L.nt = (H + 127) / 128;
-  L.P0 = o; o += up64((size_t)H * H);
-  L.P0T = o; o += up64((size_t)H * H);
-  L.P1 = o; o += up64(H);
-  L.A0T = o; o += up64((size_t)d * H);
-  L.A1T = o; o += up64((size_t)d * H);
-  L.part = o; o += up64((size_t)B * L.nt);
-  L.colpart = o; L.slabs = o; L.splits = 1;
-  if (bwd) {
-    const int w = H > d ? H : d;
-    o += up64((size_t)L.mt * w);
-    L.slabs = o;
-    L.splits = wide_splits(B, L.nt * L.nt);
-    o += up64((size_t)L.splits * H * (H > d ? H : d));
-  }
-  L.end = o;
-  return L;
-}
-
 __global__ void wide_prepare_kernel(const float* __restrict__ W0, const float* __restrict__ W1, const float* __restrict__ A0w,
                                     const float* __restrict__ A1w, int d, int H, int mode, float* __restrict__ P0,
                                     float* __restrict__ P0T, float* __restrict__ P1, float* __restrict__ A0T,
@@ -478,14 +448,14 @@ wide_tn_kernel(TnArgs p, float* __restrict__ slabs) {
     }
   }
 }
-// out[i] = chain( sum_s slabs[s][i] ):  chain 0 none, 1 *P (exp: dW = dP*P), 2 *[W >= 1e-2] (clamp)
+// chain 1 recomputes P = exp(W): the tensor-core path keeps no fp32 copy of P0, and expf gives the prepare's bits
 __global__ void wide_slab_finalize_kernel(const float* __restrict__ slabs, int splits, size_t n, int chain,
-                                          const float* __restrict__ P, const float* __restrict__ W, float* __restrict__ out) {
+                                          const float* __restrict__ W, float* __restrict__ out) {
   const size_t gstride = (size_t)gridDim.x * blockDim.x;
   for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gstride) {
     float s = 0.f;
     for (int k = 0; k < splits; ++k) s += slabs[(size_t)k * n + i];
-    if (chain == 1) s *= P[i];
+    if (chain == 1) s *= expf(W[i]);
     else if (chain == 2) s = W[i] >= kClampMin ? s : 0.f;
     out[i] = s;
   }
@@ -564,7 +534,78 @@ __global__ void wide_slab_finalize_ld_kernel(const float* __restrict__ slabs, in
   }
 }
 
-static int wide_prepare(const b200vae_icnn_params* p, int d, int H, int mode, float* ws, const WideWs& L, cudaStream_t st) {
+// ---- launchers of the kernels the tensor-core path shares (icnn_wide.cuh) ------------------------------------------------------
+int wide_row(const float* part, int npart, const float* z, const b200vae_icnn_params* p, int B, int nz, float* psi, float* s2,
+             cudaStream_t st) {
+  wide_row_kernel<<<(B + 7) / 8, 256, 0, st>>>(part, npart, z, p->A2w, p->A2b, B, nz, psi, s2);
+  return check_launch();
+}
+int wide_col_finalize(const float* colpart, int mt, int w, int chain, const float* P, const float* W, float* out,
+                      cudaStream_t st) {
+  wide_col_finalize_kernel<<<(w + 255) / 256, 256, 0, st>>>(colpart, mt, w, chain, P, W, out);
+  return check_launch();
+}
+int wide_slab_finalize(const float* slabs, int splits, size_t n, int chain, const float* W, float* out, cudaStream_t st) {
+  wide_slab_finalize_kernel<<<148 * 4, 256, 0, st>>>(slabs, splits, n, chain, W, out);
+  return check_launch();
+}
+
+// ---- workspace layout (map: icnn_wide.cuh) ---------------------------------------------------------------------------------
+// slabs of a split-batch GEMM: enough to give `ctas` CTAs over `tiles` output tiles, at least `rows` samples per slab
+static int wide_splits(int B, int tiles, int ctas, int rows, int cap) {
+  int s = (ctas + tiles - 1) / tiles, maxs = (B + rows - 1) / rows;
+  s = s < maxs ? s : maxs;
+  return s < 1 ? 1 : (s > cap ? cap : s);
+}
+WideLayout wide_ws_layout(int B, int d, int H, bool tc, bool for_backward) {
+  WideLayout L = {};
+  L.mt = (B + 127) / 128; L.nt = (H + 127) / 128;
+  L.splits = 1;
+  const size_t HH = (size_t)H * H, dH = (size_t)d * H, w = H > d ? H : d;
+  size_t o = 0;
+  auto take = [&](size_t n) { const size_t at = o; o += (n + 63) / 64 * 64; return at; };
+  if (!tc) {
+    L.P0 = take(HH); L.P0T = take(HH); L.P1 = take(H); L.A0T = take(dH); L.A1T = take(dH);
+    L.part = take((size_t)B * L.nt);
+    if (for_backward) {
+      L.colpart = take(L.mt * w);
+      L.splits = wide_splits(B, L.nt * L.nt, 148 * 2, 128, 32);
+      L.slabs = take(L.splits * H * w);
+    }
+  } else {
+    L.P0hi = take(HH); L.P0lo = take(HH); L.P0Thi = take(HH); L.P0Tlo = take(HH);
+    L.A0hi = take(dH); L.A0lo = take(dH); L.A1hi = take(dH); L.A1lo = take(dH);
+    L.A0Thi = take(dH); L.A0Tlo = take(dH); L.A1Thi = take(dH); L.A1Tlo = take(dH);
+    L.P1 = take(H); L.g1b = take((size_t)B * H);
+    L.part = take((size_t)B * L.nt * 2);                  // two per 128-column (3xTF32) / 256-column (TF32) tile
+    if (for_backward) {
+      L.colpart = take(L.mt * w);
+      L.ldb = (B + 3) / 4 * 4;
+      const size_t HB = (size_t)H * L.ldb, dB = (size_t)d * L.ldb;
+      L.g0T = take(HB); L.t0T = take(HB); L.g1T = take(HB);
+      L.vThi = take(dB); L.vTlo = take(dB); L.zThi = take(dB); L.zTlo = take(dB); L.q1Thi = take(HB); L.q1Tlo = take(HB);
+      L.splits = wide_splits(B, L.nt * ((H + 255) / 256), 148, 256, 16);
+      L.slabs = take(L.splits * H * w);
+    }
+  }
+  L.end = o;
+  return L;
+}
+
+// every wide entry's and the size query's check: shapes, and a precision id the wide kernels run (2 is reserved)
+static int wide_shape_ok(int B, int d, int nz, int H, int precision) {
+  if (B <= 0 || d <= 0 || H <= 0 || nz <= 0 || nz > d) return B200VAE_ESHAPE;
+  if (precision != B200VAE_PREC_FP32 && precision != B200VAE_PREC_TF32 && precision != B200VAE_PREC_TF32X3 &&
+      precision != B200VAE_PREC_F16X3)
+    return B200VAE_EUNSUP;
+  return B200VAE_OK;
+}
+// The wide kernels read their operands from HBM and have no fp16 variant: F16X3 runs as TF32X3.
+static int wide_precision(int precision) {
+  return precision == B200VAE_PREC_F16X3 ? B200VAE_PREC_TF32X3 : precision;
+}
+
+static int wide_prepare(const b200vae_icnn_params* p, int d, int H, int mode, float* ws, const WideLayout& L, cudaStream_t st) {
   wide_prepare_kernel<<<148 * 4, 256, 0, st>>>(p->W0, p->W1, p->A0w, p->A1w, d, H, mode, ws + L.P0, ws + L.P0T, ws + L.P1,
                                               ws + L.A0T, ws + L.A1T);
   return check_launch();
@@ -577,29 +618,16 @@ static bool wide_params_ok(const b200vae_icnn_params* p) {
 
 using namespace b200vae;
 
-namespace b200vae {   // tcgen05 forward, icnn_wide_tc.cu
-size_t wide_tc_ws_floats(int B, int d, int H);
-bool wide_tc_supported(int d, int nz, int H, int precision);
-int wide_tc_fwd(const float* z, int B, int d, int nz, int H, const b200vae_icnn_params* p, int mode, float kappa, float* psi,
-                float* xhat, float* h0, uint8_t* mask1, float* s2, float* g0, float* ws, int precision, cudaStream_t st);
-int wide_tc_bwd_rows(const float* v, const float* h0, const uint8_t* mask1, const float* s2, int B, int d, int nz, int H,
-                     const b200vae_icnn_params* p, int mode, float kappa, float* dz, float* u0, float* q1, float* g0, float* t0,
-                     float* dW1, float* db0, float* ws, float* colpart, int precision, cudaStream_t st);
-size_t wide_tc_tn_ws_floats(int B, int d, int H);
-int wide_tc_bwd_tn(const float* z, const float* v, const uint8_t* mask1, const float* s2, const float* q1, const float* g0,
-                   const float* t0, int B, int d, int nz, int H, const b200vae_icnn_params* p, int mode, const float* P1,
-                   float* dA0w, float* dA1w, float* dW0, float* ws, int precision, cudaStream_t st);
-}
-
+// A tensor-core precision gets the larger of the two paths' layouts: the query sees neither nz nor the parameters'
+// alignment, and either can send a call to the FP32 kernels.
 extern "C" size_t b200vae_icnn_wide_workspace_bytes(int B, int d, int H, int precision, int for_backward) {
-  if (B <= 0 || d <= 0 || H <= 0) return 0;
-  size_t fl = wide_layout(B, d, H, for_backward != 0).end;
+  if (wide_shape_ok(B, d, d, H, precision)) return 0;
+  size_t n = wide_ws_layout(B, d, H, false, for_backward != 0).end;
   if (precision != B200VAE_PREC_FP32) {
-    const size_t t = wide_tc_ws_floats(B, d, H);
-    if (for_backward) fl += t + wide_tc_tn_ws_floats(B, d, H);   // FP32 layout, then the tensor-core layouts (rows, batch-reduction)
-    else if (t > fl) fl = t;
+    const size_t t = wide_ws_layout(B, d, H, true, for_backward != 0).end;
+    if (t > n) n = t;
   }
-  return fl * sizeof(float);
+  return n * sizeof(float);
 }
 
 #define WIDE_CHECK() do { rc = check_launch(); if (rc) return rc; } while (0)
@@ -607,25 +635,22 @@ extern "C" size_t b200vae_icnn_wide_workspace_bytes(int B, int d, int H, int pre
 extern "C" int b200vae_icnn_wide_fwd(const float* z, int B, int d, int nz, int H, const b200vae_icnn_params* p, int weight_mode,
                                      float kappa, float* psi, float* xhat, float* h0, uint8_t* mask1, float* s2, float* g0,
                                      int precision, void* workspace, size_t ws_bytes, void* stream) {
+  int rc = wide_shape_ok(B, d, nz, H, precision);
+  if (rc) return rc;
   if (!z || !wide_params_ok(p) || !h0 || !mask1 || !s2 || !workspace || (xhat && !g0)) return B200VAE_EALIGN;
-  if (B <= 0 || d <= 0 || H <= 0 || nz <= 0 || nz > d) return B200VAE_ESHAPE;
   if (weight_mode != B200VAE_WEIGHT_EXP && weight_mode != B200VAE_WEIGHT_CLAMP) return B200VAE_EUNSUP;
-  if (precision == B200VAE_PREC_F16X3) precision = B200VAE_PREC_TF32X3;   // the wide kernels read their operands from HBM: no fp16 variant
-  if (precision < B200VAE_PREC_FP32 || precision > B200VAE_PREC_TF32X3 || precision == 2 /* reserved */) return B200VAE_EUNSUP;
-  const WideWs L = wide_layout(B, d, H, false);
   if (ws_bytes < b200vae_icnn_wide_workspace_bytes(B, d, H, precision, 0)) return B200VAE_EWS;
   if (!aligned16(workspace) || !aligned16(z) || !aligned16(h0) || !aligned4(p->A0w) || !aligned4(p->A1w) ||
       (g0 && !aligned16(g0)) || (xhat && !aligned16(xhat)))
     return B200VAE_EALIGN;
+  precision = wide_precision(precision);
   // the tcgen05 epilogues read b0, b1, A2 with 16-byte loads; parameters at odd offsets take the FP32 kernels
-  const bool p16 = aligned16(p->A0b) && aligned16(p->A1b) && aligned16(p->A2w);
+  const bool tc = wide_tc_supported(d, nz, H, precision) && aligned16(p->A0b) && aligned16(p->A1b) && aligned16(p->A2w);
+  const WideLayout L = wide_ws_layout(B, d, H, tc, false);
   cudaStream_t st = (cudaStream_t)stream;
   float* ws = (float*)workspace;
-  if (precision != B200VAE_PREC_FP32 && p16 && wide_tc_supported(d, nz, H, precision)) {   // tcgen05 forward
-    const int rc_tc = wide_tc_fwd(z, B, d, nz, H, p, weight_mode, kappa, psi, xhat, h0, mask1, s2, g0, ws, precision, st);
-    if (rc_tc != B200VAE_EUNSUP) return rc_tc;
-  }
-  int rc = wide_prepare(p, d, H, weight_mode, ws, L, st);
+  if (tc) return wide_tc_fwd(z, B, d, nz, H, p, weight_mode, kappa, psi, xhat, h0, mask1, s2, g0, ws, L, precision, st);
+  rc = wide_prepare(p, d, H, weight_mode, ws, L, st);
   if (rc) return rc;
   const dim3 gH(L.mt, L.nt), gD(L.mt, (d + 127) / 128);
   // z is [B,nz]: the input is z zero-padded to d columns, so every product with z runs over nz only
@@ -634,15 +659,13 @@ extern "C" int b200vae_icnn_wide_fwd(const float* z, int B, int d, int nz, int H
   wide_hid_kernel<<<gH, kThreads, 0, st>>>(h0, XF_X1, ws + L.P0T, z, ws + L.A1T, p->A1b, ws + L.P1, B, nz, H, 0, mask1, nullptr,
                                           ws + L.part, nullptr);
   WIDE_CHECK();
-  wide_row_kernel<<<(B + 7) / 8, 256, 0, st>>>(ws + L.part, L.nt, z, p->A2w, p->A2b, B, nz, psi, s2);
+  rc = wide_row(ws + L.part, L.nt, z, p, B, nz, psi, s2, st);
+  if (rc || !xhat) return rc;
+  wide_gx1_kernel<<<gH, kThreads, 0, st>>>(mask1, s2, ws + L.P1, ws + L.P0, h0, nullptr, B, H, g0, nullptr, nullptr);
   WIDE_CHECK();
-  if (xhat) {
-    wide_gx1_kernel<<<gH, kThreads, 0, st>>>(mask1, s2, ws + L.P1, ws + L.P0, h0, nullptr, B, H, g0, nullptr, nullptr);
-    WIDE_CHECK();
-    wide_out_kernel<<<gD, kThreads, 0, st>>>(g0, p->A0w, 1, mask1, s2, ws + L.P1, p->A1w, p->A2w, z, nz, nz, 2.f * kappa, B, d, d, H,
-                                            xhat);
-    WIDE_CHECK();
-  }
+  wide_out_kernel<<<gD, kThreads, 0, st>>>(g0, p->A0w, 1, mask1, s2, ws + L.P1, p->A1w, p->A2w, z, nz, nz, 2.f * kappa, B, d, d, H,
+                                          xhat);
+  WIDE_CHECK();
   return B200VAE_OK;
 }
 
@@ -650,100 +673,87 @@ extern "C" int b200vae_icnn_wide_bwd(const float* z, const float* v, const float
                                      int B, int d, int nz, int H, const b200vae_icnn_params* p, int weight_mode, float kappa,
                                      const b200vae_icnn_grads* g, float* dz, float* u0, float* q1, float* g0, float* t0,
                                      int precision, void* workspace, size_t ws_bytes, void* stream) {
+  int rc = wide_shape_ok(B, d, nz, H, precision);
+  if (rc) return rc;
   if (!z || !v || !h0 || !mask1 || !s2 || !wide_params_ok(p) || !u0 || !q1 || !g0 || !t0 || !workspace) return B200VAE_EALIGN;
-  if (B <= 0 || d <= 0 || H <= 0 || nz <= 0 || nz > d) return B200VAE_ESHAPE;
   if (weight_mode != B200VAE_WEIGHT_EXP && weight_mode != B200VAE_WEIGHT_CLAMP) return B200VAE_EUNSUP;
-  if (precision == B200VAE_PREC_F16X3) precision = B200VAE_PREC_TF32X3;   // the wide kernels read their operands from HBM: no fp16 variant
-  if (precision < B200VAE_PREC_FP32 || precision > B200VAE_PREC_TF32X3 || precision == 2 /* reserved */) return B200VAE_EUNSUP;
-  const WideWs L = wide_layout(B, d, H, true);
   if (ws_bytes < b200vae_icnn_wide_workspace_bytes(B, d, H, precision, 1)) return B200VAE_EWS;
   if (!aligned16(workspace) || !aligned16(z) || !aligned16(v) || !aligned16(h0) || !aligned16(u0) || !aligned16(q1) ||
       !aligned16(g0) || !aligned16(t0) || !aligned4(p->A0w) || !aligned4(p->A1w) || (dz && !aligned16(dz)))
     return B200VAE_EALIGN;
+  precision = wide_precision(precision);
+  const bool tc = wide_tc_supported(d, nz, H, precision);
+  const WideLayout L = wide_ws_layout(B, d, H, tc, true);
   cudaStream_t st = (cudaStream_t)stream;
   float* ws = (float*)workspace;
   const int chain = weight_mode == B200VAE_WEIGHT_EXP ? 1 : 2;
-  int rc = wide_prepare(p, d, H, weight_mode, ws, L, st);
-  if (rc) return rc;
-  const dim3 gH(L.mt, L.nt), gD(L.mt, (d + 127) / 128);
-  bool rows_done = false;
-  if (precision != B200VAE_PREC_FP32 && wide_tc_supported(d, nz, H, precision)) {
-    // sample-stationary GEMMs on tcgen05 (icnn_wide_tc.cu); the batch-reduction GEMMs below stay FP32
+  const dim3 gH(L.mt, L.nt);
+  if (tc) {
     rc = wide_tc_bwd_rows(v, h0, mask1, s2, B, d, nz, H, p, weight_mode, kappa, dz, u0, q1, g0, t0, g ? g->W1 : nullptr,
-                          g ? g->A0b : nullptr, ws + L.end, ws + L.colpart, precision, st);
-    if (rc == B200VAE_OK) rows_done = true;
-    else if (rc != B200VAE_EUNSUP) return rc;
-  }
-  if (!rows_done) {
-  // u0 = v A0^T, q1 = u0 * c0
-  wide_lin_kernel<<<gH, kThreads, 0, st>>>(v, ws + L.A0T, nullptr, B, d, H, 1, h0, u0, q1);
-  WIDE_CHECK();
-  // w1 = q1 P0^T + v A1^T -> dP1 (column partials) -> dW1
-  wide_hid_kernel<<<gH, kThreads, 0, st>>>(q1, XF_ID, ws + L.P0T, v, ws + L.A1T, nullptr, ws + L.P1, B, d, H, 1,
-                                          const_cast<uint8_t*>(mask1), s2, nullptr, ws + L.colpart);
-  WIDE_CHECK();
-  if (g && g->W1) {
-    wide_col_finalize_kernel<<<(H + 255) / 256, 256, 0, st>>>(ws + L.colpart, L.mt, H, chain, ws + L.P1, p->W1, g->W1);
+                          g ? g->A0b : nullptr, ws, L, precision, st);
+    if (rc) return rc;
+  } else {
+    rc = wide_prepare(p, d, H, weight_mode, ws, L, st);
+    if (rc) return rc;
+    // u0 = v A0^T, q1 = u0 * c0
+    wide_lin_kernel<<<gH, kThreads, 0, st>>>(v, ws + L.A0T, nullptr, B, d, H, 1, h0, u0, q1);
     WIDE_CHECK();
-  }
-  // gx1 -> g0, t0, db0 partials
-  wide_gx1_kernel<<<gH, kThreads, 0, st>>>(mask1, s2, ws + L.P1, ws + L.P0, h0, u0, B, H, g0, t0, ws + L.colpart);
-  WIDE_CHECK();
-  if (g && g->A0b) {
-    wide_col_finalize_kernel<<<(H + 255) / 256, 256, 0, st>>>(ws + L.colpart, L.mt, H, 0, nullptr, nullptr, g->A0b);
+    // w1 = q1 P0^T + v A1^T -> dP1 (column partials) -> dW1
+    wide_hid_kernel<<<gH, kThreads, 0, st>>>(q1, XF_ID, ws + L.P0T, v, ws + L.A1T, nullptr, ws + L.P1, B, d, H, 1,
+                                            const_cast<uint8_t*>(mask1), s2, nullptr, ws + L.colpart);
     WIDE_CHECK();
-  }
-  if (dz) {
-    // dz [B,nz]: only the gradient w.r.t. the real (unpadded) input columns is formed
-    wide_out_kernel<<<dim3(L.mt, (nz + 127) / 128), kThreads, 0, st>>>(t0, p->A0w, 0, nullptr, nullptr, nullptr, nullptr, nullptr, v,
-                                                                      d, nz, 2.f * kappa, B, d, nz, H, dz);
+    if (g && g->W1) {
+      rc = wide_col_finalize(ws + L.colpart, L.mt, H, chain, ws + L.P1, p->W1, g->W1, st);
+      if (rc) return rc;
+    }
+    // gx1 -> g0, t0, db0 partials
+    wide_gx1_kernel<<<gH, kThreads, 0, st>>>(mask1, s2, ws + L.P1, ws + L.P0, h0, u0, B, H, g0, t0, ws + L.colpart);
     WIDE_CHECK();
+    if (g && g->A0b) {
+      rc = wide_col_finalize(ws + L.colpart, L.mt, H, 0, nullptr, nullptr, g->A0b, st);
+      if (rc) return rc;
+    }
+    if (dz) {
+      // dz [B,nz]: only the gradient w.r.t. the real (unpadded) input columns is formed
+      wide_out_kernel<<<dim3(L.mt, (nz + 127) / 128), kThreads, 0, st>>>(t0, p->A0w, 0, nullptr, nullptr, nullptr, nullptr,
+                                                                        nullptr, v, d, nz, 2.f * kappa, B, d, nz, H, dz);
+      WIDE_CHECK();
+    }
   }
-  }   // !rows_done
-  if (g) {
-    if (g->A2w) {
-      wide_a2_kernel<<<L.mt, 256, 0, st>>>(v, s2, B, d, ws + L.colpart);
-      WIDE_CHECK();
-      wide_col_finalize_kernel<<<(d + 255) / 256, 256, 0, st>>>(ws + L.colpart, L.mt, d, 0, nullptr, nullptr, g->A2w);
-      WIDE_CHECK();
-    }
-    if (g->A1b) { wide_zero_kernel<<<(H + 255) / 256, 256, 0, st>>>(g->A1b, H); WIDE_CHECK(); }   // sigma'' = 0: exact zeros
-    if (g->A2b) { wide_zero_kernel<<<1, 32, 0, st>>>(g->A2b, 1); WIDE_CHECK(); }
-    bool tn_done = false;
-    if (rows_done) {                 // batch-reduction GEMMs on tcgen05 as well (transposed operands, split-K slabs)
-      rc = wide_tc_bwd_tn(z, v, mask1, s2, q1, g0, t0, B, d, nz, H, p, weight_mode, ws + L.P1, g->A0w, g->A1w, g->W0,
-                          ws + L.end + wide_tc_ws_floats(B, d, H), precision, st);
-      if (rc == B200VAE_OK) tn_done = true;
-      else if (rc != B200VAE_EUNSUP) return rc;
-    }
-    if (tn_done) return B200VAE_OK;
-    TnArgs t;
-    t.N1 = 0;
-    t.mask1 = mask1; t.s2 = s2; t.P1 = ws + L.P1; t.B = B; t.Mdim = H;
-    const int splits = L.splits;
-    t.rows_per_split = round_up((B + splits - 1) / splits, kBK);
-    const int fin_blocks = 148 * 4;
-    if (g->A0w) {   // dA0 = g0^T v + t0^T z
-      t.a1 = g0; t.xf1 = XF_ID; t.b1 = v; t.a2 = t0; t.b2 = z; t.N2 = nz; t.N = d;
-      wide_tn_kernel<<<dim3(L.nt, (d + 127) / 128, splits), kThreads, 0, st>>>(t, ws + L.slabs);
-      WIDE_CHECK();
-      wide_slab_finalize_kernel<<<fin_blocks, 256, 0, st>>>(ws + L.slabs, splits, (size_t)H * d, 0, nullptr, nullptr, g->A0w);
-      WIDE_CHECK();
-    }
-    if (g->A1w) {   // dA1 = g1^T v
-      t.a1 = nullptr; t.xf1 = XF_G1; t.b1 = v; t.a2 = nullptr; t.b2 = nullptr; t.N2 = 0; t.N = d;
-      wide_tn_kernel<<<dim3(L.nt, (d + 127) / 128, splits), kThreads, 0, st>>>(t, ws + L.slabs);
-      WIDE_CHECK();
-      wide_slab_finalize_kernel<<<fin_blocks, 256, 0, st>>>(ws + L.slabs, splits, (size_t)H * d, 0, nullptr, nullptr, g->A1w);
-      WIDE_CHECK();
-    }
-    if (g->W0) {    // dP0 = g1^T q1 -> dW0
-      t.a1 = nullptr; t.xf1 = XF_G1; t.b1 = q1; t.a2 = nullptr; t.b2 = nullptr; t.N2 = 0; t.N = H;
-      wide_tn_kernel<<<dim3(L.nt, L.nt, splits), kThreads, 0, st>>>(t, ws + L.slabs);
-      WIDE_CHECK();
-      wide_slab_finalize_kernel<<<fin_blocks, 256, 0, st>>>(ws + L.slabs, splits, (size_t)H * H, chain, ws + L.P0, p->W0, g->W0);
-      WIDE_CHECK();
-    }
+  if (!g) return B200VAE_OK;
+  if (g->A2w) {
+    wide_a2_kernel<<<L.mt, 256, 0, st>>>(v, s2, B, d, ws + L.colpart);
+    WIDE_CHECK();
+    rc = wide_col_finalize(ws + L.colpart, L.mt, d, 0, nullptr, nullptr, g->A2w, st);
+    if (rc) return rc;
+  }
+  if (g->A1b) { wide_zero_kernel<<<(H + 255) / 256, 256, 0, st>>>(g->A1b, H); WIDE_CHECK(); }   // sigma'' = 0: exact zeros
+  if (g->A2b) { wide_zero_kernel<<<1, 32, 0, st>>>(g->A2b, 1); WIDE_CHECK(); }
+  if (tc)
+    return wide_tc_bwd_tn(z, v, mask1, s2, q1, g0, t0, B, d, nz, H, p, weight_mode, g->A0w, g->A1w, g->W0, ws, L, precision, st);
+  TnArgs t;
+  t.N1 = 0;
+  t.mask1 = mask1; t.s2 = s2; t.P1 = ws + L.P1; t.B = B; t.Mdim = H;
+  t.rows_per_split = round_up((B + L.splits - 1) / L.splits, kBK);
+  if (g->A0w) {   // dA0 = g0^T v + t0^T z
+    t.a1 = g0; t.xf1 = XF_ID; t.b1 = v; t.a2 = t0; t.b2 = z; t.N2 = nz; t.N = d;
+    wide_tn_kernel<<<dim3(L.nt, (d + 127) / 128, L.splits), kThreads, 0, st>>>(t, ws + L.slabs);
+    WIDE_CHECK();
+    rc = wide_slab_finalize(ws + L.slabs, L.splits, (size_t)H * d, 0, nullptr, g->A0w, st);
+    if (rc) return rc;
+  }
+  if (g->A1w) {   // dA1 = g1^T v
+    t.a1 = nullptr; t.xf1 = XF_G1; t.b1 = v; t.a2 = nullptr; t.b2 = nullptr; t.N2 = 0; t.N = d;
+    wide_tn_kernel<<<dim3(L.nt, (d + 127) / 128, L.splits), kThreads, 0, st>>>(t, ws + L.slabs);
+    WIDE_CHECK();
+    rc = wide_slab_finalize(ws + L.slabs, L.splits, (size_t)H * d, 0, nullptr, g->A1w, st);
+    if (rc) return rc;
+  }
+  if (g->W0) {    // dP0 = g1^T q1 -> dW0
+    t.a1 = nullptr; t.xf1 = XF_G1; t.b1 = q1; t.a2 = nullptr; t.b2 = nullptr; t.N2 = 0; t.N = H;
+    wide_tn_kernel<<<dim3(L.nt, L.nt, L.splits), kThreads, 0, st>>>(t, ws + L.slabs);
+    WIDE_CHECK();
+    return wide_slab_finalize(ws + L.slabs, L.splits, (size_t)H * H, chain, p->W0, g->W0, st);
   }
   return B200VAE_OK;
 }
@@ -757,10 +767,11 @@ extern "C" int b200vae_icnn_wide_bwd_psi(const float* z, const float* gpsi, cons
                                          const float* s2, int B, int d, int nz, int H, const b200vae_icnn_params* p,
                                          int weight_mode, const b200vae_icnn_grads* g, float* dz, float* x1, float* g0,
                                          float* s2g, void* workspace, size_t ws_bytes, void* stream) {
+  int rc = wide_shape_ok(B, d, nz, H, B200VAE_PREC_FP32);
+  if (rc) return rc;
   if (!z || !gpsi || !h0 || !mask1 || !s2 || !wide_params_ok(p) || !x1 || !g0 || !s2g || !workspace) return B200VAE_EALIGN;
-  if (B <= 0 || d <= 0 || H <= 0 || nz <= 0 || nz > d) return B200VAE_ESHAPE;
   if (weight_mode != B200VAE_WEIGHT_EXP && weight_mode != B200VAE_WEIGHT_CLAMP) return B200VAE_EUNSUP;
-  const WideWs L = wide_layout(B, d, H, true);
+  const WideLayout L = wide_ws_layout(B, d, H, false, true);
   if (ws_bytes < b200vae_icnn_wide_workspace_bytes(B, d, H, B200VAE_PREC_FP32, 1)) return B200VAE_EWS;
   if (!aligned16(workspace) || !aligned16(z) || !aligned16(h0) || !aligned16(x1) || !aligned16(g0) || !aligned4(p->A0w) ||
       !aligned4(p->A1w) || (dz && !aligned16(dz)))
@@ -768,7 +779,7 @@ extern "C" int b200vae_icnn_wide_bwd_psi(const float* z, const float* gpsi, cons
   cudaStream_t st = (cudaStream_t)stream;
   float* ws = (float*)workspace;
   const int chain = weight_mode == B200VAE_WEIGHT_EXP ? 1 : 2;
-  int rc = wide_prepare(p, d, H, weight_mode, ws, L, st);
+  rc = wide_prepare(p, d, H, weight_mode, ws, L, st);
   if (rc) return rc;
   const dim3 gH(L.mt, L.nt);
   wide_psi_pre_kernel<<<148 * 4, 256, 0, st>>>(gpsi, s2, h0, B, (size_t)B * H, s2g, x1);
@@ -778,15 +789,15 @@ extern "C" int b200vae_icnn_wide_bwd_psi(const float* z, const float* gpsi, cons
     wide_hid_kernel<<<gH, kThreads, 0, st>>>(h0, XF_X1, ws + L.P0T, z, ws + L.A1T, p->A1b, ws + L.P1, B, nz, H, 2, nullptr, s2g,
                                             nullptr, ws + L.colpart);
     WIDE_CHECK();
-    wide_col_finalize_kernel<<<(H + 255) / 256, 256, 0, st>>>(ws + L.colpart, L.mt, H, chain, ws + L.P1, p->W1, g->W1);
-    WIDE_CHECK();
+    rc = wide_col_finalize(ws + L.colpart, L.mt, H, chain, ws + L.P1, p->W1, g->W1, st);
+    if (rc) return rc;
   }
   // delta0 = (delta1 P0) * 2 a0 s0 -> g0 buffer, column sums = db0
   wide_gx1_kernel<<<gH, kThreads, 0, st>>>(mask1, s2g, ws + L.P1, ws + L.P0, h0, nullptr, B, H, g0, nullptr, ws + L.colpart);
   WIDE_CHECK();
   if (g && g->A0b) {
-    wide_col_finalize_kernel<<<(H + 255) / 256, 256, 0, st>>>(ws + L.colpart, L.mt, H, 0, nullptr, nullptr, g->A0b);
-    WIDE_CHECK();
+    rc = wide_col_finalize(ws + L.colpart, L.mt, H, 0, nullptr, nullptr, g->A0b, st);
+    if (rc) return rc;
   }
   if (dz) {
     wide_out_kernel<<<dim3(L.mt, (nz + 127) / 128), kThreads, 0, st>>>(g0, p->A0w, 1, mask1, s2g, ws + L.P1, p->A1w, p->A2w, nullptr,
@@ -797,14 +808,14 @@ extern "C" int b200vae_icnn_wide_bwd_psi(const float* z, const float* gpsi, cons
   if (g->A1b) {       // db1[c] = P1[c] * sum_b delta2[b] sigma'(h1[b][c])
     wide_maskcol_kernel<<<dim3(L.mt, (H + 255) / 256), 256, 0, st>>>(mask1, s2g, B, H, ws + L.colpart);
     WIDE_CHECK();
-    wide_col_finalize_kernel<<<(H + 255) / 256, 256, 0, st>>>(ws + L.colpart, L.mt, H, 1, ws + L.P1, nullptr, g->A1b);
-    WIDE_CHECK();
+    rc = wide_col_finalize(ws + L.colpart, L.mt, H, 1, ws + L.P1, nullptr, g->A1b, st);
+    if (rc) return rc;
   }
   if (g->A2w) {       // dA2[c] = sum_b delta2[b] z[b][c] for c < nz, 0 beyond (the padded inputs are zero)
     wide_a2_kernel<<<L.mt, 256, 0, st>>>(z, s2g, B, nz, ws + L.colpart);
     WIDE_CHECK();
-    wide_col_finalize_kernel<<<(nz + 255) / 256, 256, 0, st>>>(ws + L.colpart, L.mt, nz, 0, nullptr, nullptr, g->A2w);
-    WIDE_CHECK();
+    rc = wide_col_finalize(ws + L.colpart, L.mt, nz, 0, nullptr, nullptr, g->A2w, st);
+    if (rc) return rc;
     if (d > nz) { wide_zero_kernel<<<(d - nz + 255) / 256, 256, 0, st>>>(g->A2w + nz, d - nz); WIDE_CHECK(); }
   }
   if (g->A2b) { wide_sum_kernel<<<1, 256, 0, st>>>(s2g, B, g->A2b); WIDE_CHECK(); }
@@ -812,27 +823,25 @@ extern "C" int b200vae_icnn_wide_bwd_psi(const float* z, const float* gpsi, cons
   t.mask1 = mask1; t.s2 = s2g; t.P1 = ws + L.P1; t.B = B; t.Mdim = H; t.a2 = nullptr; t.b2 = nullptr; t.N2 = 0;
   const int splits = L.splits;
   t.rows_per_split = round_up((B + splits - 1) / splits, kBK);
-  const int fin_blocks = 148 * 4;
   if (g->A0w) {       // dA0 = delta0^T z   ([H, nz] block of [H, d])
     t.a1 = g0; t.xf1 = XF_ID; t.b1 = z; t.N = nz; t.N1 = nz;
     wide_tn_kernel<<<dim3(L.nt, (nz + 127) / 128, splits), kThreads, 0, st>>>(t, ws + L.slabs);
     WIDE_CHECK();
-    wide_slab_finalize_ld_kernel<<<fin_blocks, 256, 0, st>>>(ws + L.slabs, splits, H, nz, d, g->A0w);
+    wide_slab_finalize_ld_kernel<<<148 * 4, 256, 0, st>>>(ws + L.slabs, splits, H, nz, d, g->A0w);
     WIDE_CHECK();
   }
   if (g->A1w) {       // dA1 = delta1^T z
     t.a1 = nullptr; t.xf1 = XF_G1; t.b1 = z; t.N = nz; t.N1 = nz;
     wide_tn_kernel<<<dim3(L.nt, (nz + 127) / 128, splits), kThreads, 0, st>>>(t, ws + L.slabs);
     WIDE_CHECK();
-    wide_slab_finalize_ld_kernel<<<fin_blocks, 256, 0, st>>>(ws + L.slabs, splits, H, nz, d, g->A1w);
+    wide_slab_finalize_ld_kernel<<<148 * 4, 256, 0, st>>>(ws + L.slabs, splits, H, nz, d, g->A1w);
     WIDE_CHECK();
   }
   if (g->W0) {        // dP0 = delta1^T x1 -> dW0
     t.a1 = nullptr; t.xf1 = XF_G1; t.b1 = x1; t.N = H; t.N1 = H;
     wide_tn_kernel<<<dim3(L.nt, L.nt, splits), kThreads, 0, st>>>(t, ws + L.slabs);
     WIDE_CHECK();
-    wide_slab_finalize_kernel<<<fin_blocks, 256, 0, st>>>(ws + L.slabs, splits, (size_t)H * H, chain, ws + L.P0, p->W0, g->W0);
-    WIDE_CHECK();
+    return wide_slab_finalize(ws + L.slabs, splits, (size_t)H * H, chain, p->W0, g->W0, st);
   }
   return B200VAE_OK;
 }

@@ -1,8 +1,12 @@
-// icnn_wide_tc.cu -- tcgen05 FORWARD (decode: psi + Brenier map) for wide-input ICNNs (d > 4): the MNIST-shaped decoder
-// ICNN(32,512) + ICNN(784,1024) of BASELINE configs[3] (model.py:766-805, module.py:142-148, model.py:820-828).
+// icnn_wide_tc.cu -- tcgen05 forward (decode: psi + Brenier map) AND backward (dL/dxhat) for wide-input ICNNs (d > 4): the
+// MNIST-shaped decoder ICNN(32,512) + ICNN(784,1024) of BASELINE configs[3] (model.py:766-805, module.py:142-148,
+// model.py:820-828).  b200vae_icnn_wide_fwd / _bwd (icnn_wide.cu) call these drivers at TF32 / TF32X3 (and F16X3, which
+// runs as TF32X3) when wide_tc_supported holds -- and, for the forward, b0, b1, A2 are 16-byte aligned; the psi-gradient
+// backward always runs on the FP32 kernels.
 //
-// For wide inputs every product of the sweep is a dense contraction, so the forward is four launches of ONE generic
-// tensor-core GEMM kernel  C[M,N] = xf(A1)[M,K1] . B1[N,K1]^T (+ A2[M,K2] . B2[N,K2]^T)  with different epilogues:
+// For wide inputs every product of the sweep is a dense contraction, so every GEMM of both directions is a launch of ONE
+// generic tensor-core GEMM kernel  C[M,N] = xf(A1)[M,K1] . B1[N,K1]^T (+ A2[M,K2] . B2[N,K2]^T)  with different epilogues.
+// The forward:
 //   lin : h0 = z A0^T + b0                                   (store h0)
 //   hid : h1 = sigma(h0)^2 P0^T + z A1^T + b1 -> byte mask, g1b = P1*sigma'(h1) (fp32), row partials of P1.sigma(h1)
 //   row : h2 = sum partials + A2 z + b2 -> psi, s2            (small SIMT kernel)
@@ -14,10 +18,12 @@
 // pass) and split it into tf32 hi / lo; warp 9 issues tcgen05.mma.kind::tf32 (3 MMAs per product at 3xTF32, B hi/lo
 // prepared once per forward); the accumulator (128 lanes x 256 columns of TMEM) is drained by warps 0-7 with
 // tcgen05.ld.32x32b: one thread = one sample row x 128 columns, so row partials need no shuffles and stores are
-// row-contiguous.  The saved activations (h0, byte mask, s2) have the SIMT layout: the FP32 backward (icnn_wide.cu)
-// runs unchanged on them.
+// row-contiguous.  The saved activations (h0, byte mask, s2) have the FP32 path's format, so either backward runs on them.
+// The backward runs the sample-stationary GEMMs (u0, w1, gx1, dz) with fused epilogues, then transposes its operands so
+// that the batch becomes K and runs the batch-reduction GEMMs (dA0, dA1, dP0) split over K into ordered slabs.
 #include <string.h>
 
+#include "icnn_wide.cuh"
 #include "tc_common.cuh"
 
 namespace b200vae {
@@ -332,31 +338,13 @@ wide_tc_gemm_kernel(const __grid_constant__ WtArgs a) {
 }
 
 // ---- prepare: positive weights and all operand copies, split into tf32 hi / lo ------------------------------------------------
-struct WtLayout {
-  size_t P0hi, P0lo, P0Thi, P0Tlo, A0hi, A0lo, A1hi, A1lo, A0Thi, A0Tlo, A1Thi, A1Tlo, P1, g1b, part, end;
-  int mt, nt;
-};
-static inline size_t wt_up(size_t x) { return (x + 63) / 64 * 64; }
-static WtLayout wt_layout(int B, int d, int H) {
-  WtLayout L;
-  size_t o = 0;
-  const size_t HH = wt_up((size_t)H * H), dH = wt_up((size_t)d * H);
-  L.mt = (B + 127) / 128; L.nt = (H + 127) / 128;        // row partials: two per 128-column (3xTF32) / 256-column tile
-  L.P0hi = o; o += HH; L.P0lo = o; o += HH; L.P0Thi = o; o += HH; L.P0Tlo = o; o += HH;
-  L.A0hi = o; o += dH; L.A0lo = o; o += dH; L.A1hi = o; o += dH; L.A1lo = o; o += dH;
-  L.A0Thi = o; o += dH; L.A0Tlo = o; o += dH; L.A1Thi = o; o += dH; L.A1Tlo = o; o += dH;
-  L.P1 = o; o += wt_up(H);
-  L.g1b = o; o += wt_up((size_t)B * H);
-  L.part = o; o += wt_up((size_t)B * L.nt * 2);
-  L.end = o;
-  return L;
-}
 __device__ __forceinline__ void split_store(float x, float* hi, float* lo, size_t i) {
   const float h = rn_tf32_masked(x);
   hi[i] = h; lo[i] = rn_tf32_masked(x - h);
 }
 __global__ void wide_tc_prepare_kernel(const float* __restrict__ W0, const float* __restrict__ W1, const float* __restrict__ A0w,
-                                       const float* __restrict__ A1w, int d, int H, int mode, float* __restrict__ ws, WtLayout L) {
+                                       const float* __restrict__ A1w, int d, int H, int mode, float* __restrict__ ws,
+                                       WideLayout L) {
   const size_t HH = (size_t)H * H, dH = (size_t)d * H, tot = HH + H + dH, gstride = (size_t)gridDim.x * blockDim.x;
   for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < tot; i += gstride) {
     if (i < HH) {
@@ -377,24 +365,6 @@ __global__ void wide_tc_prepare_kernel(const float* __restrict__ W0, const float
     }
   }
 }
-// h2 = sum_t part[row][t] + A2.z + b2 -> psi, s2   (z is [B, nz])
-__global__ void __launch_bounds__(256)
-wide_tc_row_kernel(const float* __restrict__ part, int npart, const float* __restrict__ z, const float* __restrict__ A2w,
-                   const float* __restrict__ A2b, int B, int nz, float* __restrict__ psi, float* __restrict__ s2) {
-  const int lane = threadIdx.x & 31, row = blockIdx.x * 8 + (threadIdx.x >> 5);
-  if (row >= B) return;
-  float s = 0.f;
-  for (int c = lane; c < nz; c += 32) s = fmaf(__ldg(A2w + c), z[(size_t)row * nz + c], s);
-  s = warp_sum(s);
-  if (lane == 0) {
-    float h2 = s + A2b[0];
-    for (int t = 0; t < npart; ++t) h2 += part[(size_t)row * npart + t];
-    const float sl = h2 > 0.f ? 1.f : kSlope;
-    if (psi) psi[row] = h2 * sl;
-    s2[row] = sl;
-  }
-}
-
 // g1b[b][n] = P1[n] * sigma'(h1[b][n]) from the saved byte mask (A operand of the backward's gx1 GEMM)
 __global__ void wide_tc_g1b_kernel(const uint8_t* __restrict__ mask, const float* __restrict__ P1, size_t n, int H,
                                    float* __restrict__ g1b) {
@@ -402,7 +372,7 @@ __global__ void wide_tc_g1b_kernel(const uint8_t* __restrict__ mask, const float
   for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gstride)
     g1b[i] = P1[i % H] * (mask[i] ? 1.f : kSlope);
 }
-// ordered column sums of a [B][H] matrix: colpart[mt][H] over 128-row blocks, then a fixed-order finalize (+ chain)
+// ordered column sums of a [B][H] matrix: colpart[mt][H] over 128-row blocks (wide_col_finalize adds them in fixed order)
 __global__ void __launch_bounds__(256)
 wide_tc_colsum_kernel(const float* __restrict__ x, int B, int H, float* __restrict__ colpart) {
   const int c = blockIdx.y * 256 + threadIdx.x, r0 = blockIdx.x * 128, r1 = min(B, r0 + 128);
@@ -410,16 +380,6 @@ wide_tc_colsum_kernel(const float* __restrict__ x, int B, int H, float* __restri
   float s = 0.f;
   for (int r = r0; r < r1; ++r) s += x[(size_t)r * H + c];
   colpart[(size_t)blockIdx.x * H + c] = s;
-}
-__global__ void wide_tc_colfin_kernel(const float* __restrict__ colpart, int mt, int H, int chain, const float* __restrict__ P,
-                                      const float* __restrict__ W, float* __restrict__ out) {
-  const int c = blockIdx.x * blockDim.x + threadIdx.x;
-  if (c >= H) return;
-  float s = 0.f;
-  for (int t = 0; t < mt; ++t) s += colpart[(size_t)t * H + c];
-  if (chain == 1) s *= P[c];
-  else if (chain == 2) s = W[c] >= kClampMin ? s : 0.f;
-  out[c] = s;
 }
 
 // Transpose [B][C] -> [C][ldo] (ldo >= B) so that the BATCH index becomes the contiguous K dimension of the batch-reduction
@@ -452,44 +412,7 @@ wide_tc_transpose_kernel(const float* __restrict__ src, const uint8_t* __restric
     }
   }
 }
-// out[i] = chain( sum_s slabs[s][i] ):  chain 0 none, 1 * exp(W) (dW = dP * P), 2 * [W >= 1e-2]
-__global__ void wide_tc_slabfin_kernel(const float* __restrict__ slabs, int splits, size_t n, int chain, const float* __restrict__ W,
-                                       float* __restrict__ out) {
-  const size_t gstride = (size_t)gridDim.x * blockDim.x;
-  for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gstride) {
-    float s = 0.f;
-    for (int k = 0; k < splits; ++k) s += slabs[(size_t)k * n + i];
-    if (chain == 1) s *= expf(W[i]);
-    else if (chain == 2) s = W[i] >= kClampMin ? s : 0.f;
-    out[i] = s;
-  }
-}
-
 // ---- host side ---------------------------------------------------------------------------------------------------------------
-typedef CUresult (*EncodeTiledFnW)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                   const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
-                                   CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-// 2-D fp32 tensor [rows][K] (row stride ld floats), boxes of 16 x box_rows, 64-byte swizzle, zero fill outside
-static int wt_map(CUtensorMap* m, const float* base, int K, int rows, int ld, int box_rows) {
-  static EncodeTiledFnW fn = nullptr;
-  if (!fn) {
-    void* p = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess && p)
-      fn = reinterpret_cast<EncodeTiledFnW>(p);
-  }
-  if (!fn) return B200VAE_ECUDA;
-  const cuuint64_t dims[2] = {(cuuint64_t)K, (cuuint64_t)rows};
-  const cuuint64_t strides[1] = {(cuuint64_t)ld * sizeof(float)};
-  const cuuint32_t box[2] = {(cuuint32_t)kKB, (cuuint32_t)box_rows};
-  const cuuint32_t estr[2] = {1, 1};
-  CUresult r = fn(m, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, const_cast<float*>(base), dims, strides, box, estr,
-                  CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                  CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) { g_last_cuda_error = 100000 + (int)r; return B200VAE_ECUDA; }
-  return B200VAE_OK;
-}
-
 template <bool X3, int S>
 static int wt_launch_s(const WtArgs& args, dim3 grid, cudaStream_t st) {
   static bool attr_done = false;
@@ -512,18 +435,11 @@ static int wt_run(const WtArgs& args, bool x3, cudaStream_t st, int splits = 1) 
   return x3 ? wt_launch<true>(args, splits, st) : wt_launch<false>(args, splits, st);
 }
 
-size_t wide_tc_ws_floats(int B, int d, int H) { return wt_layout(B, d, H).end; }
-bool wide_tc_supported(int d, int nz, int H, int precision) {
-  return (precision == B200VAE_PREC_TF32 || precision == B200VAE_PREC_TF32X3) && d % 4 == 0 && nz % 4 == 0 && H % 4 == 0;
-}
-
-// same contract as b200vae_icnn_wide_fwd (h0, mask1, s2 saved for the FP32 backward); g0 is [B,H] scratch
 int wide_tc_fwd(const float* z, int B, int d, int nz, int H, const b200vae_icnn_params* p, int mode, float kappa, float* psi,
-                float* xhat, float* h0, uint8_t* mask1, float* s2, float* g0, float* ws, int precision, cudaStream_t st) {
-  if (!wide_tc_supported(d, nz, H, precision)) return B200VAE_EUNSUP;
+                float* xhat, float* h0, uint8_t* mask1, float* s2, float* g0, float* ws, const WideLayout& L, int precision,
+                cudaStream_t st) {
   const bool x3 = precision == B200VAE_PREC_TF32X3;
   const int bn = wt_tile_n(x3);                         // rows of a B-operand TMA box = the kernel's tile width
-  const WtLayout L = wt_layout(B, d, H);
   wide_tc_prepare_kernel<<<148 * 4, 256, 0, st>>>(p->W0, p->W1, p->A0w, p->A1w, d, H, mode, ws, L);
   int rc = check_launch();
   if (rc) return rc;
@@ -532,9 +448,9 @@ int wide_tc_fwd(const float* z, int B, int d, int nz, int H, const b200vae_icnn_
   WtArgs a;
   memset(&a, 0, sizeof(a));
   // ---- lin: h0 = z A0^T + b0   (A0w is [H][d]; only its first nz columns meet non-zero inputs)
-  rc = wt_map(&a.a1, z, nz, B, nz, 128);
-  if (!rc) rc = wt_map(&a.b1hi, ws + L.A0hi, nz, H, d, wt_tile_n(true));
-  if (!rc) rc = wt_map(&a.b1lo, ws + L.A0lo, nz, H, d, wt_tile_n(true));
+  rc = tma_map_2d(&a.a1, z, nz, B, nz, 128);
+  if (!rc) rc = tma_map_2d(&a.b1hi, ws + L.A0hi, nz, H, d, wt_tile_n(true));
+  if (!rc) rc = tma_map_2d(&a.b1lo, ws + L.A0lo, nz, H, d, wt_tile_n(true));
   if (rc) return rc;
   a.a2 = a.a1; a.b2hi = a.b1hi; a.b2lo = a.b1lo;
   a.nkb1 = nkb(nz); a.nkb2 = 0; a.xf1 = WT_XF_ID; a.M = B; a.N = H; a.epi = WT_EPI_LIN; a.bias = p->A0b; a.out0 = h0;
@@ -543,26 +459,25 @@ int wide_tc_fwd(const float* z, int B, int d, int nz, int H, const b200vae_icnn_
   // ---- hid: h1 = x1 P0^T + z A1^T + b1
   WtArgs b;
   memset(&b, 0, sizeof(b));
-  rc = wt_map(&b.a1, h0, H, B, H, 128);
-  if (!rc) rc = wt_map(&b.b1hi, ws + L.P0hi, H, H, H, bn);
-  if (!rc) rc = wt_map(&b.b1lo, ws + (x3 ? L.P0lo : L.P0hi), H, H, H, bn);
-  if (!rc) rc = wt_map(&b.b2hi, ws + L.A1hi, nz, H, d, bn);
-  if (!rc) rc = wt_map(&b.b2lo, ws + (x3 ? L.A1lo : L.A1hi), nz, H, d, bn);
+  rc = tma_map_2d(&b.a1, h0, H, B, H, 128);
+  if (!rc) rc = tma_map_2d(&b.b1hi, ws + L.P0hi, H, H, H, bn);
+  if (!rc) rc = tma_map_2d(&b.b1lo, ws + (x3 ? L.P0lo : L.P0hi), H, H, H, bn);
+  if (!rc) rc = tma_map_2d(&b.b2hi, ws + L.A1hi, nz, H, d, bn);
+  if (!rc) rc = tma_map_2d(&b.b2lo, ws + (x3 ? L.A1lo : L.A1hi), nz, H, d, bn);
   if (rc) return rc;
   b.a2 = a.a1;
   b.nkb1 = nkb(H); b.nkb2 = nkb(nz); b.xf1 = WT_XF_X1; b.M = B; b.N = H; b.epi = WT_EPI_HID; b.bias = p->A1b; b.P1 = ws + L.P1;
   b.out0 = ws + L.g1b; b.mask = mask1; b.part = ws + L.part; b.npart = ((H + bn - 1) / bn) * 2;
   rc = wt_run(b, x3, st);
   if (rc) return rc;
-  wide_tc_row_kernel<<<(B + 7) / 8, 256, 0, st>>>(ws + L.part, b.npart, z, p->A2w, p->A2b, B, nz, psi, s2);
-  rc = check_launch();
+  rc = wide_row(ws + L.part, b.npart, z, p, B, nz, psi, s2, st);
   if (rc || !xhat) return rc;
   // ---- gx1: g0' = (g1b P0) * c0(h0)      B^T[k'][n] = P0[n][k'] = P0T
   WtArgs c;
   memset(&c, 0, sizeof(c));
-  rc = wt_map(&c.a1, ws + L.g1b, H, B, H, 128);
-  if (!rc) rc = wt_map(&c.b1hi, ws + L.P0Thi, H, H, H, bn);
-  if (!rc) rc = wt_map(&c.b1lo, ws + (x3 ? L.P0Tlo : L.P0Thi), H, H, H, bn);
+  rc = tma_map_2d(&c.a1, ws + L.g1b, H, B, H, 128);
+  if (!rc) rc = tma_map_2d(&c.b1hi, ws + L.P0Thi, H, H, H, bn);
+  if (!rc) rc = tma_map_2d(&c.b1lo, ws + (x3 ? L.P0Tlo : L.P0Thi), H, H, H, bn);
   if (rc) return rc;
   c.a2 = c.a1; c.b2hi = c.b1hi; c.b2lo = c.b1lo;
   c.nkb1 = nkb(H); c.nkb2 = 0; c.xf1 = WT_XF_ID; c.M = B; c.N = H; c.epi = WT_EPI_GX1; c.h0 = h0; c.out0 = g0;
@@ -571,11 +486,11 @@ int wide_tc_fwd(const float* z, int B, int d, int nz, int H, const b200vae_icnn_
   // ---- out: xhat = s2 (g0' A0 + g1b A1 + A2) + 2 kappa z      B^T[c][n] = A*w[n][c] = A*wT  ([d][H])
   WtArgs e;
   memset(&e, 0, sizeof(e));
-  rc = wt_map(&e.a1, g0, H, B, H, 128);
-  if (!rc) rc = wt_map(&e.b1hi, ws + L.A0Thi, H, d, H, bn);
-  if (!rc) rc = wt_map(&e.b1lo, ws + (x3 ? L.A0Tlo : L.A0Thi), H, d, H, bn);
-  if (!rc) rc = wt_map(&e.b2hi, ws + L.A1Thi, H, d, H, bn);
-  if (!rc) rc = wt_map(&e.b2lo, ws + (x3 ? L.A1Tlo : L.A1Thi), H, d, H, bn);
+  rc = tma_map_2d(&e.a1, g0, H, B, H, 128);
+  if (!rc) rc = tma_map_2d(&e.b1hi, ws + L.A0Thi, H, d, H, bn);
+  if (!rc) rc = tma_map_2d(&e.b1lo, ws + (x3 ? L.A0Tlo : L.A0Thi), H, d, H, bn);
+  if (!rc) rc = tma_map_2d(&e.b2hi, ws + L.A1Thi, H, d, H, bn);
+  if (!rc) rc = tma_map_2d(&e.b2lo, ws + (x3 ? L.A1Tlo : L.A1Thi), H, d, H, bn);
   if (rc) return rc;
   e.a2 = c.a1;
   e.nkb1 = nkb(H); e.nkb2 = nkb(H); e.xf1 = WT_XF_ID; e.M = B; e.N = d; e.epi = WT_EPI_OUT; e.s2 = s2; e.A2w = p->A2w; e.z = z;
@@ -583,16 +498,13 @@ int wide_tc_fwd(const float* z, int B, int d, int nz, int H, const b200vae_icnn_
   return wt_run(e, x3, st);
 }
 
-// Sample-stationary part of the backward on tcgen05 (SURVEY Appendix A): u0, q1 -> w1 -> dP1;  gx1 -> g0, t0 -> db0;  dz.
-// Leaves u0, q1, g0, t0 [B,H] filled for the batch-reduction GEMMs (dA0, dA1, dP0: FP32 kernels of icnn_wide.cu).
-// `colpart`: [ceil(B/128)][H] floats of scratch.  dW1 / db0 may be null.
+// Sample-stationary part of the backward (SURVEY Appendix A): u0, q1 -> w1 -> dP1;  gx1 -> g0, t0 -> db0;  dz.
+// Leaves u0, q1, g0, t0 [B,H] filled for wide_tc_bwd_tn.  dW1 / db0 / dz may be null.
 int wide_tc_bwd_rows(const float* v, const float* h0, const uint8_t* mask1, const float* s2, int B, int d, int nz, int H,
                      const b200vae_icnn_params* p, int mode, float kappa, float* dz, float* u0, float* q1, float* g0, float* t0,
-                     float* dW1, float* db0, float* ws, float* colpart, int precision, cudaStream_t st) {
-  if (!wide_tc_supported(d, nz, H, precision)) return B200VAE_EUNSUP;
+                     float* dW1, float* db0, float* ws, const WideLayout& L, int precision, cudaStream_t st) {
   const bool x3 = precision == B200VAE_PREC_TF32X3;
   const int bn = wt_tile_n(x3);                         // rows of a B-operand TMA box = the kernel's tile width
-  const WtLayout L = wt_layout(B, d, H);
   wide_tc_prepare_kernel<<<148 * 4, 256, 0, st>>>(p->W0, p->W1, p->A0w, p->A1w, d, H, mode, ws, L);
   int rc = check_launch();
   if (rc) return rc;
@@ -600,15 +512,14 @@ int wide_tc_bwd_rows(const float* v, const float* h0, const uint8_t* mask1, cons
   rc = check_launch();
   if (rc) return rc;
   auto nkb = [&](int K) { return (K + kKB - 1) / kKB; };
-  const int mt = (B + 127) / 128;
-  const dim3 cgrid(mt, (H + 255) / 256);
+  const dim3 cgrid(L.mt, (H + 255) / 256);
   const int chain = mode == B200VAE_WEIGHT_EXP ? 1 : 2;
   // ---- u0 = v A0^T, q1 = u0 * c0
   WtArgs a;
   memset(&a, 0, sizeof(a));
-  rc = wt_map(&a.a1, v, d, B, d, 128);
-  if (!rc) rc = wt_map(&a.b1hi, ws + L.A0hi, d, H, d, bn);
-  if (!rc) rc = wt_map(&a.b1lo, ws + (x3 ? L.A0lo : L.A0hi), d, H, d, bn);
+  rc = tma_map_2d(&a.a1, v, d, B, d, 128);
+  if (!rc) rc = tma_map_2d(&a.b1hi, ws + L.A0hi, d, H, d, bn);
+  if (!rc) rc = tma_map_2d(&a.b1lo, ws + (x3 ? L.A0lo : L.A0hi), d, H, d, bn);
   if (rc) return rc;
   a.a2 = a.a1; a.b2hi = a.b1hi; a.b2lo = a.b1lo;
   a.nkb1 = nkb(d); a.nkb2 = 0; a.xf1 = WT_XF_ID; a.M = B; a.N = H; a.epi = WT_EPI_U; a.h0 = h0; a.out0 = u0; a.out1 = q1;
@@ -617,11 +528,11 @@ int wide_tc_bwd_rows(const float* v, const float* h0, const uint8_t* mask1, cons
   // ---- e1 = s2 s1 (q1 P0^T + v A1^T)  -> column sums = dP1   (e1 parked in the g0 buffer)
   WtArgs b;
   memset(&b, 0, sizeof(b));
-  rc = wt_map(&b.a1, q1, H, B, H, 128);
-  if (!rc) rc = wt_map(&b.b1hi, ws + L.P0hi, H, H, H, bn);
-  if (!rc) rc = wt_map(&b.b1lo, ws + (x3 ? L.P0lo : L.P0hi), H, H, H, bn);
-  if (!rc) rc = wt_map(&b.b2hi, ws + L.A1hi, d, H, d, bn);
-  if (!rc) rc = wt_map(&b.b2lo, ws + (x3 ? L.A1lo : L.A1hi), d, H, d, bn);
+  rc = tma_map_2d(&b.a1, q1, H, B, H, 128);
+  if (!rc) rc = tma_map_2d(&b.b1hi, ws + L.P0hi, H, H, H, bn);
+  if (!rc) rc = tma_map_2d(&b.b1lo, ws + (x3 ? L.P0lo : L.P0hi), H, H, H, bn);
+  if (!rc) rc = tma_map_2d(&b.b2hi, ws + L.A1hi, d, H, d, bn);
+  if (!rc) rc = tma_map_2d(&b.b2lo, ws + (x3 ? L.A1lo : L.A1hi), d, H, d, bn);
   if (rc) return rc;
   b.a2 = a.a1;
   b.nkb1 = nkb(H); b.nkb2 = nkb(d); b.xf1 = WT_XF_ID; b.M = B; b.N = H; b.epi = WT_EPI_W1; b.s2 = s2;
@@ -629,19 +540,17 @@ int wide_tc_bwd_rows(const float* v, const float* h0, const uint8_t* mask1, cons
   rc = wt_run(b, x3, st);
   if (rc) return rc;
   if (dW1) {
-    wide_tc_colsum_kernel<<<cgrid, 256, 0, st>>>(g0, B, H, colpart);
+    wide_tc_colsum_kernel<<<cgrid, 256, 0, st>>>(g0, B, H, ws + L.colpart);
     rc = check_launch();
-    if (rc) return rc;
-    wide_tc_colfin_kernel<<<(H + 255) / 256, 256, 0, st>>>(colpart, mt, H, chain, ws + L.P1, p->W1, dW1);
-    rc = check_launch();
+    if (!rc) rc = wide_col_finalize(ws + L.colpart, L.mt, H, chain, ws + L.P1, p->W1, dW1, st);
     if (rc) return rc;
   }
   // ---- gx1 = s2 (g1b P0) -> g0, t0
   WtArgs c;
   memset(&c, 0, sizeof(c));
-  rc = wt_map(&c.a1, ws + L.g1b, H, B, H, 128);
-  if (!rc) rc = wt_map(&c.b1hi, ws + L.P0Thi, H, H, H, bn);
-  if (!rc) rc = wt_map(&c.b1lo, ws + (x3 ? L.P0Tlo : L.P0Thi), H, H, H, bn);
+  rc = tma_map_2d(&c.a1, ws + L.g1b, H, B, H, 128);
+  if (!rc) rc = tma_map_2d(&c.b1hi, ws + L.P0Thi, H, H, H, bn);
+  if (!rc) rc = tma_map_2d(&c.b1lo, ws + (x3 ? L.P0Tlo : L.P0Thi), H, H, H, bn);
   if (rc) return rc;
   c.a2 = c.a1; c.b2hi = c.b1hi; c.b2lo = c.b1lo;
   c.nkb1 = nkb(H); c.nkb2 = 0; c.xf1 = WT_XF_ID; c.M = B; c.N = H; c.epi = WT_EPI_GXB; c.h0 = h0; c.u0 = u0; c.s2 = s2;
@@ -649,20 +558,18 @@ int wide_tc_bwd_rows(const float* v, const float* h0, const uint8_t* mask1, cons
   rc = wt_run(c, x3, st);
   if (rc) return rc;
   if (db0) {
-    wide_tc_colsum_kernel<<<cgrid, 256, 0, st>>>(t0, B, H, colpart);
+    wide_tc_colsum_kernel<<<cgrid, 256, 0, st>>>(t0, B, H, ws + L.colpart);
     rc = check_launch();
-    if (rc) return rc;
-    wide_tc_colfin_kernel<<<(H + 255) / 256, 256, 0, st>>>(colpart, mt, H, 0, nullptr, nullptr, db0);
-    rc = check_launch();
+    if (!rc) rc = wide_col_finalize(ws + L.colpart, L.mt, H, 0, nullptr, nullptr, db0, st);
     if (rc) return rc;
   }
   if (!dz) return B200VAE_OK;
   // ---- dz [B,nz] = t0 A0[:, :nz] + 2 kappa v[:, :nz]
   WtArgs e;
   memset(&e, 0, sizeof(e));
-  rc = wt_map(&e.a1, t0, H, B, H, 128);
-  if (!rc) rc = wt_map(&e.b1hi, ws + L.A0Thi, H, nz, H, bn);
-  if (!rc) rc = wt_map(&e.b1lo, ws + (x3 ? L.A0Tlo : L.A0Thi), H, nz, H, bn);
+  rc = tma_map_2d(&e.a1, t0, H, B, H, 128);
+  if (!rc) rc = tma_map_2d(&e.b1hi, ws + L.A0Thi, H, nz, H, bn);
+  if (!rc) rc = tma_map_2d(&e.b1lo, ws + (x3 ? L.A0Tlo : L.A0Thi), H, nz, H, bn);
   if (rc) return rc;
   e.a2 = e.a1; e.b2hi = e.b1hi; e.b2lo = e.b1lo;
   e.nkb1 = nkb(H); e.nkb2 = 0; e.xf1 = WT_XF_ID; e.M = B; e.N = nz; e.epi = WT_EPI_DZ; e.v = v; e.ldv = d; e.kappa2 = 2.f * kappa;
@@ -672,80 +579,58 @@ int wide_tc_bwd_rows(const float* v, const float* h0, const uint8_t* mask1, cons
 
 // Batch-reduction GEMMs of the backward on tcgen05:  dA0 = g0^T v + t0^T z,  dA1 = g1^T v,  dP0 = g1^T q1 (-> dW0).
 // The operands are transposed first (batch -> contiguous K; B operands split hi/lo on the way), then each product is the
-// generic GEMM with M = H, K = B, split over K into `splits` slabs that are summed in fixed order.
-struct WtTnLayout { size_t g0T, t0T, g1T, vThi, vTlo, zThi, zTlo, q1Thi, q1Tlo, slabs, end; int ldb, splits; };
-static WtTnLayout wt_tn_layout(int B, int d, int nz, int H) {
-  WtTnLayout T;
-  T.ldb = (B + 3) / 4 * 4;
-  const size_t HB = wt_up((size_t)H * T.ldb), dB = wt_up((size_t)d * T.ldb), zB = wt_up((size_t)nz * T.ldb);
-  const int tiles = ((H + 127) / 128) * ((H + 255) / 256);
-  int s = (148 + tiles - 1) / tiles, maxs = (B + 255) / 256;
-  T.splits = s < maxs ? s : maxs;
-  if (T.splits < 1) T.splits = 1;
-  if (T.splits > 16) T.splits = 16;
-  size_t o = 0;
-  T.g0T = o; o += HB; T.t0T = o; o += HB; T.g1T = o; o += HB;
-  T.vThi = o; o += dB; T.vTlo = o; o += dB; T.zThi = o; o += zB; T.zTlo = o; o += zB; T.q1Thi = o; o += HB; T.q1Tlo = o; o += HB;
-  T.slabs = o; o += wt_up((size_t)T.splits * H * (H > d ? H : d));
-  T.end = o;
-  return T;
-}
-size_t wide_tc_tn_ws_floats(int B, int d, int H) { return wt_tn_layout(B, d, d, H).end; }
-
+// generic GEMM with M = H, K = B, split over K into L.splits slabs that are summed in fixed order.
 int wide_tc_bwd_tn(const float* z, const float* v, const uint8_t* mask1, const float* s2, const float* q1, const float* g0,
-                   const float* t0, int B, int d, int nz, int H, const b200vae_icnn_params* p, int mode, const float* P1,
-                   float* dA0w, float* dA1w, float* dW0, float* ws, int precision, cudaStream_t st) {
-  if (!wide_tc_supported(d, nz, H, precision)) return B200VAE_EUNSUP;
+                   const float* t0, int B, int d, int nz, int H, const b200vae_icnn_params* p, int mode, float* dA0w, float* dA1w,
+                   float* dW0, float* ws, const WideLayout& L, int precision, cudaStream_t st) {
   const bool x3 = precision == B200VAE_PREC_TF32X3;
-  const WtTnLayout T = wt_tn_layout(B, d, nz, H);
-  const int ldb = T.ldb, bn = wt_tile_n(x3);
+  const int ldb = L.ldb, bn = wt_tile_n(x3);
   int rc;
   auto transpose = [&](const float* src, int md, int C, float* hi, float* lo) {
     dim3 grid((B + 31) / 32, (C + 31) / 32);
-    wide_tc_transpose_kernel<<<grid, 256, 0, st>>>(src, mask1, s2, P1, md, B, C, ldb, hi, lo);
+    wide_tc_transpose_kernel<<<grid, 256, 0, st>>>(src, mask1, s2, ws + L.P1, md, B, C, ldb, hi, lo);
     return check_launch();
   };
-  const int nkb_all = (B + kKB - 1) / kKB, per = (nkb_all + T.splits - 1) / T.splits;
+  const int nkb_all = (B + kKB - 1) / kKB, per = (nkb_all + L.splits - 1) / L.splits;
   const int chain = mode == B200VAE_WEIGHT_EXP ? 1 : 2;
   auto gemm = [&](const float* At, const float* Bhi, const float* Blo, int N, const float* At2, const float* B2hi,
                   const float* B2lo, int N2) {
     WtArgs a;
     memset(&a, 0, sizeof(a));
-    int r = wt_map(&a.a1, At, B, H, ldb, 128);
-    if (!r) r = wt_map(&a.b1hi, Bhi, B, N, ldb, bn);
-    if (!r) r = wt_map(&a.b1lo, x3 ? Blo : Bhi, B, N, ldb, bn);
+    int r = tma_map_2d(&a.a1, At, B, H, ldb, 128);
+    if (!r) r = tma_map_2d(&a.b1hi, Bhi, B, N, ldb, bn);
+    if (!r) r = tma_map_2d(&a.b1lo, x3 ? Blo : Bhi, B, N, ldb, bn);
     if (!r && At2) {
-      r = wt_map(&a.a2, At2, B, H, ldb, 128);
-      if (!r) r = wt_map(&a.b2hi, B2hi, B, N2, ldb, bn);
-      if (!r) r = wt_map(&a.b2lo, x3 ? B2lo : B2hi, B, N2, ldb, bn);
+      r = tma_map_2d(&a.a2, At2, B, H, ldb, 128);
+      if (!r) r = tma_map_2d(&a.b2hi, B2hi, B, N2, ldb, bn);
+      if (!r) r = tma_map_2d(&a.b2lo, x3 ? B2lo : B2hi, B, N2, ldb, bn);
     } else if (!r) {
       a.a2 = a.a1; a.b2hi = a.b1hi; a.b2lo = a.b1lo;
     }
     if (r) return r;
-    a.nkb1 = per; a.nkb2 = At2 ? per : 0; a.xf1 = WT_XF_ID; a.M = H; a.N = N; a.epi = WT_EPI_SLAB; a.out0 = ws + T.slabs;
+    a.nkb1 = per; a.nkb2 = At2 ? per : 0; a.xf1 = WT_XF_ID; a.M = H; a.N = N; a.epi = WT_EPI_SLAB; a.out0 = ws + L.slabs;
     a.kb_per_split = per;
-    return wt_run(a, x3, st, T.splits);
+    return wt_run(a, x3, st, L.splits);
   };
   auto finalize = [&](size_t n, int ch, const float* W, float* out) {
-    wide_tc_slabfin_kernel<<<148 * 4, 256, 0, st>>>(ws + T.slabs, T.splits, n, ch, W, out);
-    return check_launch();
+    return wide_slab_finalize(ws + L.slabs, L.splits, n, ch, W, out, st);
   };
-  if (dA0w || dA1w) { rc = transpose(v, 0, d, ws + T.vThi, x3 ? ws + T.vTlo : nullptr); if (rc) return rc; }
-  if (dA1w || dW0) { rc = transpose(nullptr, 1, H, ws + T.g1T, nullptr); if (rc) return rc; }
+  if (dA0w || dA1w) { rc = transpose(v, 0, d, ws + L.vThi, x3 ? ws + L.vTlo : nullptr); if (rc) return rc; }
+  if (dA1w || dW0) { rc = transpose(nullptr, 1, H, ws + L.g1T, nullptr); if (rc) return rc; }
   if (dA0w) {
-    rc = transpose(g0, 0, H, ws + T.g0T, nullptr); if (rc) return rc;
-    rc = transpose(t0, 0, H, ws + T.t0T, nullptr); if (rc) return rc;
-    rc = transpose(z, 0, nz, ws + T.zThi, x3 ? ws + T.zTlo : nullptr); if (rc) return rc;
-    rc = gemm(ws + T.g0T, ws + T.vThi, ws + T.vTlo, d, ws + T.t0T, ws + T.zThi, ws + T.zTlo, nz); if (rc) return rc;
+    rc = transpose(g0, 0, H, ws + L.g0T, nullptr); if (rc) return rc;
+    rc = transpose(t0, 0, H, ws + L.t0T, nullptr); if (rc) return rc;
+    rc = transpose(z, 0, nz, ws + L.zThi, x3 ? ws + L.zTlo : nullptr); if (rc) return rc;
+    rc = gemm(ws + L.g0T, ws + L.vThi, ws + L.vTlo, d, ws + L.t0T, ws + L.zThi, ws + L.zTlo, nz); if (rc) return rc;
     rc = finalize((size_t)H * d, 0, nullptr, dA0w); if (rc) return rc;
   }
   if (dA1w) {
-    rc = gemm(ws + T.g1T, ws + T.vThi, ws + T.vTlo, d, nullptr, nullptr, nullptr, 0); if (rc) return rc;
+    rc = gemm(ws + L.g1T, ws + L.vThi, ws + L.vTlo, d, nullptr, nullptr, nullptr, 0); if (rc) return rc;
     rc = finalize((size_t)H * d, 0, nullptr, dA1w); if (rc) return rc;
   }
   if (dW0) {
-    rc = transpose(q1, 0, H, ws + T.q1Thi, x3 ? ws + T.q1Tlo : nullptr); if (rc) return rc;
-    rc = gemm(ws + T.g1T, ws + T.q1Thi, ws + T.q1Tlo, H, nullptr, nullptr, nullptr, 0); if (rc) return rc;
+    rc = transpose(q1, 0, H, ws + L.q1Thi, x3 ? ws + L.q1Tlo : nullptr); if (rc) return rc;
+    rc = gemm(ws + L.g1T, ws + L.q1Thi, ws + L.q1Tlo, H, nullptr, nullptr, nullptr, 0); if (rc) return rc;
     rc = finalize((size_t)H * H, chain, p->W0, dW0); if (rc) return rc;
   }
   return B200VAE_OK;

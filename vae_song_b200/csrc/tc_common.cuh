@@ -96,6 +96,32 @@ __device__ __forceinline__ uint64_t make_desc_sw64(uint32_t saddr) {
          ((uint64_t)4 << 61);
 }
 
+// ------------------------------------------------------------------------------------ host: TMA descriptors
+// 2-D tensor [rows][K] of fp32 (or fp16) elements, row stride `ld` elements; boxes of 64 bytes of K x box_rows rows,
+// 64-byte swizzle, zero fill outside the tensor.  The driver entry point is looked up through the runtime (no -lcuda).
+inline int tma_map_2d(CUtensorMap* m, const void* base, int K, int rows, int ld, int box_rows, bool f16 = false) {
+  typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
+                                    const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
+                                    CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
+  static const EncodeTiledFn fn = [] {
+    void* p = nullptr;
+    cudaDriverEntryPointQueryResult q;
+    const bool ok = cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess;
+    return ok ? reinterpret_cast<EncodeTiledFn>(p) : nullptr;
+  }();
+  if (!fn) return B200VAE_ECUDA;
+  const size_t esize = f16 ? 2 : sizeof(float);
+  const cuuint64_t dims[2] = {(cuuint64_t)K, (cuuint64_t)rows};
+  const cuuint64_t strides[1] = {(cuuint64_t)ld * esize};
+  const cuuint32_t box[2] = {(cuuint32_t)(64 / esize), (cuuint32_t)box_rows};
+  const cuuint32_t estr[2] = {1, 1};
+  CUresult r = fn(m, f16 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, const_cast<void*>(base), dims,
+                  strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_64B,
+                  CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  if (r != CUDA_SUCCESS) { g_last_cuda_error = 100000 + (int)r; return B200VAE_ECUDA; }
+  return B200VAE_OK;
+}
+
 template <int D>
 __device__ __forceinline__ float lin_of(const float4 q, const float (&z)[D]) {
   float h = q.w;

@@ -335,14 +335,12 @@ def _grads_struct(tensors):
 
 
 def icnn_wide_fwd(z, params, mode, kappa, want_xhat=True, precision=0):
-    """Fused FP32 forward of a wide-input ICNN (csrc/icnn_wide.cu).  Returns (psi [B], xhat [B,d] | None, saved) with
+    """Fused forward of a wide-input ICNN (b200vae_icnn_wide_fwd; an unknown precision id raises B200VaeError).  Returns (psi [B], xhat [B,d] | None, saved) with
     saved = (h0 [B,H], mask1 [B,H] uint8, s2 [B]) -- what the backward needs besides z."""
     lib = _C.load()
     B, nz = z.shape
     H, d = params[0].shape
     dev = z.device
-    if precision not in (_C.PREC_FP32, _C.PREC_TF32, _C.PREC_TF32X3, _C.PREC_F16X3):
-        raise _C.B200VaeError(f"unknown precision id {precision}; use fp32, f16x3, tf32x3 or tf32")
     ws = torch.empty(lib.b200vae_icnn_wide_workspace_bytes(B, d, H, precision, 0), dtype=torch.uint8, device=dev)
     psi = torch.empty(B, dtype=torch.float32, device=dev)
     h0 = torch.empty(B, H, dtype=torch.float32, device=dev)
@@ -363,8 +361,9 @@ class IcnnBrenierWideFn(torch.autograd.Function):
     [B,d]x[d,H] contractions as well; the path is a chain of fused FP32 tile-GEMM kernels with generated operands and
     elementwise epilogues (csrc/icnn_wide.cu): the ANALYTIC forward-then-reverse sweep and double-backward of SURVEY
     Appendix A, no autograd graph, h0 + a byte mask saved instead of ~20 activations.  `precision`: fp32 = those kernels;
-    tf32 / tf32x3 = forward and the sample-stationary GEMMs of the backward on tcgen05 (csrc/icnn_wide_tc.cu), the
-    batch-reduction GEMMs (dA0, dA1, dP0) stay FP32.  z may be NARROWER than the ICNN input ([B,nz], nz <= d): it is then
+    tf32 / tf32x3 (f16x3 runs as tf32x3) = the forward and every GEMM of the dL/dxhat backward, batch reductions included,
+    on tcgen05 (csrc/icnn_wide_tc.cu) when d, nz and H are multiples of 4 -- else, and for a forward whose b0 / b1 / A2
+    are not 16-byte aligned, the FP32 kernels; the psi-gradient term always runs on the FP32 kernels.  z may be NARROWER than the ICNN input ([B,nz], nz <= d): it is then
     taken as zero-padded to d columns -- the eye(Dx,D) pad of model.py:824 fused away -- and dz is [B,nz]."""
 
     @staticmethod
