@@ -106,6 +106,30 @@ int b200vae_icnn_decode_bwd_params(const float* z, const float* v, const uint32_
                                    const b200vae_icnn_grads* grads, int precision, void* ws, size_t ws_bytes,
                                    void* stream);
 
+/* Exact Jacobian of the Brenier map, from the same fused forward.  With the LeakyReLU masks fixed xhat is affine in z, so
+ *   jac[b] = d xhat_b / d z_b = A0^T diag(2 s0^2 gx1) A0 + 2 kappa I          (d x d, symmetric, >= 2 kappa I)
+ * where gx1 = g1 . P0 is the forward's second contraction; it is the derivative almost everywhere (wherever no pre-
+ * activation sits exactly on its kink) and NOT differentiable itself.  psi, xhat and the masks are bitwise those of
+ * b200vae_icnn_decode_fwd on the same inputs and precision; the saved-accumulator state of a for_backward workspace is left
+ * alone, so a Jacobian call may sit between a training forward and its backward.
+ *   ws: prepared by b200vae_icnn_prepare (a for_backward workspace is accepted); jac [B,d,d] (required);
+ *   jac_scratch: caller-owned, at least b200vae_icnn_jac_scratch_bytes(B, d, H, precision) bytes, 16-byte aligned (the
+ *   tensor-core precisions publish per-(row, pass, column half) partials there: Bp * ceil(H/256) * 2 * (d <= 2 ? 1 : 2)
+ *   float4, Bp = B rounded up to 256; FP32 needs none and may pass NULL).
+ * Same shape / precision rules as b200vae_icnn_decode_fwd; _scratch_bytes returns 0 where the entry refuses (and for FP32,
+ * which needs no scratch). */
+size_t b200vae_icnn_jac_scratch_bytes(int B, int d, int H, int precision);
+int b200vae_icnn_decode_jac(const float* z, int B, int d, int H, float kappa, float* psi, float* xhat, float* jac,
+                            uint32_t* mask1, uint8_t* mask2, int precision, const void* ws, size_t ws_bytes,
+                            void* jac_scratch, size_t jac_scratch_bytes, void* stream);
+
+/* Chain rule of the decoder's two Brenier maps and its singular values, one thread per sample, fp64 inside:
+ *   J[b] = J2[b] . M . J1[b]      J2 [B,Dx,Dx], M [Dx,D] (LIDVAE's B buffer), J1 [B,D,D]  ->  J [B,Dx,D] or NULL
+ *   svals [B,min(Dx,D)] or NULL: singular values of J[b] in descending order (one-sided Jacobi, fixed sweeps).
+ * 1 <= D, Dx <= 4; anything else returns B200VAE_EUNSUP. */
+int b200vae_jacobian_chain(const float* J2, const float* M, const float* J1, int B, int Dx, int D, float* J, float* svals,
+                           void* stream);
+
 /* Fused reparameterisation + Gaussian KL + reconstruction (+ latent reconstruction).
  * Replaces model.py:843 / :423-424 (z = mu + eps*exp(lv/2)), :884/:550/:606 (KL), :870/:542/:589
  * (MSE) or :872-882 (log-MSE), :551/:603 (latent recon, mean over dim 0 = L).

@@ -36,6 +36,7 @@ EXPORTS = [
     "b200vae_mi_logqz", "b200vae_nll_iw_lse", "b200vae_nll_iw_scratch_bytes", "b200vae_mlp_stack_fwd",
     "b200vae_mlp_stack_bwd", "b200vae_lipschitz_select_state_bytes", "b200vae_lipschitz_select_hist_bytes",
     "b200vae_lipschitz_quantile_ranks", "b200vae_lipschitz_select_count", "b200vae_lipschitz_select_locate",
+    "b200vae_icnn_jac_scratch_bytes", "b200vae_icnn_decode_jac", "b200vae_jacobian_chain",
 ]
 LIPSCHITZ_SELECT_PASSES = 3
 PEER_MAX_WORLD, PEER_HANDLE_BYTES = 16, 64
@@ -107,6 +108,12 @@ def load():
     lib.b200vae_icnn_decode_bwd_params.restype = i
     lib.b200vae_icnn_decode_bwd_params.argtypes = [vp, vp, vp, vp, i, i, i, C.POINTER(IcnnParams), i, C.POINTER(IcnnGrads), i,
                                                    vp, sz, vp]
+    lib.b200vae_icnn_jac_scratch_bytes.restype = sz
+    lib.b200vae_icnn_jac_scratch_bytes.argtypes = [i, i, i, i]
+    lib.b200vae_icnn_decode_jac.restype = i
+    lib.b200vae_icnn_decode_jac.argtypes = [vp, i, i, i, f, vp, vp, vp, vp, vp, i, vp, sz, vp, sz, vp]
+    lib.b200vae_jacobian_chain.restype = i
+    lib.b200vae_jacobian_chain.argtypes = [vp, vp, vp, i, i, i, vp, vp, vp]
     lib.b200vae_loss_fwd.restype = i
     lib.b200vae_loss_fwd.argtypes = [vp, vp, vp, vp, i, i, i, vp, vp, i, i, vp, vp, vp, i, i, i, vp, vp]
     lib.b200vae_loss_bwd.restype = i

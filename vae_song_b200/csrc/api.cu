@@ -187,6 +187,32 @@ extern "C" int b200vae_icnn_decode_bwd_params(const float* z, const float* v, co
                 (cudaStream_t)stream);
 }
 
+static size_t jac_scratch_of(const WsLayout& L) {
+  return (size_t)L.Bp * L.NP * 2 * tc3_jac_slots(L.d) * sizeof(float4);
+}
+
+extern "C" size_t b200vae_icnn_jac_scratch_bytes(int B, int d, int H, int precision) {
+  if (shape_ok(B, d, H, precision) || precision == B200VAE_PREC_FP32) return 0;
+  return jac_scratch_of(icnn_ws_layout(B, d, H, precision, false));
+}
+
+extern "C" int b200vae_icnn_decode_jac(const float* z, int B, int d, int H, float kappa, float* psi, float* xhat, float* jac,
+                                       uint32_t* mask1, uint8_t* mask2, int precision, const void* ws, size_t ws_bytes,
+                                       void* jac_scratch, size_t jac_scratch_bytes, void* stream) {
+  int rc = shape_ok(B, d, H, precision);
+  if (rc) return rc;
+  if (!z || !ws || !jac || !xhat || !aligned4(z)) return B200VAE_EALIGN;
+  if (ws_bytes < b200vae_icnn_workspace_bytes(B, d, H, precision, 0)) return B200VAE_EWS;
+  const WsLayout L = icnn_ws_layout(B, d, H, precision, false);
+  if (precision == B200VAE_PREC_FP32)
+    return simt_fwd_jac(z, L, kappa, psi, xhat, mask1, mask2, jac, ws_base(ws), (cudaStream_t)stream);
+  if (!jac_scratch || (reinterpret_cast<uintptr_t>(jac_scratch) & 15)) return B200VAE_EALIGN;
+  if (jac_scratch_bytes < jac_scratch_of(L)) return B200VAE_EWS;
+  // no save_forget / save_record: this variant never writes the saved accumulators, so a save stays valid across it
+  return tc3_fwd_jac(z, L, kappa, psi, xhat, mask1, mask2, jac, reinterpret_cast<float4*>(jac_scratch), precision,
+                     ws_base(ws), (cudaStream_t)stream);
+}
+
 extern "C" int b200vae_last_cuda_error(void) { return g_last_cuda_error; }
 extern "C" const char* b200vae_version(void) { return "b200vae 0.2 (sm_100a)"; }
 extern "C" long long b200vae_launch_count(void) { return g_launch_count; }

@@ -83,6 +83,8 @@ inline int dp0_splits(int B, int Hq, int clusters) {
 int simt_prepare(const b200vae_icnn_params* p, const WsLayout& L, int mode, float* ws, cudaStream_t st);
 int simt_fwd(const float* z, const WsLayout& L, float kappa, float* psi, float* xhat, uint32_t* mask1, uint8_t* mask2,
              const float* ws, cudaStream_t st);
+int simt_fwd_jac(const float* z, const WsLayout& L, float kappa, float* psi, float* xhat, uint32_t* mask1, uint8_t* mask2,
+                 float* jac, const float* ws, cudaStream_t st);
 int simt_bwd(const float* z, const float* v, const float* gpsi, const uint32_t* mask1, const uint8_t* mask2, const WsLayout& L,
              const b200vae_icnn_params* p, int mode, float kappa, const b200vae_icnn_grads* g, float* dz, float* ws,
              cudaStream_t st);
@@ -92,6 +94,13 @@ int finalize_W0_launch(const float* part, int splits, int H, int Hp, int ldp, co
 int tc3_prepare(const WsLayout& L, int precision, float* ws, cudaStream_t st);
 int tc3_fwd(const float* z, const WsLayout& L, float kappa, float* psi, float* xhat, uint32_t* mask1, uint8_t* mask2,
             int precision, float* ws, float* accsave, cudaStream_t st);
+// the same forward, also writing jac [B,d,d]; jscr: tc3_jac_slots(d) float4 per (row, pass, column half), Bp x NP x 2 of them
+inline int tc3_jac_slots(int d) { return d <= 2 ? 1 : 2; }
+int tc3_fwd_jac(const float* z, const WsLayout& L, float kappa, float* psi, float* xhat, uint32_t* mask1, uint8_t* mask2,
+                float* jac, float4* jscr, int precision, float* ws, cudaStream_t st);
+// chain + singular values of the decoder's Jacobian, jacobian.cu
+int jacobian_chain(const float* J2, const float* M, const float* J1, int B, int Dx, int D, float* J, float* svals,
+                   cudaStream_t st);
 int tc_bwd(const float* z, const float* v, const uint32_t* mask1, const uint8_t* mask2, const WsLayout& L,
            const b200vae_icnn_params* p, int mode, float kappa, const b200vae_icnn_grads* g, float* dz, int precision,
            float* ws, const float* accsave, int phase, cudaStream_t st);

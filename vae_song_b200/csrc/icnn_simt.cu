@@ -183,12 +183,19 @@ __device__ __forceinline__ float row_reduce_load(const float* scratch, int row, 
 }
 
 // ------------------------------------------------------------------------------------- forward
+// kJac: also the Jacobian of the Brenier map, J = dxhat/dz = A0^T diag(2 s0^2 gx1) A0 + 2 kappa I (jac [B][D][D]).  With the
+// masks fixed xhat is affine in z; gx1 = g1 . P0 is the phase-2 accumulator, so J costs D(D+1)/2 FMAs per (sample, unit).
 template <int D>
-__global__ void __launch_bounds__(kThreads, 2)
-icnn_fwd_kernel(const float* __restrict__ z, int B, int Hp, float kappa, const float* __restrict__ P0,
-                const float* __restrict__ P0T, const float* __restrict__ P1, const float* __restrict__ A0p,
-                const float* __restrict__ A1p, const float* __restrict__ A2p, float* __restrict__ psi,
-                float* __restrict__ xhat, uint32_t* __restrict__ mask1, uint8_t* __restrict__ mask2) {
+constexpr int kJacPairs = D * (D + 1) / 2;      // upper triangle, row-major: (0,0) (0,1) .. (0,D-1) (1,1) ..
+
+template <int D, bool kJac>
+__device__ __forceinline__ void icnn_fwd_body(const float* __restrict__ z, int B, int Hp, float kappa,
+                                              const float* __restrict__ P0, const float* __restrict__ P0T,
+                                              const float* __restrict__ P1, const float* __restrict__ A0p,
+                                              const float* __restrict__ A1p, const float* __restrict__ A2p,
+                                              float* __restrict__ psi, float* __restrict__ xhat,
+                                              uint32_t* __restrict__ mask1, uint8_t* __restrict__ mask2,
+                                              float* __restrict__ jac) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   SmemMap<D> S(smem_raw, Hp);
   const TileCoord tc;
@@ -286,6 +293,14 @@ icnn_fwd_kernel(const float* __restrict__ z, int B, int Hp, float kappa, const f
   for (int i = 0; i < 8; ++i)
 #pragma unroll
     for (int j = 0; j < D; ++j) xh[i][j] = 0.f;
+  constexpr int NJ = kJac ? kJacPairs<D> : 1;
+  float yj[8][NJ];                               // kJac: sum_n A0[n,a] A0[n,b] s0^2 gx1 over my columns
+  if constexpr (kJac) {
+#pragma unroll
+    for (int i = 0; i < 8; ++i)
+#pragma unroll
+      for (int q = 0; q < NJ; ++q) yj[i][q] = 0.f;
+  }
   AGenG1<D, true> ag;
   ag.P1s = S.P1s; ag.A1s = S.A1s; ag.maskrow = S.maskb + mg * MS; ag.s2 = S.s2s[mg]; ag.m = mg; ag.kgrp = kgrp;
 #pragma unroll
@@ -297,15 +312,27 @@ icnn_fwd_kernel(const float* __restrict__ z, int B, int Hp, float kappa, const f
 #pragma unroll
     for (int j = 0; j < 8; ++j) {
       const float* a = S.A0s + (n0 + tc.col(j)) * (D + 1);
+      float aa[NJ];
+      if constexpr (kJac) {
+#pragma unroll
+        for (int ja = 0, q = 0; ja < D; ++ja)
+#pragma unroll
+          for (int jb = ja; jb < D; ++jb, ++q) aa[q] = a[ja] * a[jb];
+      }
 #pragma unroll
       for (int i = 0; i < 8; ++i) {
         float h = a[D];
 #pragma unroll
-        for (int jj = 0; jj < D; ++jj) h = fmaf(a[jj], zr[i][jj], h);
+        for (int jj = 0; jj < D; ++jj) h = fmaf(a[jj], kJac ? S.zs[tc.row(i) * D + jj] : zr[i][jj], h);
         const float s0 = slope_of(h), a0 = h * s0;
         const float g0 = acc[i][j] * (2.f * a0) * s0;
 #pragma unroll
         for (int jj = 0; jj < D; ++jj) xh[i][jj] = fmaf(a[jj], g0, xh[i][jj]);
+        if constexpr (kJac) {
+          const float w = (s0 * s0) * acc[i][j];
+#pragma unroll
+          for (int q = 0; q < NJ; ++q) yj[i][q] = fmaf(aa[q], w, yj[i][q]);
+        }
       }
     }
   }
@@ -324,6 +351,56 @@ icnn_fwd_kernel(const float* __restrict__ z, int B, int Hp, float kappa, const f
       xhat[(size_t)(m0 + r) * D + j] = x;
     }
   }
+  if constexpr (kJac) {
+    // the same ordered cross-warp reduction, in chunks of NCH pairs (8 x 128 x NCH floats of the 32 KB scratch)
+    constexpr int NCH = NJ <= 8 ? NJ : NJ / 2;
+    static_assert(NJ % NCH == 0 && NCH <= 8, "Jacobian chunks must tile the pairs and fit the scratch");
+#pragma unroll
+    for (int c0 = 0; c0 < NJ; c0 += NCH) {
+      __syncthreads();
+#pragma unroll
+      for (int i = 0; i < 8; ++i)
+#pragma unroll
+        for (int q = 0; q < NCH; ++q) {
+          float v = yj[i][c0 + q];
+          v += __shfl_xor_sync(0xffffffffu, v, 1);
+          if (tc.txl == 0) scratch[(tc.w * 128 + tc.row(i)) * NCH + q] = v;
+        }
+      __syncthreads();
+      for (int i = tid; i < 128 * NCH; i += kThreads) {
+        const int r = i / NCH, q = i - r * NCH;
+        if (m0 + r >= B) continue;
+        int ja = 0, jb = c0 + q;                       // pair index -> (ja, jb), ja <= jb
+        while (jb >= D - ja) { jb -= D - ja; ++ja; }
+        jb += ja;
+        const float y = row_reduce_load<NCH>(scratch, r, q);
+        const float v = ja == jb ? fmaf(2.f, y, 2.f * kappa) : 2.f * y;
+        float* J = jac + (size_t)(m0 + r) * D * D;
+        J[ja * D + jb] = v;
+        J[jb * D + ja] = v;
+      }
+    }
+  }
+}
+
+template <int D>
+__global__ void __launch_bounds__(kThreads, 2)
+icnn_fwd_kernel(const float* __restrict__ z, int B, int Hp, float kappa, const float* __restrict__ P0,
+                const float* __restrict__ P0T, const float* __restrict__ P1, const float* __restrict__ A0p,
+                const float* __restrict__ A1p, const float* __restrict__ A2p, float* __restrict__ psi,
+                float* __restrict__ xhat, uint32_t* __restrict__ mask1, uint8_t* __restrict__ mask2) {
+  icnn_fwd_body<D, false>(z, B, Hp, kappa, P0, P0T, P1, A0p, A1p, A2p, psi, xhat, mask1, mask2, nullptr);
+}
+
+// one CTA per SM: the 8 x D(D+1)/2 Jacobian accumulators need the register file of the whole SM share (no spills)
+template <int D>
+__global__ void __launch_bounds__(kThreads, 1)
+icnn_fwd_jac_kernel(const float* __restrict__ z, int B, int Hp, float kappa, const float* __restrict__ P0,
+                    const float* __restrict__ P0T, const float* __restrict__ P1, const float* __restrict__ A0p,
+                    const float* __restrict__ A1p, const float* __restrict__ A2p, float* __restrict__ psi,
+                    float* __restrict__ xhat, uint32_t* __restrict__ mask1, uint8_t* __restrict__ mask2,
+                    float* __restrict__ jac) {
+  icnn_fwd_body<D, true>(z, B, Hp, kappa, P0, P0T, P1, A0p, A1p, A2p, psi, xhat, mask1, mask2, jac);
 }
 
 // ----------------------------------------------------------------------- backward, sample-stationary
@@ -696,6 +773,22 @@ static int launch_fwd(const float* z, int B, const WsLayout& L, const float* ws,
   return check_launch();
 }
 
+template <int D>
+static int launch_fwd_jac(const float* z, int B, const WsLayout& L, const float* ws, float kappa, float* psi,
+                          float* xhat, uint32_t* mask1, uint8_t* mask2, float* jac, cudaStream_t st) {
+  const size_t smem = SmemMap<D>::bytes(L.Hp);
+  static bool attr_done = false;
+  if (!attr_done) {
+    cudaFuncSetAttribute(icnn_fwd_jac_kernel<D>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
+    attr_done = true;
+  }
+  if (smem > 200 * 1024) return B200VAE_EUNSUP;
+  icnn_fwd_jac_kernel<D><<<L.n_mtiles, kThreads, smem, st>>>(z, B, L.Hp, kappa, ws + L.P0, ws + L.P0T, ws + L.P1,
+                                                              ws + L.A0p, ws + L.A1p, ws + L.A2p, psi, xhat, mask1,
+                                                              mask2, jac);
+  return check_launch();
+}
+
 template <int D, bool G>
 static int launch_bwd(const float* z, const float* v, const float* gpsi, const uint32_t* mask1,
                       const uint8_t* mask2, int B, const WsLayout& L, float* ws, float kappa, float* dz,
@@ -745,6 +838,18 @@ int simt_fwd(const float* z, const WsLayout& L, float kappa, float* psi, float* 
     case 2: return launch_fwd<2>(z, B, L, ws, kappa, psi, xhat, mask1, mask2, st);
     case 3: return launch_fwd<3>(z, B, L, ws, kappa, psi, xhat, mask1, mask2, st);
     case 4: return launch_fwd<4>(z, B, L, ws, kappa, psi, xhat, mask1, mask2, st);
+    default: return B200VAE_EUNSUP;
+  }
+}
+
+int simt_fwd_jac(const float* z, const WsLayout& L, float kappa, float* psi, float* xhat, uint32_t* mask1, uint8_t* mask2,
+                 float* jac, const float* ws, cudaStream_t st) {
+  const int B = L.B;
+  switch (L.d) {
+    case 1: return launch_fwd_jac<1>(z, B, L, ws, kappa, psi, xhat, mask1, mask2, jac, st);
+    case 2: return launch_fwd_jac<2>(z, B, L, ws, kappa, psi, xhat, mask1, mask2, jac, st);
+    case 3: return launch_fwd_jac<3>(z, B, L, ws, kappa, psi, xhat, mask1, mask2, jac, st);
+    case 4: return launch_fwd_jac<4>(z, B, L, ws, kappa, psi, xhat, mask1, mask2, jac, st);
     default: return B200VAE_EUNSUP;
   }
 }

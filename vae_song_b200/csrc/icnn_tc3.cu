@@ -344,9 +344,10 @@ __device__ __forceinline__ Unit decode_unit(int u, int T, int NP) {
   return x;
 }
 
-template <int D, int MODE>
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(k3Threads, 1)
-icnn_tc3_fwd_kernel(const __grid_constant__ Tc3Args a) {
+// JAC: also the Brenier map's Jacobian (icnn_simt.cu, icnn_fwd_body): GEMM2 units accumulate Y[a][b] = sum_o A0[o,a] A0[o,b]
+// s0^2 r (a <= b; r = gx1 / s2) beside X, publish them to jscr like scr2, and the finalizing unit writes J = 2 s2 Y + 2 kappa I.
+template <int D, int MODE, bool JAC>
+__device__ __forceinline__ void tc3_fwd_body(const Tc3Args& a, float4* __restrict__ jscr, float* __restrict__ jac) {
   using C = Tc3Cfg<MODE>;
   constexpr int S = C::S;
   constexpr bool X3 = C::HL, F16 = C::F16;                                 // X3: hi/lo operands, three (two) MMAs per K step
@@ -522,6 +523,11 @@ icnn_tc3_fwd_kernel(const __grid_constant__ Tc3Args a) {
           *reinterpret_cast<uint4*>(a.maskg + (size_t)grow * a.mask_stride + w0) = make_uint4(words[0], words[1], words[2], words[3]);
       } else {
         float X[3] = {0.f, 0.f, 0.f};
+        float Y[JAC ? (D * (D + 1)) / 2 : 1];
+        if constexpr (JAC) {
+#pragma unroll
+          for (int q = 0; q < (D * (D + 1)) / 2; ++q) Y[q] = 0.f;
+        }
 #pragma unroll
         for (int cc = 0; cc < 4; ++cc) {
           uint32_t r[32];
@@ -544,12 +550,29 @@ icnn_tc3_fwd_kernel(const __grid_constant__ Tc3Args a) {
             const float wv = f0 * __uint_as_float(r[j]);
 #pragma unroll
             for (int jj = 0; jj < D; ++jj) X[jj] = fmaf(comp(q, jj), wv, X[jj]);
+            if constexpr (JAC) {
+              const float yv = (h0 > 0.f ? 1.f : kSlope * kSlope) * __uint_as_float(r[j]);
+#pragma unroll
+              for (int ja = 0, p = 0; ja < D; ++ja)
+#pragma unroll
+                for (int jb = ja; jb < D; ++jb, ++p) Y[p] = fmaf(comp(q, ja) * comp(q, jb), yv, Y[p]);
+            }
           }
         }
         tc_fence_before();
         __syncwarp();
         if (lane == 0) mbar_arrive_remote(lead_accempty0 + 8 * buf);
         a.scr2[sidx] = make_float4(X[0], X[1], X[2], 0.f);
+        if constexpr (JAC) {
+          if constexpr (D == 1) {
+            jscr[sidx] = make_float4(Y[0], 0.f, 0.f, 0.f);
+          } else if constexpr (D == 2) {
+            jscr[sidx] = make_float4(Y[0], Y[1], Y[2], 0.f);
+          } else {
+            jscr[2 * sidx] = make_float4(Y[0], Y[1], Y[2], Y[3]);
+            jscr[2 * sidx + 1] = make_float4(Y[4], Y[5], 0.f, 0.f);
+          }
+        }
       }
       // ---- publish the unit; the last unit of this (tile, rank) combines all partials in a fixed order ----
       __threadfence();
@@ -589,6 +612,27 @@ icnn_tc3_fwd_kernel(const __grid_constant__ Tc3Args a) {
                 const float a1 = fmaf(0.8f, tp[j], kSlope * a.sumV[j]);
                 const float inner = fmaf(2.f, X[j], a1) + a.A2p[j];
                 a.xhat[(size_t)fr * D + j] = fmaf(2.f * a.kappa, zf[j], s2 * inner);
+              }
+              if constexpr (JAC) {
+                // same fixed order as scr2; J = 2 s2 Y + 2 kappa I, both triangles
+                constexpr int NS = D <= 2 ? 1 : 2;
+                float Yf[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
+                for (int q = 0; q < 2 * NP; ++q) {
+#pragma unroll
+                  for (int k = 0; k < NS; ++k) {
+                    const float4 v = __ldcg(jscr + ((size_t)fr * NP * 2 + q) * NS + k);
+                    Yf[4 * k] += v.x; Yf[4 * k + 1] += v.y; Yf[4 * k + 2] += v.z; Yf[4 * k + 3] += v.w;
+                  }
+                }
+                float* J = jac + (size_t)fr * D * D;
+#pragma unroll
+                for (int ja = 0, p = 0; ja < D; ++ja)
+#pragma unroll
+                  for (int jb = ja; jb < D; ++jb, ++p) {
+                    const float v = ja == jb ? fmaf(2.f * s2, Yf[p], 2.f * a.kappa) : (2.f * s2) * Yf[p];
+                    J[ja * D + jb] = v;
+                    J[jb * D + ja] = v;
+                  }
               }
             }
           }
@@ -911,6 +955,18 @@ icnn_tc3_fwd_kernel(const __grid_constant__ Tc3Args a) {
     tc_fence_after();
     asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512));
   }
+}
+
+template <int D, int MODE>
+__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(k3Threads, 1)
+icnn_tc3_fwd_kernel(const __grid_constant__ Tc3Args a) {
+  tc3_fwd_body<D, MODE, false>(a, nullptr, nullptr);
+}
+
+template <int D, int MODE>
+__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(k3Threads, 1)
+icnn_tc3_fwd_jac_kernel(const __grid_constant__ Tc3Args a, float4* __restrict__ jscr, float* __restrict__ jac) {
+  tc3_fwd_body<D, MODE, true>(a, jscr, jac);
 }
 
 // =====================================================================================================
@@ -2339,11 +2395,21 @@ static int launch_tc3(const Tc3Args& args, int units, cudaStream_t st) {
   return check_launch();
 }
 
-int tc3_fwd(const float* z, const WsLayout& L, float kappa, float* psi, float* xhat, uint32_t* mask1, uint8_t* mask2,
-            int precision, float* ws, float* accsave, cudaStream_t st) {
+template <int D, int MODE>
+static int launch_tc3_jac(const Tc3Args& args, int units, float4* jscr, float* jac, cudaStream_t st) {
+  const size_t smem = tc3_smem_bytes<MODE>(args.Hq);
+  static int max_clusters = 0;
+  if (max_clusters == 0)
+    max_clusters = max_clusters_for(reinterpret_cast<const void*>(icnn_tc3_fwd_jac_kernel<D, MODE>), smem, k3Threads);
+  const int G = units < max_clusters ? units : max_clusters;
+  icnn_tc3_fwd_jac_kernel<D, MODE><<<2 * G, k3Threads, smem, st>>>(args, jscr, jac);
+  return check_launch();
+}
+
+// the arguments of one pair-kernel forward (both variants); returns the unit count, or a negative error code
+static int tc3_fwd_args(const float* z, const WsLayout& L, float kappa, float* psi, float* xhat, uint32_t* mask1,
+                        uint8_t* mask2, int mode, float* ws, float* accsave, Tc3Args& args) {
   if (L.Bp / 256 > kTc3MaxTiles) return B200VAE_EUNSUP;
-  const int mode = tc3_mode(precision);
-  Tc3Args args;
   {
     Tc3Maps mp;
     int rc = get_maps3(ws, L, mode, &mp);
@@ -2374,7 +2440,15 @@ int tc3_fwd(const float* z, const WsLayout& L, float kappa, float* psi, float* x
   // measured by leaving each out), 2.0e-6 in four (0.544 ms)
   args.cscr = reinterpret_cast<float4*>(ws + L.cscr);
   args.NC = (mode != kTf32 && L.Hq % kTc3ChunkK == 0) ? L.Hq / kTc3ChunkK : 1;
-  const int units = (args.want_x ? 2 : 1) * args.T * args.NP;
+  return (args.want_x ? 2 : 1) * args.T * args.NP;
+}
+
+int tc3_fwd(const float* z, const WsLayout& L, float kappa, float* psi, float* xhat, uint32_t* mask1, uint8_t* mask2,
+            int precision, float* ws, float* accsave, cudaStream_t st) {
+  const int mode = tc3_mode(precision);
+  Tc3Args args;
+  const int units = tc3_fwd_args(z, L, kappa, psi, xhat, mask1, mask2, mode, ws, accsave, args);
+  if (units < 0) return units;
 #define B200VAE_TC3(DD)                                                       \
   return mode == kF16 ? launch_tc3<DD, kF16>(args, units, st)                 \
          : mode == kX3 ? launch_tc3<DD, kX3>(args, units, st) : launch_tc3<DD, kTf32>(args, units, st)
@@ -2384,6 +2458,24 @@ int tc3_fwd(const float* z, const WsLayout& L, float kappa, float* psi, float* x
     default: B200VAE_TC3(3);
   }
 #undef B200VAE_TC3
+}
+
+int tc3_fwd_jac(const float* z, const WsLayout& L, float kappa, float* psi, float* xhat, uint32_t* mask1, uint8_t* mask2,
+                float* jac, float4* jscr, int precision, float* ws, cudaStream_t st) {
+  const int mode = tc3_mode(precision);
+  Tc3Args args;
+  const int units = tc3_fwd_args(z, L, kappa, psi, xhat, mask1, mask2, mode, ws, nullptr, args);
+  if (units < 0) return units;
+#define B200VAE_TC3J(DD)                                                                    \
+  return mode == kF16 ? launch_tc3_jac<DD, kF16>(args, units, jscr, jac, st)                \
+         : mode == kX3 ? launch_tc3_jac<DD, kX3>(args, units, jscr, jac, st)                \
+                       : launch_tc3_jac<DD, kTf32>(args, units, jscr, jac, st)
+  switch (L.d) {
+    case 1: B200VAE_TC3J(1);
+    case 2: B200VAE_TC3J(2);
+    default: B200VAE_TC3J(3);
+  }
+#undef B200VAE_TC3J
 }
 
 }  // namespace b200vae

@@ -22,7 +22,8 @@ import torch
 
 from . import model as _model
 from .train import train_model  # noqa: F401  (lipschitz.py:23-44, same signature)
-from .utils import estimate_lipschitz_allpairs, estimate_local_lipschitz, estimate_local_lipschitz_batched, reparameterize
+from .utils import (estimate_lipschitz_allpairs, estimate_local_lipschitz, estimate_local_lipschitz_batched,
+                    estimate_local_lipschitz_jacobian, reparameterize)
 
 DEFAULT_EMPTY_CELL_FILL_VALUE = -5.0     # lipschitz.py:19
 
@@ -117,12 +118,18 @@ def _get_data_based_lipschitz(model, test_dataset, device, num_samples=5000, num
                               empty_cell_fill_value=DEFAULT_EMPTY_CELL_FILL_VALUE, pairs="sampled"):
     """lipschitz.py:157-194 -> (inverse_lipschitz, lipschitz, bi_lipschitz) floats.  pairs="all" (an extension) takes the
     same triple over every pair of the same `num_samples` points instead of `num_pairs_lips` random pairs: exact
-    quantiles, utils.estimate_lipschitz_allpairs(quantile=0.05)."""
-    if pairs not in ("sampled", "all"):
-        raise ValueError(f"pairs must be 'sampled' or 'all', got {pairs!r}")
+    quantiles, utils.estimate_lipschitz_allpairs(quantile=0.05).  pairs="jacobian" (an extension, LIDVAE only) takes it
+    over the decoder's local constants at those points: the extreme singular values of its exact Jacobian,
+    utils.estimate_local_lipschitz_jacobian(quantile=0.05)."""
+    if pairs not in ("sampled", "all", "jacobian"):
+        raise ValueError(f"pairs must be 'sampled', 'all' or 'jacobian', got {pairs!r}")
+    if pairs == "jacobian" and not hasattr(model, "decode_jacobian"):
+        raise ValueError(f"pairs='jacobian' needs a decoder with an exact Jacobian (LIDVAE), not {type(model).__name__}")
     model.eval()
     with torch.no_grad():
         z, _, _ = _data_based_samples(model, test_dataset, device, num_samples)
+        if pairs == "jacobian":
+            return estimate_local_lipschitz_jacobian(model, z, quantile=0.05)
         if pairs == "all":
             r = estimate_lipschitz_allpairs(model.decode, z, quantile=0.05)
             return r["inverse_lipschitz"], r["lipschitz"], r["bi_lipschitz"]
@@ -201,9 +208,10 @@ def build_parser():
     p.add_argument("--wu_repeat_interval", type=int, default=10)
     p.add_argument("--precision", type=str, default="fp32", choices=["fp32", "f16x3", "tf32x3", "tf32"],
                    help="arithmetic of the ICNN contractions (extension; fp32 = the parity path)")
-    p.add_argument("--lipschitz_pairs", type=str, default="sampled", choices=["sampled", "all"],
-                   help="pairs of the data-based Lipschitz estimate (extension): the reference's random pairs, or every "
-                        "pair of the 5000 samples with exact quantiles; the per-cell grids always sample")
+    p.add_argument("--lipschitz_pairs", type=str, default="sampled", choices=["sampled", "all", "jacobian"],
+                   help="pairs of the data-based Lipschitz estimate (extension): the reference's random pairs, every "
+                        "pair of the 5000 samples with exact quantiles, or (lidvae only) no pairs but the singular values "
+                        "of the decoder's exact Jacobian at the 5000 samples; the per-cell grids always sample")
     return p
 
 
@@ -227,6 +235,8 @@ def evaluate(model, dataset, K, K_z, z_min, z_max, latent_dim, device, num_pairs
 
 def main(argv=None):
     args = build_parser().parse_args(argv)
+    if args.lipschitz_pairs == "jacobian" and args.model != "lidvae":
+        raise ValueError("--lipschitz_pairs jacobian needs --model lidvae (the decoder's exact Jacobian)")
     os.makedirs(args.output_dir, exist_ok=True)
     seed = 42 if args.seed is None else args.seed
     random.seed(seed); np.random.seed(seed); torch.manual_seed(seed)

@@ -413,6 +413,31 @@ class LIDVAE(VAE):
         _, y = self.decoder[1].brenier(x, self.il_factor)
         return self.decoder[2](y)
 
+    def decode_jacobian(self, input):
+        """(recon, J [B,Dx,D], svals [B,min(Dx,D)]): decode(input), the decoder's exact Jacobian J = J2(x) . B . J1(z) and
+        its singular values (descending) -- two fused Brenier-map forwards that also return their Jacobians
+        (module.ICNN.brenier_jacobian) and one chain kernel (ops.jacobian_chain); the model's `B` buffer is the middle
+        factor, so a user-modified B is honoured like decode() honours it.  recon is what decode() computes with the same
+        kernels.  sigma_min >= inverse_lipschitz^2 is the decoder's inverse-Lipschitz guarantee (each map is 2 kappa-strongly
+        monotone, kappa = inverse_lipschitz / 2).  Plain tensors, no autograd graph (not differentiable).  Decoders whose
+        second ICNN is wider than the fused kernels take (the image-shaped ones, Dx > 4) raise B200VaeError."""
+        first, second = self.decoder[0], self.decoder[1]
+        for ic in (first, second):
+            ic.precision = self.precision
+        Dx, D = self.B.shape
+        if Dx > module.ICNN.FUSED_MAX_D or D > module.ICNN.FUSED_MAX_D:
+            raise _C.B200VaeError(f"decode_jacobian: the decoder's ICNN inputs (D = {D}, Dx = {Dx}) exceed the fused "
+                                  f"kernels' limit of {module.ICNN.FUSED_MAX_D}")
+        with torch.no_grad():
+            _, x, J1 = first.brenier_jacobian(input, self.il_factor)
+            if not self._B_is_eye():                       # the same x as decode() computes
+                x = F.linear(x, self.B)
+            elif Dx != D:
+                x = F.pad(x, (0, Dx - D))
+            _, y, J2 = second.brenier_jacobian(x, self.il_factor)
+            J, svals = ops.jacobian_chain(J2, self.B, J1)
+            return self.decoder[2](y), J, svals
+
     def _prepare_decoder_early(self, input):
         """Training steps on the fused d <= 4 kernels: start building both ICNNs' prepared operands (they depend on the
         weights only) on side streams before the encoder runs -- ops.icnn_prepare_early.  Anything this cannot predict

@@ -109,6 +109,23 @@ class ICNN(nn.Module):
 
     defer_param_grads_ok = True      # see ops.set_defer_hint; model.LIDVAE clears it on its second ICNN
 
+    def brenier_jacobian(self, input, kappa=0.0):
+        """(psi [B], xhat [B,d], jac [B,d,d]): brenier() plus the exact Jacobian d xhat / d z = A0^T diag(2 s0^2 gx1) A0
+        + 2 kappa I, from the same fused forward (symmetric, >= 2 kappa I).  Plain tensors without an autograd graph:
+        the Jacobian is not differentiable.  Every batch size runs the fused kernels (also FP32 below FP32_TILED_BELOW).
+        Limits: d <= 4 (FP32), d <= 3 and H <= 1024 (tensor-core precisions); B200VaeError otherwise."""
+        prec = self._prec()
+        d, H = self.in_channel, self.hidden_channel
+        if d > self.FUSED_MAX_D:
+            raise _C.B200VaeError(f"brenier_jacobian: input width d = {d} exceeds the fused kernels' limit d <= "
+                                  f"{self.FUSED_MAX_D}")
+        if prec != _C.PREC_FP32 and (d > 3 or H > 1024):
+            raise _C.B200VaeError(f"brenier_jacobian: precision {self.precision!r} needs d <= 3 and H <= 1024 "
+                                  f"(got d = {d}, H = {H}); use precision='fp32'")
+        if not hasattr(self, "_infer_cache"):
+            self._infer_cache = {}
+        return ops.icnn_brenier_jacobian(input, float(kappa), self._mode(), prec, self._flat_params(), self._infer_cache)
+
 
 class PlainConvolution(nn.Module):
     """conv3x3-BN-LReLU twice, no skip connection (module.py:4-26; stock cuDNN layers, outside the hot path)."""

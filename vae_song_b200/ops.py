@@ -223,6 +223,62 @@ def icnn_brenier_inference(z, kappa, mode, precision, params, cache):
     return psi, xhat
 
 
+# ---- exact Jacobians (b200vae_icnn_decode_jac, b200vae_jacobian_chain) ------------------------------------------------
+# With the LeakyReLU masks fixed the Brenier map is affine in z, so its Jacobian A0^T diag(2 s0^2 gx1) A0 + 2 kappa I comes out
+# of the same fused forward.  These functions return plain tensors: the Jacobian is NOT differentiable (no autograd graph;
+# a Jacobian penalty in training would need its own backward).
+def icnn_decode_jac(z, ws, d, H, kappa, precision, save_masks=False):
+    """(psi [B], xhat [B,d], jac [B,d,d], mask1 | None, mask2 | None) on a prepared workspace `ws`."""
+    lib = _C.load()
+    B, dev = z.shape[0], z.device
+    Hp = (H + 127) // 128 * 128
+    psi = torch.empty(B, dtype=torch.float32, device=dev)
+    xhat = torch.empty(B, d, dtype=torch.float32, device=dev)
+    jac = torch.empty(B, d, d, dtype=torch.float32, device=dev)
+    mask1 = torch.empty(B, Hp // 32, dtype=torch.int32, device=dev) if save_masks else None
+    mask2 = torch.empty(B, dtype=torch.uint8, device=dev) if save_masks else None
+    nscr = lib.b200vae_icnn_jac_scratch_bytes(B, d, H, precision)
+    scr = torch.empty(nscr, dtype=torch.uint8, device=dev) if nscr else None
+    _C.check(lib.b200vae_icnn_decode_jac(_ptr(z), B, d, H, float(kappa), _ptr(psi), _ptr(xhat), _ptr(jac), _ptr(mask1),
+                                         _ptr(mask2), precision, _ptr(ws), ws.numel(), _ptr(scr), nscr, _stream()),
+             "icnn_decode_jac")
+    return psi, xhat, jac, mask1, mask2
+
+
+def icnn_brenier_jacobian(z, kappa, mode, precision, params, cache):
+    """(psi [B], xhat [B,d], jac [B,d,d] = d xhat / d z) without an autograd graph; the prepared workspace is shared with
+    icnn_brenier_inference through `cache` (same key).  jac is not differentiable."""
+    z = _req(z.detach(), "z")
+    params = [_req(p.detach(), k) for p, k in zip(params, PARAM_FIELDS)]
+    H, d = params[0].shape
+    if z.dim() != 2 or z.shape[1] != d:
+        raise _C.B200VaeError(f"z must be [B,{d}], got {tuple(z.shape)}")
+    key = (z.shape[0], mode, precision, z.device, torch.cuda.current_stream().cuda_stream, _param_state(params))
+    if cache.get("key") != key:
+        cache["ws"] = icnn_prepare(params, d, H, mode, precision, z.shape[0], False)
+        cache["key"] = key
+    psi, xhat, jac, _, _ = icnn_decode_jac(z, cache["ws"], d, H, kappa, precision)
+    return psi, xhat, jac
+
+
+def jacobian_chain(J2, M, J1, want_J=True, want_svals=True):
+    """J = J2 . M . J1 [B,Dx,D] and its singular values [B,min(Dx,D)] (descending), one kernel, fp64 inside; either output
+    may be skipped (None returned).  J2 [B,Dx,Dx], M [Dx,D], J1 [B,D,D]; Dx, D <= 4.  Not differentiable."""
+    lib = _C.load()
+    J2, M, J1 = (_req(t.detach(), n) for t, n in ((J2, "J2"), (M, "M"), (J1, "J1")))
+    B, Dx, D = J2.shape[0], M.shape[0], M.shape[1]
+    if J2.shape != (B, Dx, Dx) or J1.shape != (B, D, D):
+        raise _C.B200VaeError(f"jacobian_chain: shapes J2 {tuple(J2.shape)}, M {tuple(M.shape)}, J1 {tuple(J1.shape)} "
+                              "do not chain")
+    J = torch.empty(B, Dx, D, dtype=torch.float32, device=J1.device) if want_J else None
+    s = torch.empty(B, min(Dx, D), dtype=torch.float32, device=J1.device) if want_svals else None
+    if B == 0:
+        return J, s
+    _C.check(lib.b200vae_jacobian_chain(_ptr(J2), _ptr(M), _ptr(J1), B, Dx, D, _ptr(J), _ptr(s), _stream()),
+             "jacobian_chain")
+    return J, s
+
+
 class IcnnBrenierFn(torch.autograd.Function):
     """(psi [B], xhat [B,d]) = fused ICNN potential + Brenier map.  Replaces module.py:142-148 followed
     by model.py:820-822.  backward = the double-backward PyTorch would run through autograd.grad."""

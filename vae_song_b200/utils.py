@@ -211,6 +211,21 @@ def estimate_local_lipschitz(func, X, num_pairs=2000, metric=2, quantile=0.05, e
     return res[0], res[1], res[2]
 
 
+def estimate_local_lipschitz_jacobian(model, Z, quantile=0.05, eps=1e-3):
+    """The reference's (inverse_lipschitz, lipschitz, bi_lipschitz) triple (utils.py:563-567) on the decoder's LOCAL
+    constants instead of finite-pair ratios: per point, the smallest and largest singular values of the exact Jacobian
+    (model.decode_jacobian), A = max(quantile(sigma_min, q), eps), B = quantile(sigma_max, 1 - q) (torch.quantile's linear
+    rule) -> (1/A, B, max(1/A, B)) as Python floats; (0, 0, 0) for an empty Z."""
+    if Z.size(0) == 0:
+        return 0.0, 0.0, 0.0
+    _, _, s = model.decode_jacobian(Z)
+    A = torch.quantile(s[:, -1], quantile).clamp(min=eps)
+    Bq = torch.quantile(s[:, 0], 1 - quantile)
+    invA = 1.0 / A
+    res = torch.stack([invA, Bq, torch.maximum(invA, Bq)]).tolist()
+    return res[0], res[1], res[2]
+
+
 def estimate_local_lipschitz_batched(func, X_list, num_pairs=2000, quantile=0.05, eps=1e-3, use_grad=False):
     """`estimate_local_lipschitz` for MANY sample sets at once (the per-cell loops of lipschitz.py:48-154 call the
     estimator up to 512 times, each with 2 small decodes, 2 sorts and 3 `.item()` syncs).  Here all cells share
