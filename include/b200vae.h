@@ -130,6 +130,32 @@ int b200vae_icnn_decode_jac(const float* z, int B, int d, int H, float kappa, fl
 int b200vae_jacobian_chain(const float* J2, const float* M, const float* J1, int B, int Dx, int D, float* J, float* svals,
                            void* stream);
 
+/* Left inverse of the Brenier map: z = T^{-1}(x), T = grad(psi + kappa|.|^2), by batched Newton steps (csrc/inverse.cu).
+ * z* is the unique minimiser of f(z) = psi(z) + kappa|z|^2 - <x, z>; its gradient xhat(z) - x and Hessian jac come from
+ * b200vae_icnn_decode_jac.  One ROUND is
+ *     b200vae_icnn_decode_jac(z_trial, ...) -> xhat, jac;   b200vae_brenier_newton_step(x, xhat, jac, ..., round, ...)
+ * after one b200vae_brenier_inverse_init.  The step kernel takes a Newton step by Cholesky with a line search on the sign
+ * of (xhat - x)^T p (psi is not used), one thread per row in fp64, and writes the next trial point, the accepted z [B,d],
+ * status [B] int32 (B200VAE_INV_*) and err_bound [B] = ||xhat(z) - x|| / (2 kappa) >= ||z - z*|| (+inf at kappa = 0).
+ * A finished row keeps z and its trial point equals z; final_round != 0 turns rows still active into MAXITER.
+ *   state: caller-owned, b200vae_brenier_inverse_state_bytes(B, d) bytes, 16-byte aligned, set by _init; its first four
+ *   bytes after round k hold, at int32 index (k & 1), the number of rows still active (integer atomics: deterministic).
+ *   tolerance: a row converges when ||xhat(z) - x|| <= tol_rel ||x|| + tol_abs.  z0 [B,d] or NULL (start at 0).
+ * 1 <= d <= 4 (B200VAE_EUNSUP above), B >= 1; null pointers (z0 excepted) B200VAE_EALIGN; a short state B200VAE_EWS. */
+#define B200VAE_INV_ACTIVE 0
+#define B200VAE_INV_CONVERGED 1   /* ||xhat(z) - x|| <= tol                                                        */
+#define B200VAE_INV_MAXITER 2     /* still active after the last round                                             */
+#define B200VAE_INV_STALLED 3     /* line search collapsed at t = 0 (x in a jump of the gradient / at a kink), or  */
+                                  /* the step no longer moves z in fp32                                            */
+#define B200VAE_INV_SINGULAR 4    /* Cholesky of jac failed (kappa = 0 only)                                       */
+#define B200VAE_INV_NONFINITE 5   /* x, z0 or xhat(z) not finite                                                   */
+size_t b200vae_brenier_inverse_state_bytes(int B, int d);
+int b200vae_brenier_inverse_init(const float* x, const float* z0, int B, int d, float tol_rel, float tol_abs, void* state,
+                                 size_t state_bytes, float* z_trial, float* z, int* status, float* err_bound, void* stream);
+int b200vae_brenier_newton_step(const float* x, const float* xhat, const float* jac, int B, int d, float kappa, int round,
+                                int final_round, void* state, size_t state_bytes, float* z_trial, float* z, int* status,
+                                float* err_bound, void* stream);
+
 /* Fused reparameterisation + Gaussian KL + reconstruction (+ latent reconstruction).
  * Replaces model.py:843 / :423-424 (z = mu + eps*exp(lv/2)), :884/:550/:606 (KL), :870/:542/:589
  * (MSE) or :872-882 (log-MSE), :551/:603 (latent recon, mean over dim 0 = L).

@@ -37,8 +37,11 @@ EXPORTS = [
     "b200vae_mlp_stack_bwd", "b200vae_lipschitz_select_state_bytes", "b200vae_lipschitz_select_hist_bytes",
     "b200vae_lipschitz_quantile_ranks", "b200vae_lipschitz_select_count", "b200vae_lipschitz_select_locate",
     "b200vae_icnn_jac_scratch_bytes", "b200vae_icnn_decode_jac", "b200vae_jacobian_chain",
+    "b200vae_brenier_inverse_state_bytes", "b200vae_brenier_inverse_init", "b200vae_brenier_newton_step",
 ]
 LIPSCHITZ_SELECT_PASSES = 3
+# per-row status of the Newton left inverse (B200VAE_INV_*); a larger value is a worse outcome
+INV_ACTIVE, INV_CONVERGED, INV_MAXITER, INV_STALLED, INV_SINGULAR, INV_NONFINITE = range(6)
 PEER_MAX_WORLD, PEER_HANDLE_BYTES = 16, 64
 
 
@@ -114,6 +117,12 @@ def load():
     lib.b200vae_icnn_decode_jac.argtypes = [vp, i, i, i, f, vp, vp, vp, vp, vp, i, vp, sz, vp, sz, vp]
     lib.b200vae_jacobian_chain.restype = i
     lib.b200vae_jacobian_chain.argtypes = [vp, vp, vp, i, i, i, vp, vp, vp]
+    lib.b200vae_brenier_inverse_state_bytes.restype = sz
+    lib.b200vae_brenier_inverse_state_bytes.argtypes = [i, i]
+    lib.b200vae_brenier_inverse_init.restype = i
+    lib.b200vae_brenier_inverse_init.argtypes = [vp, vp, i, i, f, f, vp, sz, vp, vp, vp, vp, vp]
+    lib.b200vae_brenier_newton_step.restype = i
+    lib.b200vae_brenier_newton_step.argtypes = [vp, vp, vp, i, i, f, i, i, vp, sz, vp, vp, vp, vp, vp]
     lib.b200vae_loss_fwd.restype = i
     lib.b200vae_loss_fwd.argtypes = [vp, vp, vp, vp, i, i, i, vp, vp, i, i, vp, vp, vp, i, i, i, vp, vp]
     lib.b200vae_loss_bwd.restype = i

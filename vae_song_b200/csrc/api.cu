@@ -213,6 +213,41 @@ extern "C" int b200vae_icnn_decode_jac(const float* z, int B, int d, int H, floa
                      ws_base(ws), (cudaStream_t)stream);
 }
 
+static int inverse_shape_ok(int B, int d) {
+  if (B <= 0 || d <= 0) return B200VAE_ESHAPE;
+  return d <= 4 ? B200VAE_OK : B200VAE_EUNSUP;
+}
+
+extern "C" size_t b200vae_brenier_inverse_state_bytes(int B, int d) {
+  return inverse_shape_ok(B, d) ? 0 : inverse_state_bytes(B);
+}
+
+extern "C" int b200vae_brenier_inverse_init(const float* x, const float* z0, int B, int d, float tol_rel, float tol_abs,
+                                            void* state, size_t state_bytes, float* z_trial, float* z, int* status,
+                                            float* err_bound, void* stream) {
+  int rc = inverse_shape_ok(B, d);
+  if (rc) return rc;
+  if (!x || !state || !z_trial || !z || !status || !err_bound || !aligned16(state) || !aligned4(x) ||
+      (z0 && !aligned4(z0)))
+    return B200VAE_EALIGN;
+  if (state_bytes < inverse_state_bytes(B)) return B200VAE_EWS;
+  return brenier_inverse_init(x, z0, B, d, tol_rel, tol_abs, state, z_trial, z, status, err_bound, (cudaStream_t)stream);
+}
+
+extern "C" int b200vae_brenier_newton_step(const float* x, const float* xhat, const float* jac, int B, int d, float kappa,
+                                           int round, int final_round, void* state, size_t state_bytes, float* z_trial,
+                                           float* z, int* status, float* err_bound, void* stream) {
+  int rc = inverse_shape_ok(B, d);
+  if (rc) return rc;
+  if (round < 0) return B200VAE_ESHAPE;
+  if (!x || !xhat || !jac || !state || !z_trial || !z || !status || !err_bound || !aligned16(state) || !aligned4(x) ||
+      !aligned4(xhat) || !aligned4(jac))
+    return B200VAE_EALIGN;
+  if (state_bytes < inverse_state_bytes(B)) return B200VAE_EWS;
+  return brenier_newton_step(x, xhat, jac, B, d, kappa, round, final_round, state, z_trial, z, status, err_bound,
+                             (cudaStream_t)stream);
+}
+
 extern "C" int b200vae_last_cuda_error(void) { return g_last_cuda_error; }
 extern "C" const char* b200vae_version(void) { return "b200vae 0.2 (sm_100a)"; }
 extern "C" long long b200vae_launch_count(void) { return g_launch_count; }

@@ -101,6 +101,12 @@ int tc3_fwd_jac(const float* z, const WsLayout& L, float kappa, float* psi, floa
 // chain + singular values of the decoder's Jacobian, jacobian.cu
 int jacobian_chain(const float* J2, const float* M, const float* J1, int B, int Dx, int D, float* J, float* svals,
                    cudaStream_t st);
+// Newton left inverse of the Brenier map, inverse.cu
+size_t inverse_state_bytes(int B);
+int brenier_inverse_init(const float* x, const float* z0, int B, int d, float tol_rel, float tol_abs, void* state,
+                         float* ztrial, float* z, int* status, float* err, cudaStream_t st);
+int brenier_newton_step(const float* x, const float* xhat, const float* jac, int B, int d, float kappa, int round,
+                        int final_round, void* state, float* ztrial, float* z, int* status, float* err, cudaStream_t st);
 int tc_bwd(const float* z, const float* v, const uint32_t* mask1, const uint8_t* mask2, const WsLayout& L,
            const b200vae_icnn_params* p, int mode, float kappa, const b200vae_icnn_grads* g, float* dz, int precision,
            float* ws, const float* accsave, int phase, cudaStream_t st);

@@ -438,6 +438,43 @@ class LIDVAE(VAE):
             J, svals = ops.jacobian_chain(J2, self.B, J1)
             return self.decoder[2](y), J, svals
 
+    def decode_inverse(self, recon, z0=None, max_iter=ops.INVERSE_MAX_ITER, tol=None):
+        """(z [B,D], status [B] int32, err_bound [B]): the decoder's left inverse, z with decode(z) ~ recon, by batched
+        Newton steps on both Brenier maps (module.ICNN.brenier_inverse): x = T1^{-1}(recon), x1 = B^+ x (a slice when
+        B = eye(Dx, D); a user-modified B through its pseudo-inverse -- rank-deficient B raises), z = T0^{-1}(x1).
+        err_bound = e0 + ||B^+||_2 e1 / (2 kappa) bounds ||z - z*|| (T0^{-1} is 1/(2 kappa)-Lipschitz; +inf at
+        inverse_lipschitz = 0); status is the worse of the two stages' (_C.INV_*, larger = worse).  z0 [B,D] warm-starts
+        stage 0 and B . T0(z0) stage 1.  Plain tensors, no autograd graph.  Decoders whose ICNN inputs are wider than 4
+        (the image-shaped ones) raise B200VaeError."""
+        first, second = self.decoder[0], self.decoder[1]
+        for ic in (first, second):
+            ic.precision = self.precision
+        Dx, D = self.B.shape
+        if Dx > module.ICNN.FUSED_MAX_D or D > module.ICNN.FUSED_MAX_D:
+            raise _C.B200VaeError(f"decode_inverse: the decoder's ICNN inputs (D = {D}, Dx = {Dx}) exceed the fused "
+                                  f"kernels' limit of {module.ICNN.FUSED_MAX_D}")
+        eye = self._B_is_eye()
+        with torch.no_grad():
+            if eye:
+                pinv_norm = 1.0
+            else:
+                s = torch.linalg.svdvals(self.B.double())
+                if s[-1] <= s[0] * D * torch.finfo(torch.float32).eps:
+                    raise _C.B200VaeError(f"decode_inverse: the decoder's B buffer is rank-deficient (singular values "
+                                          f"{s.tolist()}); it has no left inverse")
+                pinv = torch.linalg.pinv(self.B.double()).float()
+                pinv_norm = float(1.0 / s[-1])
+            x0 = None
+            if z0 is not None:
+                _, x0 = first.brenier(z0, self.il_factor)
+                x0 = F.pad(x0, (0, Dx - D)) if eye else F.linear(x0, self.B)
+            x, st1, e1, _ = second.brenier_inverse(recon.reshape(recon.shape[0], -1), self.il_factor, z0=x0,
+                                                   max_iter=max_iter, tol=tol)
+            x1 = x[:, :D].contiguous() if eye else F.linear(x, pinv)
+            z, st0, e0, _ = first.brenier_inverse(x1, self.il_factor, z0=z0, max_iter=max_iter, tol=tol)
+            bound = e0 + pinv_norm * e1 / (2.0 * self.il_factor) if self.il_factor > 0 else torch.full_like(e0, float("inf"))
+            return z, torch.maximum(st0, st1), bound
+
     def _prepare_decoder_early(self, input):
         """Training steps on the fused d <= 4 kernels: start building both ICNNs' prepared operands (they depend on the
         weights only) on side streams before the encoder runs -- ops.icnn_prepare_early.  Anything this cannot predict

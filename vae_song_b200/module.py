@@ -109,22 +109,33 @@ class ICNN(nn.Module):
 
     defer_param_grads_ok = True      # see ops.set_defer_hint; model.LIDVAE clears it on its second ICNN
 
+    def _check_jacobian_limits(self, what):
+        d, H = self.in_channel, self.hidden_channel
+        if d > self.FUSED_MAX_D:
+            raise _C.B200VaeError(f"{what}: input width d = {d} exceeds the fused kernels' limit d <= {self.FUSED_MAX_D}")
+        if self._prec() != _C.PREC_FP32 and (d > 3 or H > 1024):
+            raise _C.B200VaeError(f"{what}: precision {self.precision!r} needs d <= 3 and H <= 1024 "
+                                  f"(got d = {d}, H = {H}); use precision='fp32'")
+        if not hasattr(self, "_infer_cache"):
+            self._infer_cache = {}
+
     def brenier_jacobian(self, input, kappa=0.0):
         """(psi [B], xhat [B,d], jac [B,d,d]): brenier() plus the exact Jacobian d xhat / d z = A0^T diag(2 s0^2 gx1) A0
         + 2 kappa I, from the same fused forward (symmetric, >= 2 kappa I).  Plain tensors without an autograd graph:
         the Jacobian is not differentiable.  Every batch size runs the fused kernels (also FP32 below FP32_TILED_BELOW).
         Limits: d <= 4 (FP32), d <= 3 and H <= 1024 (tensor-core precisions); B200VaeError otherwise."""
-        prec = self._prec()
-        d, H = self.in_channel, self.hidden_channel
-        if d > self.FUSED_MAX_D:
-            raise _C.B200VaeError(f"brenier_jacobian: input width d = {d} exceeds the fused kernels' limit d <= "
-                                  f"{self.FUSED_MAX_D}")
-        if prec != _C.PREC_FP32 and (d > 3 or H > 1024):
-            raise _C.B200VaeError(f"brenier_jacobian: precision {self.precision!r} needs d <= 3 and H <= 1024 "
-                                  f"(got d = {d}, H = {H}); use precision='fp32'")
-        if not hasattr(self, "_infer_cache"):
-            self._infer_cache = {}
-        return ops.icnn_brenier_jacobian(input, float(kappa), self._mode(), prec, self._flat_params(), self._infer_cache)
+        self._check_jacobian_limits("brenier_jacobian")
+        return ops.icnn_brenier_jacobian(input, float(kappa), self._mode(), self._prec(), self._flat_params(),
+                                         self._infer_cache)
+
+    def brenier_inverse(self, x, kappa=0.0, z0=None, max_iter=ops.INVERSE_MAX_ITER, tol=None):
+        """(z [B,d], status [B] int32, err_bound [B], rounds): the left inverse z = T^{-1}(x) of brenier()'s map
+        T = grad(psi + kappa|.|^2), by batched Newton steps on the fused Jacobian kernels (ops.icnn_brenier_inverse;
+        status values _C.INV_*).  ||z - T^{-1}(x)|| <= err_bound = ||T(z) - x|| / (2 kappa) on every row (+inf at
+        kappa = 0).  Plain tensors, not differentiable.  Same limits as brenier_jacobian."""
+        self._check_jacobian_limits("brenier_inverse")
+        return ops.icnn_brenier_inverse(x, float(kappa), self._mode(), self._prec(), self._flat_params(), self._infer_cache,
+                                        z0=z0, max_iter=max_iter, tol=tol)
 
 
 class PlainConvolution(nn.Module):

@@ -205,21 +205,27 @@ def _param_state(params):
     return (_weights_epoch[0],) + tuple((p.data_ptr(), p._version, tuple(p.shape)) for p in params)
 
 
+def _cached_ws(z, mode, precision, params, cache, name="z"):
+    """(z, H, d, prepared inference workspace) -- the workspace kept in `cache` and rebuilt only when its key changes."""
+    z = _req(z.detach(), name)
+    params = [_req(p.detach(), k) for p, k in zip(params, PARAM_FIELDS)]
+    H, d = params[0].shape
+    if z.dim() != 2 or z.shape[1] != d:
+        raise _C.B200VaeError(f"{name} must be [B,{d}], got {tuple(z.shape)}")
+    key = (z.shape[0], mode, precision, z.device, torch.cuda.current_stream().cuda_stream, _param_state(params))
+    if cache.get("key") != key:
+        cache["ws"] = icnn_prepare(params, d, H, mode, precision, z.shape[0], False)
+        cache["key"] = key
+    return z, H, d, cache["ws"]
+
+
 def icnn_brenier_inference(z, kappa, mode, precision, params, cache):
     """(psi, xhat) without an autograd graph -- evaluation loops (utils.estimate_local_lipschitz*, lipschitz.py's per-cell
     sweeps, decode under no_grad).  The prepared workspace (positive weights in every kernel layout: 4 launches) is kept in
     `cache` (a dict owned by the module) and reused while the parameters are unchanged (their `_version` counters and data
     pointers), the batch size and the precision are the same; module.py:110 re-materialises exp(W) on every call instead."""
-    z = _req(z.detach(), "z")
-    params = [_req(p.detach(), k) for p, k in zip(params, PARAM_FIELDS)]
-    H, d = params[0].shape
-    if z.dim() != 2 or z.shape[1] != d:
-        raise _C.B200VaeError(f"z must be [B,{d}], got {tuple(z.shape)}")
-    key = (z.shape[0], mode, precision, z.device, torch.cuda.current_stream().cuda_stream, _param_state(params))
-    if cache.get("key") != key:
-        cache["ws"] = icnn_prepare(params, d, H, mode, precision, z.shape[0], False)
-        cache["key"] = key
-    psi, xhat, _, _ = icnn_decode_fwd(z, cache["ws"], d, H, mode, kappa, precision, True, True, False)
+    z, H, d, ws = _cached_ws(z, mode, precision, params, cache)
+    psi, xhat, _, _ = icnn_decode_fwd(z, ws, d, H, mode, kappa, precision, True, True, False)
     return psi, xhat
 
 
@@ -248,17 +254,64 @@ def icnn_decode_jac(z, ws, d, H, kappa, precision, save_masks=False):
 def icnn_brenier_jacobian(z, kappa, mode, precision, params, cache):
     """(psi [B], xhat [B,d], jac [B,d,d] = d xhat / d z) without an autograd graph; the prepared workspace is shared with
     icnn_brenier_inference through `cache` (same key).  jac is not differentiable."""
-    z = _req(z.detach(), "z")
-    params = [_req(p.detach(), k) for p, k in zip(params, PARAM_FIELDS)]
-    H, d = params[0].shape
-    if z.dim() != 2 or z.shape[1] != d:
-        raise _C.B200VaeError(f"z must be [B,{d}], got {tuple(z.shape)}")
-    key = (z.shape[0], mode, precision, z.device, torch.cuda.current_stream().cuda_stream, _param_state(params))
-    if cache.get("key") != key:
-        cache["ws"] = icnn_prepare(params, d, H, mode, precision, z.shape[0], False)
-        cache["key"] = key
-    psi, xhat, jac, _, _ = icnn_decode_jac(z, cache["ws"], d, H, kappa, precision)
+    z, H, d, ws = _cached_ws(z, mode, precision, params, cache)
+    psi, xhat, jac, _, _ = icnn_decode_jac(z, ws, d, H, kappa, precision)
     return psi, xhat, jac
+
+
+# ---- left inverse (b200vae_brenier_inverse_init, b200vae_brenier_newton_step) -----------------------------------------
+# z = T^{-1}(x) for T = grad(psi + kappa|.|^2): Newton steps on f(z) = psi(z) + kappa|z|^2 - <x, z>, whose gradient and
+# Hessian come from the Jacobian forward.  One round = one b200vae_icnn_decode_jac at every row's trial point + one step
+# kernel (csrc/inverse.cu).  Plain tensors, not differentiable.
+INVERSE_TOL = {_C.PREC_FP32: 1e-5, _C.PREC_TF32: 5e-3, _C.PREC_TF32X3: 1e-5, _C.PREC_F16X3: 1e-5}   # declared xhat accuracy
+INVERSE_MAX_ITER = 100
+INVERSE_CHECK_EVERY = 4
+
+
+def icnn_brenier_inverse(x, kappa, mode, precision, params, cache, z0=None, max_iter=INVERSE_MAX_ITER, tol=None):
+    """(z [B,d], status [B] int32 (_C.INV_*), err_bound [B], rounds): z ~ T^{-1}(x) with ||z - T^{-1}(x)|| <= err_bound
+    (= ||xhat(z) - x|| / (2 kappa), +inf at kappa = 0).  A row converges when ||xhat(z) - x|| <= tol (||x|| + 1); tol
+    defaults to the precision's declared xhat accuracy.  z0 [B,d] warm-starts (default 0).  The prepared workspace is the
+    one of icnn_brenier_inference / icnn_brenier_jacobian (same `cache`, same key).  Eager: stops once every row has
+    finished, reading the device's count of active rows (4 bytes) every INVERSE_CHECK_EVERY rounds; while a CUDA graph is
+    being captured: exactly max_iter rounds.  Rows still active after the last round are MAXITER."""
+    lib = _C.load()
+    x, H, d, ws = _cached_ws(x, mode, precision, params, cache, "x")
+    B, dev = x.shape[0], x.device
+    if max_iter < 1:
+        raise _C.B200VaeError(f"max_iter must be >= 1, got {max_iter}")
+    if z0 is not None:
+        z0 = _req(z0.detach(), "z0")
+        if z0.shape != x.shape:
+            raise _C.B200VaeError(f"z0 must be {tuple(x.shape)}, got {tuple(z0.shape)}")
+    tol = INVERSE_TOL[precision] if tol is None else float(tol)
+    nst = lib.b200vae_brenier_inverse_state_bytes(B, d)
+    state = torch.empty(nst, dtype=torch.uint8, device=dev)
+    trial = torch.empty(B, d, dtype=torch.float32, device=dev)
+    z = torch.empty(B, d, dtype=torch.float32, device=dev)
+    status = torch.empty(B, dtype=torch.int32, device=dev)
+    err = torch.empty(B, dtype=torch.float32, device=dev)
+    psi = torch.empty(B, dtype=torch.float32, device=dev)
+    xhat = torch.empty(B, d, dtype=torch.float32, device=dev)
+    jac = torch.empty(B, d, d, dtype=torch.float32, device=dev)
+    nscr = lib.b200vae_icnn_jac_scratch_bytes(B, d, H, precision)
+    scr = torch.empty(nscr, dtype=torch.uint8, device=dev) if nscr else None
+    active = state[:8].view(torch.int32)
+    st = _stream()
+    _C.check(lib.b200vae_brenier_inverse_init(_ptr(x), _ptr(z0), B, d, tol, tol, _ptr(state), nst, _ptr(trial), _ptr(z),
+                                              _ptr(status), _ptr(err), st), "brenier_inverse_init")
+    capturing = torch.cuda.is_current_stream_capturing()
+    rounds = max_iter
+    for k in range(max_iter):
+        _C.check(lib.b200vae_icnn_decode_jac(_ptr(trial), B, d, H, float(kappa), _ptr(psi), _ptr(xhat), _ptr(jac), None,
+                                             None, precision, _ptr(ws), ws.numel(), _ptr(scr), nscr, st), "icnn_decode_jac")
+        _C.check(lib.b200vae_brenier_newton_step(_ptr(x), _ptr(xhat), _ptr(jac), B, d, float(kappa), k,
+                                                 1 if k == max_iter - 1 else 0, _ptr(state), nst, _ptr(trial), _ptr(z),
+                                                 _ptr(status), _ptr(err), st), "brenier_newton_step")
+        if not capturing and (k + 1) % INVERSE_CHECK_EVERY == 0 and k + 1 < max_iter and int(active[k & 1]) == 0:
+            rounds = k + 1
+            break
+    return z, status, err, rounds
 
 
 def jacobian_chain(J2, M, J1, want_J=True, want_svals=True):
